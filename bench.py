@@ -17,6 +17,7 @@ GPUs (4 chains per GPU at N = 8), every GPU evaluates the prediction of the mini
 when N > 1.  At N = 1 the two coincide.
 
   python bench.py --gpus N --steps K --warmup W      (N > 1 under torch.distributed.run)
+  python bench.py ... --dump-outputs DIR             also write the last timed epoch's outputs to DIR/*.npy
   python bench.py --impl reference ...               CPU arm: the SEAL-3.4.5-equivalent oracle
                                                      (SEAL itself is not installable here) on the
                                                      host cores, bounded sample, same metric
@@ -277,6 +278,23 @@ def workload_config(n_gpus, scaling="strong"):
     }
 
 
+def dump_outputs(path, grad, neww, weights):
+    """What a caller of the timed epoch receives, as float64 .npy files (3 MB in all): the gradient and updated weight
+    ciphertexts and the decrypted updated weights.  A ciphertext's RNS residues [batch][size][limbs][N] reach 2^60, more
+    than float64 holds exactly, so each is stored as two exact halves: <name>_hi = residue >> 30, <name>_lo = residue mod
+    2^30.  Every epoch encrypts the sigmoid's constant term afresh (Tree_cipher) from the seeded encryptor's stream, so
+    the arrays depend on how many epochs ran before the last one (--warmup, --steps); the public key is drawn after the
+    doubling mode's Galois keys, so they also depend on --no-fast.  Runs with the same arguments write the same arrays."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"weights": np.asarray(weights, dtype=np.float64)}
+    for name, ct in (("gradient_ct", grad), ("weights_ct", neww)):
+        words = ct.numpy()
+        arrays[name + "_hi"] = (words >> np.uint64(30)).astype(np.float64)
+        arrays[name + "_lo"] = (words & np.uint64((1 << 30) - 1)).astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------ GPU arm
 def strong_units(rank, world):
     """(mini-batch, feature) gradient units of `rank` when ONE problem is split over `world` GPUs: a contiguous block
@@ -433,6 +451,8 @@ def run_gpu(args):
     problems_per_step = 1 if strong else world
     value = problems_per_step * args.steps / (ms / 1e3)
     got, err = check(neww, want) if rank == 0 else (None, None)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, grad, neww, got)
 
     e2e_steps = args.steps
     ms_e2e, (_, neww_e2e), _, _, _ = timed(lambda: prob.e2e(out_host), 1, e2e_steps)
@@ -442,10 +462,9 @@ def run_gpu(args):
 
     fast = None
     if keys_fast is not None:
-        ms_fast, (_, neww_fast), launches_fast, _, _ = timed(prob.fast, 2, max(2, args.steps))
-        fast_steps_timed = max(2, args.steps)
-        fast = {"value": problems_per_step * fast_steps_timed / (ms_fast / 1e3), "unit": UNIT, "ms_per_step": ms_fast / fast_steps_timed,
-                "gpu_launches_per_step_per_gpu": int(launches_fast) // fast_steps_timed,
+        ms_fast, (_, neww_fast), launches_fast, _, _ = timed(prob.fast, 2, args.steps)
+        fast = {"value": problems_per_step * args.steps / (ms_fast / 1e3), "unit": UNIT, "ms_per_step": ms_fast / args.steps,
+                "gpu_launches_per_step_per_gpu": int(launches_fast) // args.steps,
                 "note": "rotate-and-sum by log2(%d) doubling rotations instead of the reference's %d unit rotations "
                         "(SURVEY 8 f4): NOT the reference's op sequence, ciphertexts are not bit-identical, decrypted "
                         "weights agree within noise; reported for information, the headline value is the reference "
@@ -459,9 +478,8 @@ def run_gpu(args):
     if world > 1 and strong and not args.no_weak:
         Xw, yw = synthetic_shard(seed=10 + rank)
         probw = Problem(Xw, yw, all_units, R_PER_GPU * world)
-        wsteps = max(1, min(args.steps, 2))
-        ms_w, (_, neww_w), _, _, _ = timed(probw.resident, 1, wsteps)
-        weak = {"value": world * wsteps / (ms_w / 1e3), "unit": UNIT, "scaling": "weak", "ms_per_step": ms_w / wsteps, "steps": wsteps,
+        ms_w, (_, neww_w), _, _, _ = timed(probw.resident, 1, args.steps)
+        weak = {"value": world * args.steps / (ms_w / 1e3), "unit": UNIT, "scaling": "weak", "ms_per_step": ms_w / args.steps, "steps": args.steps,
                 "note": "every GPU holds its own 8 x 32768 shard (N independent problems, one combined update)"}
         if rank == 0:
             sh = [synthetic_shard(seed=10 + r) for r in range(world)]
@@ -785,8 +803,12 @@ def keyswitch_sweep(torch, eng, ctx15, ev15, keys15):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="timed epochs of every config-5 epoch leg (headline, e2e, doubling mode, weak scaling); the "
+                         "config-1, linear-transform and key-switch sweep legs time fixed repetition counts")
+    ap.add_argument("--warmup", type=int, default=3,
+                    help="untimed epochs before the headline leg; the later legs warm up with their own fixed counts "
+                         "(1 to 3 calls)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-sweep", action="store_true", help="skip the key-switch ops/s sweep")
@@ -798,7 +820,15 @@ def main():
                     help="strong: one 8 x 32768 problem split over the GPUs (default, BASELINE config 5); weak: one shard per GPU")
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling leg reported beside the strong one at N > 1")
     ap.add_argument("--no-config1", action="store_true", help="skip the config-1 (pulsar CSV) leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed epoch computed to DIR/<name>.npy (float64); inputs, keys and encryption "
+                         "randomness are seeded, so runs with the same arguments write the same arrays and two builds can "
+                         "be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.ncu and args.dump_outputs:
+        ap.error("--dump-outputs needs the timed epochs, which --ncu does not run")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # started as plain `python bench.py --gpus N`: relaunch as one process per GPU
         import socket

@@ -44,19 +44,32 @@ def _host_stamp():
 
 
 def build(force=False):
+    global _LIB_PATH
     stamp_path = _LIB_PATH + ".hoststamp"
     stamp = _host_stamp()
     if not force and os.path.exists(_LIB_PATH) and os.path.exists(stamp_path):
         with open(stamp_path) as fh:
             if fh.read().strip() == stamp:
                 return _LIB_PATH
+    src_dir = os.path.dirname(_LIB_PATH)
+    if not os.access(src_dir, os.W_OK):
+        # a read-only tree built on another host: compile a private copy in a temporary directory instead
+        import atexit
+        import shutil
+        import tempfile
+        src_dir = tempfile.mkdtemp(prefix="ckks_oracle_")
+        atexit.register(shutil.rmtree, src_dir, True)
+        for f in ("ckks_oracle.c", "ckks_oracle.h", "Makefile"):
+            shutil.copy(os.path.join(_HERE, f), src_dir)
+        _LIB_PATH = os.path.join(src_dir, "libckks_oracle.so")
+        stamp_path = _LIB_PATH + ".hoststamp"
     import fcntl
     with open(_LIB_PATH + ".lock", "w") as lock:          # one builder at a time (torchrun ranks, xdist workers)
         fcntl.flock(lock, fcntl.LOCK_EX)
         try:
             if not force and os.path.exists(_LIB_PATH) and os.path.exists(stamp_path) and open(stamp_path).read().strip() == stamp:
                 return _LIB_PATH
-            subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "libckks_oracle.so"])
+            subprocess.check_call(["make", "-C", src_dir, "-s", "-B", "libckks_oracle.so"])
             with open(stamp_path, "w") as fh:
                 fh.write(stamp + "\n")
         finally:

@@ -1,12 +1,13 @@
 #!/bin/bash
 # Builds the reference's own hot-path programs, UNCHANGED, against the seal/seal.h shim and
-# libckks_b200.so.  Only works where /root/reference exists (the build container); the binaries
-# land in tests/cpp/_build/ (git-ignored, shipped to the GPU box by gpurun) so that they can be
-# run on a B200:   cd gpurun_out && ../tests/cpp/_build/matrix_mult_benchmark
+# libckks_b200.so.  The reference's sources are not part of this repository: pass a checkout of them
+# as $1 or in CKKS_REFERENCE_DIR.  The binaries land in tests/cpp/_build/ (git-ignored), where the GPU
+# tests run them.
 set -e
 ROOT="$(cd "$(dirname "$0")/../.." && pwd)"
 PKG="$ROOT/seal-fyp-logistic-regression_b200"
-REF="${1:-/root/reference}"
+REF="${1:-$CKKS_REFERENCE_DIR}"
+[ -d "$REF" ] || { echo "usage: $0 REFERENCE_DIR (or set CKKS_REFERENCE_DIR)" >&2; exit 2; }
 OUT="$ROOT/tests/cpp/_build"
 mkdir -p "$OUT"
 for f in 4_ckks matrix_mult_benchmark matrix_multiplication linear_transformation2 linear_transformation polynomial matrix_transpose benchmark logistic_regression_ckks; do

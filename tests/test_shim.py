@@ -1,7 +1,9 @@
 """The C++ drop-in boundary: seal/seal.h over libckks_b200.so.
-CPU: the reference's own hot-path sources compile and link UNCHANGED against the shim (only where
-/root/reference exists -- it does not travel to the GPU box).  GPU: a driver written the way the
-reference writes its programs runs end to end through the shim."""
+CPU: the reference's own hot-path sources compile and link UNCHANGED against the shim.  GPU: a driver written
+the way the reference writes its programs runs end to end through the shim.  The reference's sources are not
+part of this repository: the tests that compile or run them read a checkout of MarwanNour/SEAL-FYP-Logistic-Regression
+named by CKKS_REFERENCE_DIR (build() then also builds the reference programs into tests/cpp/_build/) and skip
+without one."""
 import os
 import subprocess
 
@@ -11,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG_DIR = os.path.join(ROOT, "seal-fyp-logistic-regression_b200")
 LIB = os.path.join(PKG_DIR, "libckks_b200.so")
 INC = ["-I", os.path.join(ROOT, "include"), "-I", os.path.join(PKG_DIR, "include")]
-REF = "/root/reference"
+REF = os.environ.get("CKKS_REFERENCE_DIR", "")
 DRIVER = os.path.join(ROOT, "tests", "cpp", "shim_driver")
 
 HOT_PATH_FILES = ["linear_transformation.cpp", "linear_transformation2.cpp", "polynomial.cpp",
@@ -29,7 +31,7 @@ def build_driver():
     return DRIVER
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources are only present in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="needs CKKS_REFERENCE_DIR: a checkout of the reference's sources")
 @pytest.mark.parametrize("name", HOT_PATH_FILES)
 def test_reference_sources_build_unchanged(pkg, name, tmp_path):
     """`those files link against it unchanged` (BASELINE.json north_star): compile + link, no edits"""
@@ -61,7 +63,7 @@ REF_BUILD = os.path.join(ROOT, "tests", "cpp", "_build")
 def _run_ref(name, cwd, stdin=None, timeout=600):
     exe = os.path.join(REF_BUILD, name)
     if not os.path.exists(exe):
-        pytest.skip("reference binary %s was not prebuilt (needs /root/reference at build time)" % name)
+        pytest.skip("reference binary %s was not prebuilt (build() builds it when CKKS_REFERENCE_DIR names the reference's sources)" % name)
     res = subprocess.run([exe], cwd=cwd, input=stdin, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=timeout)
     assert res.returncode == 0, res.stdout[-2000:]
     return res.stdout
