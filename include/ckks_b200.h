@@ -122,6 +122,12 @@ int ckks_add_plain(ckks_ctx *ctx, const ckks_view *ct, const ckks_view *pt, cons
 /* Evaluator::add_many (helper.h:233,259,276,320): out (batch 1) = sum over the batch of `in`;
  * also the mod-q add that combines all-gathered partial ciphertexts across GPUs */
 int ckks_add_many(ckks_ctx *ctx, const ckks_view *in, const ckks_view *out, ckks_stream s);
+/* out[m] = sum_{g < groups} in[g * out->batch + m]  (mod q_j), for m < out->batch.
+ * in->batch == groups * out->batch; same size / limbs; out must not alias in.  Bit-identical to
+ * ckks_add_many applied to each group.  The reduce-scatter step of sharded workloads (NCCL's sum
+ * is not modular). */
+int ckks_add_many_grouped(ckks_ctx *ctx, const ckks_view *in, int groups, const ckks_view *out,
+                          ckks_stream s);
 /* SEAL's "result ciphertext is transparent" test: *flag_dev (device int32, one per batch entry)
  * is set to 1 when polys 1.. of the entry are all zero */
 int ckks_is_transparent(ckks_ctx *ctx, const ckks_view *ct, int32_t *flag_dev, ckks_stream s);

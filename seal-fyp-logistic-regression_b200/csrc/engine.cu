@@ -557,6 +557,21 @@ extern "C" int ckks_add_many(ckks_ctx *c, const ckks_view *in, const ckks_view *
     return CKKS_OK;
 }
 
+extern "C" int ckks_add_many_grouped(ckks_ctx *c, const ckks_view *in, int groups, const ckks_view *o, ckks_stream s) {
+    int rc;
+    if ((rc = check_view(c, in, "in")) || (rc = check_view(c, o, "out"))) return rc;
+    if (groups < 1) return fail(CKKS_ERR_INVALID, "add_many_grouped: groups must be at least 1");
+    if ((long long)groups * o->batch != in->batch)
+        return fail(CKKS_ERR_INVALID, "add_many_grouped: in batch must be groups x out batch");
+    if (o->size != in->size || o->limbs != in->limbs) return fail(CKKS_ERR_INVALID, "destination parameter mismatch");
+    if (o->data == in->data) return fail(CKKS_ERR_INVALID, "add_many_grouped: out must not alias in");
+    CU(cudaSetDevice(c->device));
+    k_ew_add_many_grouped<<<ew_grid(c, in->size * in->limbs, o->batch), 256, 0, (cudaStream_t)s>>>(
+        dv(in), dv(o), groups, o->batch, in->limbs, c->n, c->t);
+    LAUNCH_CHECK(c);
+    return CKKS_OK;
+}
+
 extern "C" int ckks_is_transparent(ckks_ctx *c, const ckks_view *ct, int32_t *flags, ckks_stream s) {
     int rc;
     if ((rc = check_view(c, ct, "encrypted"))) return rc;

@@ -1416,6 +1416,25 @@ __global__ void __launch_bounds__(256) k_ew_add_many(DView in, DView o, int B, i
     *vpw(o, 0, s, j, n, c) = acc;
 }
 
+// out[m] = in[m] + in[M + m] + ... + in[(G-1) M + m] for m = blockIdx.z: G independent add_many over strided groups
+// (the reduce-scatter sum of sharded workloads).  Lazy 64-bit sum: 8 canonical words of a prime below 2^61 fit, so
+// the running sum is brought back below p after every 7 further terms; one reduction at the end gives the same
+// canonical residue as add_many's sequential modular adds.
+__global__ void __launch_bounds__(256) k_ew_add_many_grouped(DView in, DView o, int G, int M, int L, int n, Tables t) {
+    EW_PROLOGUE(L)
+    const int b = blockIdx.z;
+    ulonglong2 acc = *vp(in, b, s, j, n, c);
+    for (int g = 1; g < G; g++) {
+        ulonglong2 y = *vp(in, g * M + b, s, j, n, c);
+        acc.x += y.x;
+        acc.y += y.y;
+        if (g % 7 == 0) { acc.x = reduce64(acc.x, m); acc.y = reduce64(acc.y, m); }
+    }
+    acc.x = reduce64(acc.x, m);
+    acc.y = reduce64(acc.y, m);
+    *vpw(o, b, s, j, n, c) = acc;
+}
+
 // fused multiply + add_many: out = sum_b a[b] (.) b[b]
 //   PLAIN: b is a plaintext batch (every poly of a[b] times pt[b]), output size = size of a
 //   else : size-2 x size-2 ciphertext products, output size 3 (Linear_Transform_Cipher)

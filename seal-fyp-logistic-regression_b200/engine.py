@@ -262,6 +262,17 @@ class Evaluator:
         out.limbs, out.scale = cts.limbs, cts.scale
         return out
 
+    def add_many_grouped(self, cts, groups, out=None):
+        """batch G*M -> batch M: out[m] = sum_g cts[g*M + m] (mod q), add_many of every strided group in one kernel"""
+        if groups < 1 or cts.batch % groups:
+            raise capi.CkksInvalidArgument("add_many_grouped: in batch must be groups x out batch")
+        out = cts[0:cts.batch // groups].like() if out is None else out
+        out.limbs = cts.limbs
+        vi, vo = cts.view(), out.view()
+        check(self.lib.ckks_add_many_grouped(self.h, C.byref(vi), int(groups), C.byref(vo), _stream()))
+        out.limbs, out.scale = cts.limbs, cts.scale
+        return out
+
     def multiply(self, a, b, out=None):
         """ct x ct; b may be a single ciphertext multiplied into every entry of a"""
         if a.limbs != b.limbs or (a.batch != b.batch and b.batch != 1):

@@ -4,10 +4,14 @@ with no collective in the data path, and the partial ciphertexts are combined wi
 all-gather followed by the mod-q add kernel (NCCL's sum is not modular).  Modular addition is
 associative and commutative, so the combined ciphertext is bit-identical to the sequential
 add_many of the reference (helper.h:259, logistic_regression_ckks.cpp:316)."""
+import math
+
 import torch
 import torch.distributed as dist
 
+from . import capi
 from .engine import Ciphertext
+from .workloads import _stack, duplicate_fill, force_scale_pow2
 
 
 def world():
@@ -137,3 +141,127 @@ def sharded_linear_transform_plain(ev, ct_new_rots_fn, diags_local, d, plans_ste
     rots = ct_new_rots_fn(plans_steps)
     part = ev.multiply_plain_sum(rots, diags_local)
     return combine_partials(ev, part)
+
+
+# ------------------------------------------------------------------ sharded CC_Matrix_Multiplication
+class TorchExchange:
+    """the two collectives of sharded_cc_matrix_multiplication over the default torch.distributed group (NCCL on GPUs).
+    Tests substitute an emulation with the same two methods; every tensor is [batch, ...] and splits count batch entries."""
+
+    def __init__(self):
+        self.rank, self.world = world()
+
+    def all_gather(self, t):
+        """[b, ...] on every rank -> [world * b, ...], rank-major"""
+        if self.world == 1:
+            return t
+        out = torch.empty((self.world * t.shape[0],) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
+        dist.all_gather_into_tensor(out, t.contiguous())
+        return out
+
+    def all_to_all(self, t, send_counts, recv_counts):
+        """block q of `t` (send_counts[q] entries) goes to rank q; the result holds recv_counts[g] entries from each rank g,
+        rank-major"""
+        if self.world == 1:
+            return t
+        out = torch.empty((sum(recv_counts),) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
+        dist.all_to_all_single(out, t.contiguous(), output_split_sizes=list(recv_counts), input_split_sizes=list(send_counts))
+        return out
+
+
+def owned_block(n_units, rank, world_size):
+    """contiguous partition of range(n_units): the first n_units mod G ranks own one unit more.  Contiguous blocks let the
+    reduce-scatter send one slice of the stacked partials to each rank."""
+    base, extra = divmod(n_units, world_size)
+    start = rank * base + min(rank, extra)
+    return range(start, start + base + (1 if rank < extra else 0))
+
+
+def _zeros(ct, size, batch, scale):
+    return Ciphertext(ct.ctx, torch.zeros((batch, size, ct.cap, ct.ctx.n), dtype=torch.int64, device=ct.data.device),
+                      ct.limbs, scale)
+
+
+def _combine(ev, part, exchange):
+    """sum of one batch-1 partial ciphertext over the ranks (mod q), on every rank"""
+    gathered = exchange.all_gather(part.data)
+    return ev.add_many(Ciphertext(part.ctx, gathered, part.limbs, part.scale))
+
+
+def _partial_sparse_transform(ev, rots, s_mine, pos, dset):
+    """this rank's share of linear_transform_plain_sparse: `rots` are the rotations by this rank's steps (`pos`: step ->
+    batch index), `s_mine` their sum.  default (.) (sum_mine rot - sum_{mine & index} rot) + sum_{mine & index} special (.) rot;
+    modular products and sums distribute exactly, so the ranks' partials add up to the unsharded transform word for word."""
+    hit = [i for i, l in enumerate(dset.index) if l in pos]
+    if not hit:
+        return ev.multiply_plain(s_mine, dset.default)
+    dev = rots.data.device
+    sel = Ciphertext(rots.ctx, rots.data.index_select(0, torch.tensor([pos[dset.index[i]] for i in hit], device=dev)),
+                     rots.limbs, rots.scale)
+    sp = dset.special
+    special = Ciphertext(sp.ctx, sp.data.index_select(0, torch.tensor(hit, device=dev)), sp.limbs, sp.scale)
+    rest = ev.sub(s_mine, ev.add_many(sel))
+    return ev.add(ev.multiply_plain(rest, dset.default), ev.multiply_plain_sum(sel, special))
+
+
+def _partial_transforms(ev, X, dsets, mine, keys, plans):
+    """this rank's partials of the transforms `dsets` of X (all sharing the rotations of X + rot(X, -n)) -> one batch"""
+    n = dsets[0].n
+    scale = X.scale * dsets[0].default.scale
+    if not mine:
+        return _zeros(X, 2, len(dsets), scale)
+    rots = ev.rotate_plan(duplicate_fill(ev, X, n, keys), plans.get(mine))
+    s_mine = ev.add_many(rots)
+    pos = {l: i for i, l in enumerate(mine)}
+    return _stack([_partial_sparse_transform(ev, rots, s_mine, pos, ds) for ds in dsets])
+
+
+def _rescaled_pow2_scale(ctx, scale, limbs):
+    """the scale rescale_to_next + force_scale_pow2 give a ciphertext at `limbs` limbs with `scale`"""
+    return float(2.0 ** int(math.log2(scale / float(ctx.primes[limbs - 1]))))
+
+
+def sharded_cc_matrix_multiplication(ev, ctA, ctB, d, sigma, tau, V, W, keys, plans, rank, world_size, exchange):
+    """cc_matrix_multiplication_sparse (CC_Matrix_Multiplication, matrix_mult_benchmark.cpp:13-71) with its d^2 rotations
+    of each transformed ciphertext sharded over `world_size` ranks (SURVEY 8(e)); every rank returns the product,
+    bit-identical to the one-GPU function.  `exchange`: TorchExchange, or a test emulation with its two methods.
+
+    Step 1: each rank rotates dup(ctA) / dup(ctB) by its prefix-aware share of range(d^2) and computes its partial of the
+    sigma / tau transform; all-gather + mod-q add gives A0 and B0 on every rank.
+    Step 2: the same share of the rotations of dup(A0) / dup(B0) gives every rank a partial A_k / B_k for all d-1 k.  Rank r
+    owns the contiguous block K_r of k: one all-to-all sends each block to its owner, ckks_add_many_grouped sums the
+    world_size contributions of every owned k.  The sum is taken before the rescale, which rounds and does not commute
+    with it.
+    Step 3: each rank rescales its A_k / B_k, forces the scales and accumulates sum_{k in K_r} A_k x B_k; all-gather +
+    mod-q add of these size-3 partials, then + mod_switch(A0 x B0)."""
+    dd = d * d
+    mine = shard_rotations_shared(list(range(dd)), rank, world_size)
+    X0 = []
+    for ct, ds in ((ctA, sigma), (ctB, tau)):
+        X0.append(_combine(ev, _partial_transforms(ev, ct, [ds], mine, keys, plans), exchange))
+    A0, B0 = X0
+
+    counts = [len(owned_block(d - 1, q, world_size)) for q in range(world_size)]
+    own = counts[rank]
+    XK = []
+    for X, dsets in ((A0, V), (B0, W)):
+        part = _partial_transforms(ev, X, dsets, mine, keys, plans)
+        recv = exchange.all_to_all(part.data, counts, [own] * world_size)
+        XK.append(ev.add_many_grouped(Ciphertext(part.ctx, recv, part.limbs, part.scale), world_size) if own else part)
+    Ak, Bk = XK
+
+    ctAB = ev.multiply(A0, B0)
+    ev.mod_switch_to_next_inplace(ctAB)
+    if own:
+        for X in (Ak, Bk):
+            ev.rescale_to_next_inplace(X)
+            force_scale_pow2(X)
+        rest = ev.multiply_sum(Ak, Bk)
+    else:                                   # more ranks than products: this rank adds zero
+        scale = (_rescaled_pow2_scale(A0.ctx, Ak.scale, Ak.limbs) * _rescaled_pow2_scale(B0.ctx, Bk.scale, Bk.limbs))
+        rest = _zeros(Ak, 3, 1, scale)
+        rest.limbs = Ak.limbs - 1
+    rest = _combine(ev, rest, exchange)
+    if rest.scale != ctAB.scale:
+        raise capi.CkksInvalidArgument("scale mismatch")
+    return ev.add(ctAB, rest)
