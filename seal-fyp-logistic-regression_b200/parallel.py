@@ -6,12 +6,14 @@ associative and commutative, so the combined ciphertext is bit-identical to the 
 add_many of the reference (helper.h:259, logistic_regression_ckks.cpp:316)."""
 import math
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
 from . import capi
 from .engine import Ciphertext
-from .workloads import _stack, duplicate_fill, force_scale_pow2
+from .lr import _poly, apply_gradient, folded_coeffs
+from .workloads import _stack, cipher_dot_product, duplicate_fill, force_scale_pow2
 
 
 def world():
@@ -145,8 +147,8 @@ def sharded_linear_transform_plain(ev, ct_new_rots_fn, diags_local, d, plans_ste
 
 # ------------------------------------------------------------------ sharded CC_Matrix_Multiplication
 class TorchExchange:
-    """the two collectives of sharded_cc_matrix_multiplication over the default torch.distributed group (NCCL on GPUs).
-    Tests substitute an emulation with the same two methods; every tensor is [batch, ...] and splits count batch entries."""
+    """the collectives of the sharded workloads over the default torch.distributed group (NCCL on GPUs).  Tests substitute
+    an emulation with the same methods; every tensor is [batch, ...] and splits count batch entries."""
 
     def __init__(self):
         self.rank, self.world = world()
@@ -167,6 +169,13 @@ class TorchExchange:
         out = torch.empty((sum(recv_counts),) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
         dist.all_to_all_single(out, t.contiguous(), output_split_sizes=list(recv_counts), input_split_sizes=list(send_counts))
         return out
+
+    def broadcast(self, t, src=0):
+        """rank src's `t` on every rank; the other ranks pass a contiguous tensor of the same shape and dtype to receive into"""
+        if self.world == 1:
+            return t
+        dist.broadcast(t, src)
+        return t
 
 
 def owned_block(n_units, rank, world_size):
@@ -265,3 +274,133 @@ def sharded_cc_matrix_multiplication(ev, ctA, ctB, d, sigma, tau, V, W, keys, pl
     if rest.scale != ctAB.scale:
         raise capi.CkksInvalidArgument("scale mismatch")
     return ev.add(ctAB, rest)
+
+
+# ------------------------------------------------------------------ sharded config-1 training iteration
+def config1_shards(R, C, rank, world_size):
+    """this rank's contiguous block of the R sample rows (prediction) and of the C feature columns (gradient).  Every row
+    and every feature belongs to exactly one rank; with more ranks than features (or rows) the last ranks own none."""
+    return owned_block(R, rank, world_size), owned_block(C, rank, world_size)
+
+
+def config1_keyswitches(R, C, rank, world_size, degree=3):
+    """key switches of this rank in one sharded_update_weights with the Horner polynomial (rank 0 evaluates it): per own
+    row 1 relinearisation + rotate_vector(-C) + C - 1 chain steps, per own feature 1 + rotate_vector(-R) + R - 1; a
+    rotation by a step without its own Galois key costs the NAF weight of the step (power-of-two keys)"""
+    rows, feats = config1_shards(R, C, rank, world_size)
+    return (len(rows) * (1 + naf_weight(C) + C - 1) + (degree if rank == 0 else 0)
+            + len(feats) * (1 + naf_weight(R) + R - 1))
+
+
+def _one_hot(ids, width):
+    m = np.zeros((len(ids), width))
+    m[np.arange(len(ids)), list(ids)] = 1.0
+    return m
+
+
+def _active(ct):
+    """`ct` with its buffer cut to the active limbs: what an exchange has to move"""
+    if ct.cap == ct.limbs:
+        return ct
+    return Ciphertext(ct.ctx, ct.data[:, :, : ct.limbs].contiguous(), ct.limbs, ct.scale)
+
+
+def _zero_partial(ctx, limbs, scale):
+    return Ciphertext(ctx, torch.zeros((1, 2, limbs, ctx.n), dtype=torch.int64, device=ctx.device), limbs, scale)
+
+
+def _broadcast_ct(ctx, ct, rank, exchange):
+    """rank 0's ciphertext `ct` on every rank (the other ranks pass None): shape, level and scale first (exact in
+    float64), then the active limbs"""
+    head = torch.zeros(4, dtype=torch.float64, device=ctx.device)
+    if rank == 0:
+        ct = _active(ct)
+        head = torch.tensor([ct.batch, ct.size, ct.limbs, ct.scale], dtype=torch.float64, device=ctx.device)
+    batch, size, limbs, scale = exchange.broadcast(head).tolist()
+    batch, size, limbs = int(batch), int(size), int(limbs)
+    data = ct.data if rank == 0 else torch.empty((batch, size, limbs, ctx.n), dtype=torch.int64, device=ctx.device)
+    return Ciphertext(ctx, exchange.broadcast(data), limbs, scale)
+
+
+def sharded_update_weights(ev, rows_local, row_ids, cols_local, feature_ids, labels, weights, lr, R, C, scale, keys,
+                           encoder, encryptor, rank, world_size, exchange, degree=3, method="horner", mark=None):
+    """lr.update_weights (logistic_regression_ckks.cpp:269-345, config 1) with its R row dot products and its C feature
+    dot products sharded over `world_size` ranks; every rank returns the new-weights ciphertext, bit-identical to the
+    one-GPU function on the full inputs.
+
+    rows_local / row_ids: this rank's row ciphertexts and their row indices, cols_local / feature_ids: its feature-column
+    ciphertexts and their feature indices (config1_shards; either may be an empty batch, which still carries level and
+    scale).  labels and weights are replicated.  `exchange`: TorchExchange, or a test emulation with its all_gather and
+    broadcast.  `encryptor`: rank 0's, which makes exactly the calls of the one-GPU function (the polynomial encrypts its
+    top coefficient); the other ranks pass None.  `mark(name)`, when given, is called as each phase ends.
+
+    Prediction: cipher_dot_product of the own rows with the weights, the one-hot masks e_i of the own rows only, fused
+    multiply_plain_sum; all-gather + mod-q add of the partials BEFORE relinearize / rescale (the rescale rounds and does
+    not commute with the sum).  Rank 0 rescales, evaluates the sigmoid polynomial, subtracts the labels and broadcasts
+    pred - labels.  Gradient: cipher_dot_product of the own feature columns with pred - labels (R - 1 dependent unit
+    rotations each; a chain cannot be split without changing the ciphertext, so this phase shards at most C ways), masks
+    e_j, multiply_plain_sum, all-gather + mod-q add before the rescale; the learning-rate tail runs on every rank."""
+    if not 0 <= rank < world_size or rows_local.batch != len(row_ids) or cols_local.batch != len(feature_ids):
+        raise ValueError("sharded_update_weights: rank or shard sizes do not match")
+    mark = mark or (lambda name: None)
+    ctx = weights.ctx
+    if rows_local.batch:
+        results = cipher_dot_product(ev, rows_local, weights, C, keys)
+        mask_pt = encoder.encode(_one_hot(row_ids, R), scale)
+        ev.mod_switch_to_next_inplace(mask_pt)
+        part = ev.multiply_plain_sum(results, mask_pt)
+    else:
+        part = _zero_partial(ctx, weights.limbs - 1,
+                             _rescaled_pow2_scale(ctx, rows_local.scale * weights.scale, weights.limbs) * scale)
+    mark("prediction")
+    lin = _combine(ev, _active(part), exchange)
+    mark("combine_prediction")
+    pred_labels = None
+    if rank == 0:
+        lin = ev.relinearize(lin, keys)
+        ev.rescale_to_next_inplace(lin)
+        force_scale_pow2(lin)
+        pred = _poly(method)(ev, lin, folded_coeffs(degree), scale, keys, encoder, encryptor)
+        lab = ev.mod_switch_to(labels, pred.limbs)
+        if lab.scale != pred.scale:
+            pred.scale = lab.scale
+        pred_labels = ev.sub(pred, lab)
+    pred_labels = _broadcast_ct(ctx, pred_labels, rank, exchange)
+    mark("polynomial_broadcast")
+    cols = ev.mod_switch_to(cols_local, pred_labels.limbs)
+    if cols.batch:
+        grads = cipher_dot_product(ev, cols, pred_labels, R, keys)
+        mask_pt = encoder.encode(_one_hot(feature_ids, C), scale, limbs=grads.limbs)
+        part = ev.multiply_plain_sum(grads, mask_pt)
+    else:
+        part = _zero_partial(ctx, pred_labels.limbs - 1,
+                             _rescaled_pow2_scale(ctx, cols.scale * pred_labels.scale, pred_labels.limbs) * scale)
+    mark("gradient")
+    gradient = _combine(ev, _active(part), exchange)
+    mark("combine_gradient")
+    gradient = ev.relinearize(gradient, keys)
+    ev.rescale_to_next_inplace(gradient)
+    force_scale_pow2(gradient)
+    new_weights = apply_gradient(ev, gradient, weights, lr, R, scale, encoder)
+    mark("tail")
+    return new_weights
+
+
+def sharded_train_cipher(ev, rows_local, row_ids, cols_local, feature_ids, labels, weights, lr, iters, layout, scale, keys,
+                         encoder, encryptor, decryptor, rank, world_size, exchange, degree=3, method="horner"):
+    """lr.train_cipher (logistic_regression_ckks.cpp:348-385, repair R4) over sharded_update_weights: after every
+    iteration rank 0, the key holder (only it has a `decryptor` and an `encryptor`), decrypts and decodes the weights,
+    re-packs them (RowLayout.weights), encodes them at the top level, re-encrypts them and broadcasts the ciphertext.
+    Rank 0's encryptor sees the calls of the one-GPU train_cipher in the same order, so with the same seeds every rank
+    returns a ciphertext bit-identical to it."""
+    new_weights = weights
+    for _ in range(iters):
+        new_weights = sharded_update_weights(ev, rows_local, row_ids, cols_local, feature_ids, labels, new_weights, lr,
+                                             layout.R, layout.C, scale, keys, encoder, encryptor, rank, world_size, exchange,
+                                             degree=degree, method=method)
+        fresh = None
+        if rank == 0:
+            decoded = encoder.decode(decryptor.decrypt(new_weights))[0, : layout.C]
+            fresh = encryptor.encrypt(encoder.encode(layout.weights(decoded), scale))
+        new_weights = _broadcast_ct(weights.ctx, fresh, rank, exchange)
+    return new_weights
