@@ -128,6 +128,18 @@ int ckks_add_many(ckks_ctx *ctx, const ckks_view *in, const ckks_view *out, ckks
  * is not modular). */
 int ckks_add_many_grouped(ckks_ctx *ctx, const ckks_view *in, int groups, const ckks_view *out,
                           ckks_stream s);
+/* Constant-coefficient sums, e.g. the baby-step sums of a polynomial in the Chebyshev basis:
+ *   out[g * M + m] = sum_{i < terms} in[i * M + m] (.) const(coeffs[g * terms + i], scales[g * terms + i])
+ *                    (+ const(const_coeffs[g], const_scales[g]) added to poly 0)
+ * for g < groups, m < M = in->batch / terms; out->batch == groups * M.  const(c, s) is the constant
+ * plaintext ckks_encode_scalar(c, s) writes (residues of nearbyint(c * s)), so the result is
+ * bit-identical to multiply_plain by each such plaintext, add_many, add_plain.  Terms whose residues
+ * are zero are skipped; every input word is read once for all groups.  const_coeffs / const_scales
+ * may both be NULL (no constant).  CKKS_ERR_INVALID: bad shapes, terms or groups < 1,
+ * (terms + 1) * limbs > 2048, out overlapping in, a scale <= 0 or a non-finite c * s. */
+int ckks_multiply_const_sum(ckks_ctx *ctx, const ckks_view *in, int terms, int groups,
+                            const double *coeffs, const double *scales, const double *const_coeffs,
+                            const double *const_scales, const ckks_view *out, ckks_stream s);
 /* SEAL's "result ciphertext is transparent" test: *flag_dev (device int32, one per batch entry)
  * is set to 1 when polys 1.. of the entry are all zero */
 int ckks_is_transparent(ckks_ctx *ctx, const ckks_view *ct, int32_t *flag_dev, ckks_stream s);

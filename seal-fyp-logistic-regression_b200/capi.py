@@ -68,6 +68,8 @@ SIGNATURES = {
     "ckks_add_plain": (C.c_int, [C.c_void_p, _VP, _VP, _VP, C.c_void_p]),
     "ckks_add_many": (C.c_int, [C.c_void_p, _VP, _VP, C.c_void_p]),
     "ckks_add_many_grouped": (C.c_int, [C.c_void_p, _VP, C.c_int, _VP, C.c_void_p]),
+    "ckks_multiply_const_sum": (C.c_int, [C.c_void_p, _VP, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          _VP, C.c_void_p]),
     "ckks_is_transparent": (C.c_int, [C.c_void_p, _VP, C.c_void_p, C.c_void_p]),
     "ckks_ksk_words": (C.c_size_t, [C.c_void_p]),
     "ckks_relinearize": (C.c_int, [C.c_void_p, _VP, C.c_void_p, _VP, C.c_void_p]),

@@ -5,6 +5,7 @@
 // and nothing falls back to the CPU.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstdlib>
 #include <cstdio>
@@ -1578,6 +1579,69 @@ extern "C" int ckks_encode_scalar(ckks_ctx *c, double value, double scale, const
     for (int l = 0; l < out->limbs; l++) cr.r[l] = host_residue(r, c->primes[l]);
     k_enc_fill<<<dim3((c->n + 255) / 256, out->limbs, out->batch), 256, 0, (cudaStream_t)s>>>(dv(out), cr, c->n);
     LAUNCH_CHECK(c);
+    return CKKS_OK;
+}
+
+// ------------------------------------------------------------------------------------ constant-coefficient sums
+// words from the first to one past the last active word of a view
+static size_t view_words(const ckks_view *v, int n) {
+    return (size_t)(v->batch - 1) * v->batch_stride + (size_t)(v->size - 1) * v->poly_stride + (size_t)v->limbs * n;
+}
+
+extern "C" int ckks_multiply_const_sum(ckks_ctx *c, const ckks_view *in, int terms, int groups, const double *coeffs,
+                                       const double *scales, const double *const_coeffs, const double *const_scales,
+                                       const ckks_view *out, ckks_stream s) {
+    int rc;
+    if ((rc = check_view(c, in, "in")) || (rc = check_view(c, out, "out"))) return rc;
+    if (terms < 1 || groups < 1) return fail(CKKS_ERR_INVALID, "multiply_const_sum: terms and groups must be at least 1");
+    if (in->batch % terms) return fail(CKKS_ERR_INVALID, "multiply_const_sum: in batch must be terms x out batch / groups");
+    const int M = in->batch / terms;
+    if ((long long)groups * M != out->batch)
+        return fail(CKKS_ERR_INVALID, "multiply_const_sum: out batch must be groups x in batch / terms");
+    if (out->size != in->size || out->limbs != in->limbs) return fail(CKKS_ERR_INVALID, "destination parameter mismatch");
+    if (in->batch > 1 && in->batch_stride == 0) return fail(CKKS_ERR_INVALID, "multiply_const_sum: in entries must be distinct");
+    if (out->batch > 1 && out->batch_stride == 0) return fail(CKKS_ERR_INVALID, "multiply_const_sum: out entries must be distinct");
+    const uint64_t *ib = (const uint64_t *)in->data, *ob = (const uint64_t *)out->data;
+    if (ob < ib + view_words(in, c->n) && ib < ob + view_words(out, c->n))
+        return fail(CKKS_ERR_INVALID, "multiply_const_sum: out must not alias in");
+    if (!coeffs || !scales) return fail(CKKS_ERR_INVALID, "multiply_const_sum: null coefficients");
+    if (!const_coeffs != !const_scales) return fail(CKKS_ERR_INVALID, "multiply_const_sum: constant values and scales go together");
+    const int L = in->limbs;
+    // the same checks and residues as ckks_encode_scalar(value, scale) for every constant
+    auto residues = [&](double value, double scale, u64 *r) {
+        if (!(scale > 0.0)) return fail(CKKS_ERR_INVALID, "scale out of bounds");
+        const double v = nearbyint(value * scale);
+        if (!std::isfinite(v)) return fail(CKKS_ERR_INVALID, "multiply_const_sum: constant times scale is not finite");
+        for (int l = 0; l < L; l++) r[l] = host_residue(v, c->primes[l]);
+        return (int)CKKS_OK;
+    };
+    const size_t per_group = (size_t)(terms + 1) * L;
+    if (per_group > CONST_SUM_WORDS) return fail(CKKS_ERR_INVALID, "multiply_const_sum: (terms + 1) x limbs exceeds 2048");
+    const int chunk = (int)std::min<size_t>(CONST_SUM_GROUPS, CONST_SUM_WORDS / per_group);
+    std::vector<ConstSumTable> tabs((groups + chunk - 1) / chunk);
+    for (int g0 = 0, k = 0; g0 < groups; g0 += chunk, k++) {
+        const int G = std::min(chunk, groups - g0);
+        u64 *r = tabs[k].r, *r0 = r + (size_t)G * terms * L;
+        for (int g = 0; g < G; g++) {
+            for (int i = 0; i < terms; i++) {
+                const size_t q = (size_t)(g0 + g) * terms + i;
+                if ((rc = residues(coeffs[q], scales[q], r + ((size_t)g * terms + i) * L))) return rc;
+            }
+            if (const_coeffs) {
+                if ((rc = residues(const_coeffs[g0 + g], const_scales[g0 + g], r0 + (size_t)g * L))) return rc;
+            } else {
+                for (int l = 0; l < L; l++) r0[(size_t)g * L + l] = 0;
+            }
+        }
+    }
+    CU(cudaSetDevice(c->device));
+    for (int g0 = 0, k = 0; g0 < groups; g0 += chunk, k++) {
+        const int G = std::min(chunk, groups - g0);
+        DView o = dv(out);
+        o.data += (size_t)g0 * M * out->batch_stride;
+        k_ew_const_sum<<<ew_grid(c, in->size * L, M), 256, 0, (cudaStream_t)s>>>(dv(in), o, tabs[k], G, terms, M, L, c->n, c->t);
+        LAUNCH_CHECK(c);
+    }
     return CKKS_OK;
 }
 

@@ -1532,6 +1532,94 @@ __global__ void __launch_bounds__(256) k_ew_mul_sum(DView a, DView b, DView o, i
     }
 }
 
+// constant-coefficient sums (ckks_multiply_const_sum).  The residues of the encoded constants are computed on the host
+// (as ckks_encode_scalar does) and travel in the kernel parameters: words [g][i][j] of the G x T term constants of the
+// launch, then [g][j] of the G constants added to poly 0.
+#define CONST_SUM_WORDS 2048
+#define CONST_SUM_GROUPS 8
+struct ConstSumTable {
+    u64 r[CONST_SUM_WORDS];
+};
+// out[g * M + m] = sum_{i < T} in[i * M + m] (.) r[g][i]  (+ r0[g] on poly 0), for g < G <= CONST_SUM_GROUPS, m = blockIdx.z.
+// Every input word is read once for all G outputs; a term whose residue is zero on this limb is not read.  The products
+// are summed lazily (FP64 below 2^41, 128-bit otherwise, as k_ew_mul_sum) and reduced once: the canonical result equals
+// SEAL's multiply_plain by each constant plaintext, add_many, add_plain.
+__global__ void __launch_bounds__(256) k_ew_const_sum(DView in, DView o, const __grid_constant__ ConstSumTable tab, int G,
+                                                      int T, int M, int L, int n, Tables t) {
+    EW_PROLOGUE(L)
+    const int b = blockIdx.z;
+    const u64 *r = tab.r, *r0 = tab.r + (size_t)G * T * L;
+    const FpConst f = t.fp[j];
+    if (f.ok != 0.0) {
+        double s0[CONST_SUM_GROUPS], s1[CONST_SUM_GROUPS];
+#pragma unroll
+        for (int g = 0; g < CONST_SUM_GROUPS; g++) s0[g] = s1[g] = 0.0;
+        for (int i = 0; i < T; i++) {
+            bool any = false;
+            for (int g = 0; g < G; g++) any |= r[(g * T + i) * L + j] != 0;
+            if (!any) continue;
+            const ulonglong2 x = *vp(in, i * M + b, s, j, n, c);
+            const double xx = fp_from_u64(x.x), xy = fp_from_u64(x.y);
+#pragma unroll
+            for (int g = 0; g < CONST_SUM_GROUPS; g++) {
+                if (g >= G) break;
+                const u64 w = r[(g * T + i) * L + j];
+                if (!w) continue;
+                const double wd = fp_from_u64(w);
+                s0[g] = __dadd_rn(s0[g], fp_mulmod(xx, wd, f));
+                s1[g] = __dadd_rn(s1[g], fp_mulmod(xy, wd, f));
+            }
+            if ((i & 255) == 255) {   // |term| < 2p: 256 of them stay below 2^50
+#pragma unroll
+                for (int g = 0; g < CONST_SUM_GROUPS; g++) { s0[g] = fp_reduce(s0[g], f); s1[g] = fp_reduce(s1[g], f); }
+            }
+        }
+#pragma unroll
+        for (int g = 0; g < CONST_SUM_GROUPS; g++) {
+            if (g >= G) break;
+            ulonglong2 v;
+            v.x = fp_to_canonical(s0[g], f);
+            v.y = fp_to_canonical(s1[g], f);
+            if (s == 0) { v.x = addmod(v.x, r0[g * L + j], m.p); v.y = addmod(v.y, r0[g * L + j], m.p); }
+            *vpw(o, g * M + b, s, j, n, c) = v;
+        }
+        return;
+    }
+    u64 lo0[CONST_SUM_GROUPS], hi0[CONST_SUM_GROUPS], lo1[CONST_SUM_GROUPS], hi1[CONST_SUM_GROUPS];
+#pragma unroll
+    for (int g = 0; g < CONST_SUM_GROUPS; g++) lo0[g] = hi0[g] = lo1[g] = hi1[g] = 0;
+    for (int i = 0; i < T; i++) {
+        bool any = false;
+        for (int g = 0; g < G; g++) any |= r[(g * T + i) * L + j] != 0;
+        if (!any) continue;
+        const ulonglong2 x = *vp(in, i * M + b, s, j, n, c);
+#pragma unroll
+        for (int g = 0; g < CONST_SUM_GROUPS; g++) {
+            if (g >= G) break;
+            const u64 w = r[(g * T + i) * L + j];
+            if (!w) continue;
+            mac128(lo0[g], hi0[g], x.x, w);
+            mac128(lo1[g], hi1[g], x.y, w);
+        }
+        if ((i & 15) == 15) {   // 16 products of residues below 2^61 fit in 128 bits
+#pragma unroll
+            for (int g = 0; g < CONST_SUM_GROUPS; g++) {
+                lo0[g] = barrett128(lo0[g], hi0[g], m); hi0[g] = 0;
+                lo1[g] = barrett128(lo1[g], hi1[g], m); hi1[g] = 0;
+            }
+        }
+    }
+#pragma unroll
+    for (int g = 0; g < CONST_SUM_GROUPS; g++) {
+        if (g >= G) break;
+        ulonglong2 v;
+        v.x = barrett128(lo0[g], hi0[g], m);
+        v.y = barrett128(lo1[g], hi1[g], m);
+        if (s == 0) { v.x = addmod(v.x, r0[g * L + j], m.p); v.y = addmod(v.y, r0[g * L + j], m.p); }
+        *vpw(o, g * M + b, s, j, n, c) = v;
+    }
+}
+
 // strided limb copy (mod-switch drop into a differently laid out view)
 __global__ void __launch_bounds__(256) k_ew_copy(DView a, DView o, int L, int n) {
     const int s = blockIdx.y / L, j = blockIdx.y % L;

@@ -273,6 +273,64 @@ class Evaluator:
         out.limbs, out.scale = cts.limbs, cts.scale
         return out
 
+    def multiply_const_sum(self, cts, coeffs, pt_scales, constant=None, groups=1, out=None):
+        """Constant-coefficient sums of T terms for `groups` sets of coefficients, in one kernel:
+            out[g*M + m] = sum_i cts_i[m] * coeffs[g][i]  (+ constant[g])
+        bit-identical to SEAL's multiply_plain(cts_i, encode(coeffs[g][i], pt_scales[g][i])), add_many and
+        add_plain(encode(constant[g], result scale)).
+
+        cts       : a list of T Ciphertexts of batch M (each with its own scale), or one Ciphertext whose batch is T*M
+                    (entry i*M + m is term i of sum m)
+        coeffs    : [groups][T] (or [T] when groups == 1)
+        pt_scales : the scale each coefficient is encoded at: a number, [T] (every group) or [groups][T]
+        constant  : None or [groups] values added to poly 0, encoded at the result scale
+        As SEAL's add requires, every term's ct.scale * pt_scale must be the same number, which is the result's scale
+        ("scale mismatch" otherwise); "scale out of bounds" as multiply_plain.  Returns a Ciphertext of batch groups * M."""
+        if isinstance(cts, Ciphertext):
+            cts = [cts]
+        cts = list(cts)
+        coeffs = np.asarray(coeffs, dtype=np.float64).reshape(groups, -1)
+        T = coeffs.shape[1] if len(cts) == 1 else len(cts)
+        if len(cts) == 1 and cts[0].batch % T:
+            raise capi.CkksInvalidArgument("multiply_const_sum: in batch must be terms x out batch / groups")
+        if coeffs.shape[1] != T:
+            raise capi.CkksInvalidArgument("multiply_const_sum: coeffs must have groups x terms entries")
+        first = cts[0]
+        for c in cts[1:]:
+            if c.limbs != first.limbs or c.batch != first.batch or c.size != first.size:
+                raise capi.CkksInvalidArgument("encrypted1 and encrypted2 parameter mismatch")
+        pt = np.broadcast_to(np.asarray(pt_scales, dtype=np.float64), (groups, T))
+        ct_scales = [c.scale for c in cts] if len(cts) == T else [first.scale] * T
+        scale = ct_scales[0] * float(pt[0, 0])
+        for g in range(groups):
+            for i in range(T):
+                if ct_scales[i] * float(pt[g, i]) != scale:
+                    raise capi.CkksInvalidArgument("scale mismatch")
+        self._scale_ok(scale, first.limbs)
+        if len(cts) == 1:
+            src = first
+        else:   # one [T*M] input: the terms side by side (active limbs only)
+            L = first.limbs
+            src = Ciphertext(first.ctx, torch.cat([c.data[:, :, :L] for c in cts], dim=0), L, first.scale)
+        M = src.batch // T
+        if out is None:
+            out = Ciphertext(self.ctx, torch.empty((groups * M, src.size, src.cap, self.ctx.n), dtype=torch.int64,
+                                                   device=src.data.device), src.limbs, scale)
+        out.limbs = src.limbs
+        cf = np.ascontiguousarray(coeffs)
+        ps = np.ascontiguousarray(pt)
+        if constant is not None:
+            k0 = np.ascontiguousarray(np.asarray(constant, dtype=np.float64).reshape(groups))
+            s0 = np.full(groups, scale)
+            k0p, s0p = k0.ctypes.data, s0.ctypes.data
+        else:
+            k0p = s0p = None
+        vi, vo = src.view(), out.view()
+        check(self.lib.ckks_multiply_const_sum(self.h, C.byref(vi), int(T), int(groups), cf.ctypes.data, ps.ctypes.data,
+                                               k0p, s0p, C.byref(vo), _stream()))
+        out.scale = scale
+        return out
+
     def multiply(self, a, b, out=None):
         """ct x ct; b may be a single ciphertext multiplied into every entry of a"""
         if a.limbs != b.limbs or (a.batch != b.batch and b.batch != 1):

@@ -16,6 +16,12 @@ level bookkeeping, never the evaluator op sequence of an individual ciphertext:
   R5  standardised features are the ones encrypted (:570 vs :582-590);
   R6  the 1/8 input scaling of the sigmoid approximation is folded into the coefficients.
 
+method="chebyshev" (opt-in, not the reference's) replaces the degree-3 polynomial, which is fitted on [-8, 8] while the
+pulsar data reach |x.w| = 38, by the Chebyshev interpolant of the sigmoid on [-B, B] (ChebyshevSigmoid, default degree 63,
+B = 48) evaluated by workloads.chebyshev_cipher with exact scales.  The 1/B input scaling is folded into the one-hot
+prediction masks (e_i / B), so it costs no level; the polynomial takes chebyshev_depth(63) = 7 levels, so config 1 needs
+{60, 40 x 12, 60}.
+
 Two layouts:
   * `RowLayout`     -- the reference's: one ciphertext per sample row for the prediction and one per
                        feature column for the gradient (config 1, R + C <= N/2 slots).
@@ -31,7 +37,8 @@ import numpy as np
 import torch
 
 from .engine import Ciphertext
-from .workloads import cipher_dot_product, force_scale_pow2, horner_cipher, tree_cipher
+from .workloads import (chebyshev_cipher, chebyshev_interpolant, cipher_dot_product, force_scale_pow2, horner_cipher,
+                        tree_cipher)
 
 # logistic_regression_ckks.cpp:247,251,255 (zero coefficients are written 0.00001 there because
 # Tree_cipher dereferences every coefficient plaintext)
@@ -52,11 +59,31 @@ def sigmoid_approx(x, degree):
     return sum(c * x ** i for i, c in enumerate(folded_coeffs(degree)))
 
 
-def plain_epoch(X, y, w, lr, degree):
+class ChebyshevSigmoid:
+    """the sigmoid as sum c_i T_i(x / bound): its Chebyshev interpolant of `degree` on [-bound, bound].  Degree 63 on
+    [-48, 48] is within 1e-2 of the sigmoid there (largest at the steep centre) and its coefficients are bounded
+    (sum |c_i| < 2): monomial coefficients of the same fit would be ~48^-63 and vanish at scale 2^40."""
+
+    def __init__(self, degree=63, bound=48.0):
+        self.degree, self.bound = int(degree), float(bound)
+        self.coeffs = chebyshev_interpolant(lambda x: 1.0 / (1.0 + np.exp(-x)), self.bound, self.degree)
+
+    def __call__(self, x):
+        return np.polynomial.chebyshev.chebval(np.asarray(x) / self.bound, self.coeffs)
+
+
+SIGMOID_CHEBYSHEV = ChebyshevSigmoid()
+
+
+def plain_epoch(X, y, w, lr, degree=3, method="horner", sigmoid=None):
     """plaintext semantics of one update_weights (logistic_regression.cpp:136-178 with the
-    polynomial sigmoid): w - lr/R * X^T (sigma(Xw) - y)"""
+    polynomial sigmoid): w - lr/R * X^T (sigma(Xw) - y).  method="chebyshev": sigma is `sigmoid`
+    (a ChebyshevSigmoid, default SIGMOID_CHEBYSHEV) and `degree` is not used."""
     R = X.shape[0]
-    p = sigmoid_approx(X @ w, degree)
+    if method == "chebyshev":
+        p = (sigmoid or SIGMOID_CHEBYSHEV)(X @ w)
+    else:
+        p = sigmoid_approx(X @ w, degree)
     return w - (lr / R) * (X.T @ (p - y))
 
 
@@ -67,7 +94,24 @@ def _bcast(ct, batch):
 
 
 def _poly(method):
+    if method == "chebyshev":
+        raise ValueError("method='chebyshev' is implemented for the row layout (predict_cipher_weights) only")
     return tree_cipher if method == "tree" else horner_cipher
+
+
+def prediction_masks(masks, method, sigmoid):
+    """the one-hot prediction masks, divided by the sigmoid's bound for method="chebyshev" (the polynomial's input is
+    x.w / B; folding 1/B into the mask costs no level)"""
+    return masks / (sigmoid or SIGMOID_CHEBYSHEV).bound if method == "chebyshev" else masks
+
+
+def sigmoid_cipher(ev, lin, scale, keys, encoder, encryptor, degree, method, sigmoid):
+    """the sigmoid polynomial of the prediction: the reference's (forced power-of-two scale on its input, then
+    Horner_cipher / Tree_cipher) or, for method="chebyshev", chebyshev_cipher with exact scales, landing on `scale`"""
+    if method == "chebyshev":
+        return chebyshev_cipher(ev, lin, (sigmoid or SIGMOID_CHEBYSHEV).coeffs, keys, scale=scale)
+    force_scale_pow2(lin)
+    return _poly(method)(ev, lin, folded_coeffs(degree), scale, keys, encoder, encryptor)
 
 
 class RowLayout:
@@ -102,29 +146,30 @@ class RowLayout:
         return out
 
 
-def predict_cipher_weights(ev, features, weights, C, scale, keys, encoder, encryptor, degree=3, method="horner"):
+def predict_cipher_weights(ev, features, weights, C, scale, keys, encoder, encryptor, degree=3, method="horner",
+                           sigmoid=None):
     """predict_cipher_weights (logistic_regression_ckks.cpp:208-266): per-row dot product with the
     weights, one-hot mask at slot i, add_many, rescale, sigmoid polynomial.  `features`: batch of R
-    row ciphertexts; `weights`: one ciphertext."""
+    row ciphertexts; `weights`: one ciphertext.  method="chebyshev": masks e_i / B and the
+    ChebyshevSigmoid `sigmoid` (no encryptor needed)."""
     R = features.batch
     results = cipher_dot_product(ev, features, weights, C, keys)          # hot loop 1, batched over rows
     masks = np.zeros((R, R))
     masks[np.arange(R), np.arange(R)] = 1.0
-    mask_pt = encoder.encode(masks, scale)
+    mask_pt = encoder.encode(prediction_masks(masks, method, sigmoid), scale)
     ev.mod_switch_to_next_inplace(mask_pt)                                # :227
     ev.multiply_plain_inplace(results, mask_pt)
     lin = ev.add_many(results)
     lin = ev.relinearize(lin, keys)                                       # no-op on size 2 (:236)
     ev.rescale_to_next_inplace(lin)
-    force_scale_pow2(lin)
-    return _poly(method)(ev, lin, folded_coeffs(degree), scale, keys, encoder, encryptor)
+    return sigmoid_cipher(ev, lin, scale, keys, encoder, encryptor, degree, method, sigmoid)
 
 
 def update_weights(ev, features, features_T, labels, weights, lr, scale, keys, encoder, encryptor,
-                   degree=3, method="horner"):
+                   degree=3, method="horner", sigmoid=None):
     """update_weights (logistic_regression_ckks.cpp:269-345) with repairs R3"""
     R, C = features.batch, features_T.batch
-    pred = predict_cipher_weights(ev, features, weights, C, scale, keys, encoder, encryptor, degree, method)
+    pred = predict_cipher_weights(ev, features, weights, C, scale, keys, encoder, encryptor, degree, method, sigmoid)
     lab = ev.mod_switch_to(labels, pred.limbs)                            # :286
     if lab.scale != pred.scale:
         pred.scale = lab.scale                                            # both are 2^40 after the forced scales
@@ -150,7 +195,7 @@ def update_weights(ev, features, features_T, labels, weights, lr, scale, keys, e
 
 
 def train_cipher(ev, features, features_T, labels, weights, lr, iters, layout, scale, keys, encoder, encryptor, decryptor,
-                 degree=3, method="horner"):
+                 degree=3, method="horner", sigmoid=None):
     """train_cipher (logistic_regression_ckks.cpp:348-385): `iters` x (update_weights, then the key holder
     decrypts, decodes and re-encrypts the weights).  Repair R4: the decoded weights are re-packed
     (RowLayout.weights) and encoded at the top level -- the reference re-encrypts the exhausted low-level
@@ -158,7 +203,7 @@ def train_cipher(ev, features, features_T, labels, weights, lr, iters, layout, s
     new_weights = weights
     for _ in range(iters):
         new_weights = update_weights(ev, features, features_T, labels, new_weights, lr, scale, keys, encoder, encryptor,
-                                     degree=degree, method=method)
+                                     degree=degree, method=method, sigmoid=sigmoid)
         decoded = encoder.decode(decryptor.decrypt(new_weights))[0, : layout.C]
         new_weights = encryptor.encrypt(encoder.encode(layout.weights(decoded), scale))
     return new_weights

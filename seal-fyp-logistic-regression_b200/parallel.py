@@ -12,8 +12,8 @@ import torch.distributed as dist
 
 from . import capi
 from .engine import Ciphertext
-from .lr import _poly, apply_gradient, folded_coeffs
-from .workloads import _stack, cipher_dot_product, duplicate_fill, force_scale_pow2
+from .lr import SIGMOID_CHEBYSHEV, apply_gradient, prediction_masks, sigmoid_cipher
+from .workloads import _stack, chebyshev_keyswitches, cipher_dot_product, duplicate_fill, force_scale_pow2
 
 
 def world():
@@ -283,12 +283,14 @@ def config1_shards(R, C, rank, world_size):
     return owned_block(R, rank, world_size), owned_block(C, rank, world_size)
 
 
-def config1_keyswitches(R, C, rank, world_size, degree=3):
+def config1_keyswitches(R, C, rank, world_size, degree=3, method="horner", sigmoid=None):
     """key switches of this rank in one sharded_update_weights with the Horner polynomial (rank 0 evaluates it): per own
     row 1 relinearisation + rotate_vector(-C) + C - 1 chain steps, per own feature 1 + rotate_vector(-R) + R - 1; a
-    rotation by a step without its own Galois key costs the NAF weight of the step (power-of-two keys)"""
+    rotation by a step without its own Galois key costs the NAF weight of the step (power-of-two keys).  With
+    method="chebyshev" rank 0's polynomial costs chebyshev_keyswitches(sigmoid degree) relinearisations."""
     rows, feats = config1_shards(R, C, rank, world_size)
-    return (len(rows) * (1 + naf_weight(C) + C - 1) + (degree if rank == 0 else 0)
+    poly = chebyshev_keyswitches((sigmoid or SIGMOID_CHEBYSHEV).degree) if method == "chebyshev" else degree
+    return (len(rows) * (1 + naf_weight(C) + C - 1) + (poly if rank == 0 else 0)
             + len(feats) * (1 + naf_weight(R) + R - 1))
 
 
@@ -323,7 +325,8 @@ def _broadcast_ct(ctx, ct, rank, exchange):
 
 
 def sharded_update_weights(ev, rows_local, row_ids, cols_local, feature_ids, labels, weights, lr, R, C, scale, keys,
-                           encoder, encryptor, rank, world_size, exchange, degree=3, method="horner", mark=None):
+                           encoder, encryptor, rank, world_size, exchange, degree=3, method="horner", mark=None,
+                           sigmoid=None):
     """lr.update_weights (logistic_regression_ckks.cpp:269-345, config 1) with its R row dot products and its C feature
     dot products sharded over `world_size` ranks; every rank returns the new-weights ciphertext, bit-identical to the
     one-GPU function on the full inputs.
@@ -346,7 +349,7 @@ def sharded_update_weights(ev, rows_local, row_ids, cols_local, feature_ids, lab
     ctx = weights.ctx
     if rows_local.batch:
         results = cipher_dot_product(ev, rows_local, weights, C, keys)
-        mask_pt = encoder.encode(_one_hot(row_ids, R), scale)
+        mask_pt = encoder.encode(prediction_masks(_one_hot(row_ids, R), method, sigmoid), scale)
         ev.mod_switch_to_next_inplace(mask_pt)
         part = ev.multiply_plain_sum(results, mask_pt)
     else:
@@ -359,8 +362,7 @@ def sharded_update_weights(ev, rows_local, row_ids, cols_local, feature_ids, lab
     if rank == 0:
         lin = ev.relinearize(lin, keys)
         ev.rescale_to_next_inplace(lin)
-        force_scale_pow2(lin)
-        pred = _poly(method)(ev, lin, folded_coeffs(degree), scale, keys, encoder, encryptor)
+        pred = sigmoid_cipher(ev, lin, scale, keys, encoder, encryptor, degree, method, sigmoid)
         lab = ev.mod_switch_to(labels, pred.limbs)
         if lab.scale != pred.scale:
             pred.scale = lab.scale
@@ -387,7 +389,7 @@ def sharded_update_weights(ev, rows_local, row_ids, cols_local, feature_ids, lab
 
 
 def sharded_train_cipher(ev, rows_local, row_ids, cols_local, feature_ids, labels, weights, lr, iters, layout, scale, keys,
-                         encoder, encryptor, decryptor, rank, world_size, exchange, degree=3, method="horner"):
+                         encoder, encryptor, decryptor, rank, world_size, exchange, degree=3, method="horner", sigmoid=None):
     """lr.train_cipher (logistic_regression_ckks.cpp:348-385, repair R4) over sharded_update_weights: after every
     iteration rank 0, the key holder (only it has a `decryptor` and an `encryptor`), decrypts and decodes the weights,
     re-packs them (RowLayout.weights), encodes them at the top level, re-encrypts them and broadcasts the ciphertext.
@@ -397,7 +399,7 @@ def sharded_train_cipher(ev, rows_local, row_ids, cols_local, feature_ids, label
     for _ in range(iters):
         new_weights = sharded_update_weights(ev, rows_local, row_ids, cols_local, feature_ids, labels, new_weights, lr,
                                              layout.R, layout.C, scale, keys, encoder, encryptor, rank, world_size, exchange,
-                                             degree=degree, method=method)
+                                             degree=degree, method=method, sigmoid=sigmoid)
         fresh = None
         if rank == 0:
             decoded = encoder.decode(decryptor.decrypt(new_weights))[0, : layout.C]

@@ -325,6 +325,195 @@ def tree_cipher(ev, x, coeffs, scale, keys, encoder, encryptor):
     return enc_result
 
 
+# ------------------------------------------------------------------ polynomials in the Chebyshev basis
+def chebyshev_interpolant(f, B, degree):
+    """coefficients c_0..c_degree of the Chebyshev interpolant of f on [-B, B]: f(x) ~ sum c_i T_i(x / B)
+    (interpolation at the degree + 1 Chebyshev points of the first kind)"""
+    k = np.arange(degree + 1)
+    t = np.cos(np.pi * (k + 0.5) / (degree + 1))
+    v = np.asarray(f(B * t), dtype=np.float64)
+    c = 2.0 / (degree + 1) * np.cos(np.outer(k, np.pi * (k + 0.5) / (degree + 1))) @ v
+    c[0] /= 2.0
+    return c
+
+
+def _bsgs_shape(degree):
+    """(m, l): the polynomial is padded to 2^m coefficients, the baby steps are T_1..T_{2^l - 1}, the giant steps
+    T_{2^l}, ..., T_{2^(m-1)}"""
+    if degree < 1:
+        raise ValueError("chebyshev: degree must be at least 1")
+    m = max(1, int(degree).bit_length())   # 2^m > degree
+    return m, (m + 1) // 2
+
+
+def _basis_doublings(m, l):
+    """the power basis T_1..T_{2^K} is built by K doublings: up to the first giant step T_{2^l} when there are giant
+    steps, else up to the last baby step T_{2^l - 1}"""
+    top = (1 << l) if m > l else (1 << l) - 1
+    return max(0, (top - 1).bit_length())
+
+
+def chebyshev_depth(degree):
+    """levels chebyshev_cipher consumes for a polynomial of this degree: the doublings of the power basis, one for the
+    baby-step sums and one per giant step (m + 1 = ceil(log2(degree + 1)) + 1 when there are giant steps)"""
+    m, l = _bsgs_shape(degree)
+    return _basis_doublings(m, l) + 1 + (m - l)
+
+
+def chebyshev_keyswitches(degree):
+    """relinearisations of one chebyshev_cipher per input ciphertext: 2^k products in doubling k of the power basis, one
+    square per further giant step, 2^(m-1-k) products at the giant step T_{2^k}"""
+    m, l = _bsgs_shape(degree)
+    K = _basis_doublings(m, l)
+    return (1 << K) - 1 + max(0, m - 1 - K) + ((1 << (m - l)) - 1)
+
+
+def chebyshev_split(coeffs, degree_pow2, l):
+    """the baby-step polynomials ("leaves") of sum c_i T_i padded to 2^m coefficients: p = q T_{2^(m-1)} + r, recursively
+    down to 2^l coefficients; leaf g collects the divisions by T_{2^k} whose quotient it is part of in bit k - l of g.
+    Division by T_n (c of length 2n): q_0 = c_n, q_j = 2 c_{n+j}, r_i = c_i - c_{2n-i} (r_0 = c_0)."""
+    c = np.zeros(degree_pow2)
+    c[:len(coeffs)] = coeffs
+
+    def rec(c):
+        if len(c) <= (1 << l):
+            return [c]
+        n = len(c) // 2
+        q = np.empty(n)
+        q[0] = c[n]
+        q[1:] = 2.0 * c[n + 1:]
+        r = c[:n].copy()
+        r[1:] -= c[2 * n - 1:n:-1]
+        return rec(r) + rec(q)
+    return rec(c)
+
+
+def _repeat(ct, times):
+    """`times` copies of a batch (a batch of 1 is broadcast by multiply as it is)"""
+    if times == 1 or ct.batch == 1:
+        return ct
+    return Ciphertext(ct.ctx, ct.data[:, :, :ct.limbs].repeat(times, 1, 1, 1), ct.limbs, ct.scale)
+
+
+def chebyshev_cipher(ev, t, coeffs, keys, scale=None):
+    """sum_i coeffs[i] T_i(t) for a batch of M ciphertexts holding t in [-1, 1], by baby steps and giant steps
+    (T_{a+b} = 2 T_a T_b - T_{|a-b|}); consumes chebyshev_depth(degree) levels and needs only the relinearisation key.
+
+    1. Power basis, one depth level at a time: [T_1..T_{2^k}] (uniform scale s_k) times T_{2^k} is one batched multiply +
+       relinearize; one grouped multiply_const_sum forms T_{2^k + j} = 2 T_j T_{2^k} - T_{2^k - j} (and - 1 for j = 2^k)
+       and carries T_1..T_{2^k} over (times 1 encoded at s_k), all at scale s_k^2; one batched rescale.  Giant steps
+       beyond the basis: T_{2n} = 2 T_n^2 - 1.
+    2. Baby-step sums: the 2^(m-l) leaves of chebyshev_split, sum_{i < 2^l} c_i T_i, in ONE multiply_const_sum over
+       T_1..T_{2^l - 1} with every constant encoded at the leaf scale rho; rescale.
+    3. Giant steps T_{2^k}, k = l..m-1: u_j = Y_{2j+1} T_{2^k} + Y_{2j}; the products are relinearized and one
+       multiply_const_sum adds them to the Y_{2j} lifted by a constant 1 encoded at the giant step's scale, so both
+       terms carry exactly the product's scale before the rescale.
+
+    Scales are exact: every sum adds terms whose scales are the same float (constants are encoded at the scale that
+    makes them so) and nothing is reassigned.  The leaf scale rho is the one free parameter; it is chosen by replaying
+    the evaluator's scale arithmetic so that the result carries `scale` (default t.scale): exactly when some float rho
+    gets there, else the nearest float reachable (a few 1e-16 relative).  This avoids the up to 1e-5 relative error per
+    rescale of forcing power-of-two scales when the primes are only near 2^40."""
+    ctx = t.ctx
+    coeffs = np.asarray(coeffs, dtype=np.float64)
+    degree = len(coeffs) - 1
+    m, l = _bsgs_shape(degree)
+    K, b, M = _basis_doublings(m, l), 1 << l, t.batch
+    target = float(t.scale if scale is None else scale)
+    if t.limbs <= chebyshev_depth(degree):
+        raise capi.CkksInvalidArgument("chebyshev: %d levels needed, the input has %d limbs"
+                                       % (chebyshev_depth(degree), t.limbs))
+    # 1. power basis [T_1..T_{2^k}], entry (j-1)*M + m
+    basis = ev.mod_switch_to(t, t.limbs)
+    for k in range(K):
+        h = 1 << k
+        top = basis[(h - 1) * M:h * M]
+        prods = ev.relinearize(ev.multiply(basis, _repeat(top, h)), keys)       # T_j T_h, scale s_k^2
+        cf = np.zeros((2 * h, 2 * h))
+        konst = np.zeros(2 * h)
+        for j in range(1, h + 1):
+            cf[j - 1, h + j - 1] = 1.0                                          # carry T_j
+            cf[h + j - 1, j - 1] = 2.0                                          # T_{h+j} = 2 T_j T_h - T_{h-j}
+            if j < h:
+                cf[h + j - 1, h + (h - j) - 1] = -1.0
+            else:
+                konst[h + j - 1] = -1.0
+        pts = [1.0] * h + [basis.scale] * h
+        cs = ev.multiply_const_sum(_split_terms(prods, h) + _split_terms(basis, h), cf, pts, constant=konst, groups=2 * h)
+        basis = ev.rescale_to_next_inplace(cs)
+    giants = {}
+    if m > l:
+        giants[l] = basis[(b - 1) * M:b * M]
+        for k in range(l, m - 1):
+            g = giants[k]
+            sq = ev.relinearize(ev.multiply(g, g), keys)
+            giants[k + 1] = ev.rescale_to_next_inplace(ev.multiply_const_sum(sq, [2.0], 1.0, constant=[-1.0]))
+    # the leaf scale rho that makes the result's scale exactly `target`
+    L = basis.limbs
+    drops = [ctx.primes[L - 1 - i] for i in range(m - l + 1)]
+    gscales = [giants[k].scale for k in range(l, m)]
+
+    def result_scale(rho):
+        sc = basis.scale * rho / float(drops[0])
+        for q, gs in zip(drops[1:], gscales):
+            sc = sc * gs / float(q)
+        return sc
+    guess = target / basis.scale
+    for q in drops:
+        guess *= float(q)
+    for gs in gscales:
+        guess /= gs
+    rho = _solve_scale(result_scale, target, guess)
+    # 2. every baby-step sum in one launch
+    leaves = chebyshev_split(coeffs, 1 << m, l)
+    G = len(leaves)
+    cf = np.stack([leaf[1:b] for leaf in leaves])
+    Y = ev.multiply_const_sum(basis[0:(b - 1) * M], cf, rho, constant=[leaf[0] for leaf in leaves], groups=G)
+    ev.rescale_to_next_inplace(Y)
+    # 3. giant steps: u_j = Y_{2j+1} T_{2^k} + Y_{2j}
+    for k in range(l, m):
+        n = Y.batch // (2 * M)
+        odd = Ciphertext(ctx, torch.cat([Y.data[(2 * j + 1) * M:(2 * j + 2) * M, :, :Y.limbs] for j in range(n)], dim=0),
+                         Y.limbs, Y.scale)
+        g = ev.mod_switch_to(giants[k], Y.limbs)
+        prods = ev.relinearize(ev.multiply(odd, _repeat(g, n)), keys)
+        cf = np.zeros((n, 3 * n))
+        for j in range(n):
+            cf[j, j] = 1.0                                                      # Y_{2j+1} T_{2^k}
+            cf[j, n + 2 * j] = 1.0                                              # Y_{2j}, times 1 encoded at T_{2^k}'s scale
+        pts = [1.0] * n + [g.scale] * (2 * n)
+        Y = ev.multiply_const_sum(_split_terms(prods, n) + _split_terms(Y, 2 * n), cf, pts, groups=n)
+        ev.rescale_to_next_inplace(Y)
+    return Y
+
+
+def _split_terms(ct, T):
+    """a batch of T*M ciphertexts -> T views of M entries"""
+    M = ct.batch // T
+    return [ct[i * M:(i + 1) * M] for i in range(T)]
+
+
+def _solve_scale(fn, target, x):
+    """x with fn(x) == target for a non-decreasing float function fn close to proportional, else the closest x found"""
+    for _ in range(8):                                       # proportional corrections
+        y = fn(x)
+        if y == target:
+            return x
+        x = x * (target / y)
+    best, gap = x, abs(fn(x) - target)
+    up = fn(x) < target
+    for _ in range(4096):                                    # then float steps towards the target
+        x = math.nextafter(x, math.inf if up else 0.0)
+        y = fn(x)
+        if y == target:
+            return x
+        if abs(y - target) < gap:
+            best, gap = x, abs(y - target)
+        if (y > target) == up:
+            break
+    return best
+
+
 # ------------------------------------------------------------------ diagonal sets with a shared default
 class DiagonalSet:
     """The plaintext diagonals of one matrix in de-duplicated form: `default` is the plaintext shared
