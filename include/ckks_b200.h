@@ -219,6 +219,12 @@ int ckks_multiply_plain_sum(ckks_ctx *ctx, const ckks_view *cts, const ckks_view
 /* out (batch 1, size 3) = sum_b a[b] x b[b] for size-2 inputs -- multiply + add_many,
  * helper.h:222-233, matrix_multiplication.cpp:123-129 */
 int ckks_multiply_sum(ckks_ctx *ctx, const ckks_view *a, const ckks_view *b, const ckks_view *out, ckks_stream s);
+/* `groups` sums against the same b in one launch: out[g] (size 3) = sum_i a[g*T + i] x b[i], T = b->batch,
+ * a->batch = groups * T, out->batch = groups -- per group multiply + add_many (the column-layout prediction:
+ * one sum per mini-batch over its feature columns times the weight broadcasts).  groups = 1 is ckks_multiply_sum.
+ * CKKS_ERR_INVALID for groups < 1, mismatched batch, limbs or sizes, and out aliasing an input. */
+int ckks_multiply_sum_grouped(ckks_ctx *ctx, const ckks_view *a, const ckks_view *b, int groups, const ckks_view *out,
+                              ckks_stream s);
 
 /* ---- rescale / mod switch */
 /* Evaluator::rescale_to_next_inplace (helper.h:441,543; matrix_multiplication.cpp:71-72):

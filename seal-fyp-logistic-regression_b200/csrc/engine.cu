@@ -1379,25 +1379,32 @@ extern "C" int ckks_rotate_plan_hoisted(ckks_ctx *c, const ckks_rotplan *p, cons
 }
 
 // ------------------------------------------------------------------------------------ fused products
-static int mul_sum(ckks_ctx *c, bool plain, const ckks_view *a, const ckks_view *b, const ckks_view *o, cudaStream_t st) {
+// out[g] = sum_i a[g*T + i] (.) b[i], g < groups, T = b->batch
+static int mul_sum(ckks_ctx *c, bool plain, const ckks_view *a, const ckks_view *b, int groups, const ckks_view *o,
+                   cudaStream_t st) {
     int rc;
     if ((rc = check_view(c, a, "a")) || (rc = check_view(c, b, "b")) || (rc = check_view(c, o, "out"))) return rc;
-    if (a->batch != b->batch || a->limbs != b->limbs || o->limbs != a->limbs || o->batch != 1)
+    if (groups < 1) return fail(CKKS_ERR_INVALID, "multiply_sum: groups must be at least 1");
+    if ((long long)groups * b->batch != a->batch || a->limbs != b->limbs || o->limbs != a->limbs || o->batch != groups)
         return fail(CKKS_ERR_INVALID, "multiply_sum: parameter mismatch");
     if (plain ? (b->size != 1 || o->size != a->size) : (a->size != 2 || b->size != 2 || o->size != 3))
         return fail(CKKS_ERR_INVALID, "multiply_sum: size mismatch");
     if (o->data == a->data || o->data == b->data) return fail(CKKS_ERR_INVALID, "multiply_sum: out must not alias an input");
     CU(cudaSetDevice(c->device));
-    if (plain) k_ew_mul_sum<true><<<ew_grid(c, a->size * a->limbs, 1), 256, 0, st>>>(dv(a), dv(b), dv(o), a->batch, a->limbs, c->n, c->t);
-    else k_ew_mul_sum<false><<<ew_grid(c, a->limbs, 1), 256, 0, st>>>(dv(a), dv(b), dv(o), a->batch, a->limbs, c->n, c->t);
+    if (plain) k_ew_mul_sum<true><<<ew_grid(c, a->size * a->limbs, 1), 256, 0, st>>>(dv(a), dv(b), dv(o), b->batch, a->limbs, c->n, c->t);
+    else k_ew_mul_sum<false><<<ew_grid(c, a->limbs, groups), 256, 0, st>>>(dv(a), dv(b), dv(o), b->batch, a->limbs, c->n, c->t);
     LAUNCH_CHECK(c);
     return CKKS_OK;
 }
 extern "C" int ckks_multiply_plain_sum(ckks_ctx *c, const ckks_view *cts, const ckks_view *pts, const ckks_view *o, ckks_stream s) {
-    return mul_sum(c, true, cts, pts, o, (cudaStream_t)s);
+    return mul_sum(c, true, cts, pts, 1, o, (cudaStream_t)s);
 }
 extern "C" int ckks_multiply_sum(ckks_ctx *c, const ckks_view *a, const ckks_view *b, const ckks_view *o, ckks_stream s) {
-    return mul_sum(c, false, a, b, o, (cudaStream_t)s);
+    return mul_sum(c, false, a, b, 1, o, (cudaStream_t)s);
+}
+extern "C" int ckks_multiply_sum_grouped(ckks_ctx *c, const ckks_view *a, const ckks_view *b, int groups, const ckks_view *o,
+                                         ckks_stream s) {
+    return mul_sum(c, false, a, b, groups, o, (cudaStream_t)s);
 }
 
 // ------------------------------------------------------------------------------------ rescale

@@ -1435,13 +1435,16 @@ __global__ void __launch_bounds__(256) k_ew_add_many_grouped(DView in, DView o, 
     *vpw(o, b, s, j, n, c) = acc;
 }
 
-// fused multiply + add_many: out = sum_b a[b] (.) b[b]
+// fused multiply + add_many: out[g] = sum_b a[g*B + b] (.) b[b] for g = blockIdx.z (b shared by every group)
 //   PLAIN: b is a plaintext batch (every poly of a[b] times pt[b]), output size = size of a
-//   else : size-2 x size-2 ciphertext products, output size 3 (Linear_Transform_Cipher)
+//   else : size-2 x size-2 ciphertext products, output size 3 (Linear_Transform_Cipher; with several groups the
+//          column-layout prediction, one sum per mini-batch against the same weight broadcasts)
 // 128-bit lazy sums with a reduction every 16 terms; identical to SEAL's sequential
 // multiply + add_inplace because the sum is taken modulo q either way.
 template <bool PLAIN>
 __global__ void __launch_bounds__(256) k_ew_mul_sum(DView a, DView b, DView o, int B, int L, int n, Tables t) {
+    a.data += (u64)blockIdx.z * B * a.bs;
+    o.data += (u64)blockIdx.z * o.bs;
     const int s = PLAIN ? blockIdx.y / L : 0, j = blockIdx.y % L;
     const u64 c = ((u64)blockIdx.x * blockDim.x + threadIdx.x) * 2;
     if (c >= (u64)n) return;

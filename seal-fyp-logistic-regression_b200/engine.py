@@ -587,6 +587,20 @@ class Evaluator:
         out.scale = scale
         return out
 
+    def multiply_sum_grouped(self, a, b, groups, out=None):
+        """batch groups*T times batch T -> batch groups: out[g] = sum_i multiply(a[g*T + i], b[i]), then add_many per
+        group, in one kernel; b is shared by every group (no repeat)"""
+        if a.limbs != b.limbs or groups < 1 or a.batch != groups * b.batch:
+            raise capi.CkksInvalidArgument("encrypted1 and encrypted2 parameter mismatch")
+        scale = a.scale * b.scale
+        self._scale_ok(scale, a.limbs)
+        out = a[0:groups].like(size=3) if out is None else out
+        out.limbs = a.limbs
+        va, vb, vo = a.view(), b.view(), out.view()
+        check(self.lib.ckks_multiply_sum_grouped(self.h, C.byref(va), C.byref(vb), int(groups), C.byref(vo), _stream()))
+        out.scale = scale
+        return out
+
 
 class RotPlan:
     """a fixed list of rotation steps (one per batch entry) compiled into batched rounds"""

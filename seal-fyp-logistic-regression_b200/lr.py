@@ -20,7 +20,8 @@ method="chebyshev" (opt-in, not the reference's) replaces the degree-3 polynomia
 pulsar data reach |x.w| = 38, by the Chebyshev interpolant of the sigmoid on [-B, B] (ChebyshevSigmoid, default degree 63,
 B = 48) evaluated by workloads.chebyshev_cipher with exact scales.  The 1/B input scaling is folded into the one-hot
 prediction masks (e_i / B), so it costs no level; the polynomial takes chebyshev_depth(63) = 7 levels, so config 1 needs
-{60, 40 x 12, 60}.
+{60, 40 x 12, 60}.  The column layout accepts it too: there the 1/B is folded into the weight broadcasts (the key
+holder encrypts w_j / B), and an iteration takes 1 + 7 + 1 + 1 + 1 = 11 levels ({60, 40 x 11, 60}).
 
 Two layouts:
   * `RowLayout`     -- the reference's: one ciphertext per sample row for the prediction and one per
@@ -37,8 +38,8 @@ import numpy as np
 import torch
 
 from .engine import Ciphertext
-from .workloads import (chebyshev_cipher, chebyshev_interpolant, cipher_dot_product, force_scale_pow2, horner_cipher,
-                        tree_cipher)
+from .workloads import (chebyshev_cipher, chebyshev_depth, chebyshev_interpolant, cipher_dot_product, force_scale_pow2,
+                        horner_cipher, tree_cipher)
 
 # logistic_regression_ckks.cpp:247,251,255 (zero coefficients are written 0.00001 there because
 # Tree_cipher dereferences every coefficient plaintext)
@@ -94,8 +95,6 @@ def _bcast(ct, batch):
 
 
 def _poly(method):
-    if method == "chebyshev":
-        raise ValueError("method='chebyshev' is implemented for the row layout (predict_cipher_weights) only")
     return tree_cipher if method == "tree" else horner_cipher
 
 
@@ -229,9 +228,36 @@ class ColumnLayout:
         out[:, : self.B] = y.reshape(self.M, self.B)
         return out
 
+    def weights(self, w):
+        """the packed weights apply_gradient updates: slot j holds w_j for j < C"""
+        out = np.zeros(self.slots)
+        out[: self.C] = w
+        return out
+
+    def weight_broadcasts(self, w, method="tree", sigmoid=None):
+        """-> [C][slots]: row j holds w_j in every slot, divided by the sigmoid's bound for method="chebyshev" (the
+        polynomial's input is x.w / bound; folding 1/bound into the broadcasts costs no level)"""
+        w = np.asarray(w, dtype=np.float64)
+        if method == "chebyshev":
+            w = w / (sigmoid or SIGMOID_CHEBYSHEV).bound
+        return np.repeat(w[:, None], self.slots, axis=1)
+
+
+def column_rescales(method="tree", degree=7, sigmoid=None):
+    """levels one column-layout iteration (column_epoch_gradient + apply_gradient) consumes: the prediction, the
+    sigmoid polynomial, the dot product, the mask and the learning rate, one rescale each except the polynomial's
+    ceil(log2 degree) + 1 (Tree_cipher), degree (Horner_cipher) or chebyshev_depth (chebyshev_cipher)"""
+    if method == "chebyshev":
+        poly = chebyshev_depth((sigmoid or SIGMOID_CHEBYSHEV).degree)
+    elif method == "tree":
+        poly = (degree - 1).bit_length() + 1
+    else:
+        poly = degree
+    return 1 + poly + 1 + 1 + 1
+
 
 def column_epoch_gradient(ev, cols, labels, w_bcast, C, B, scale, keys, encoder, encryptor, degree=7,
-                          method="tree", dot_method="reference", units=None, combine=None):
+                          method="tree", dot_method="reference", units=None, combine=None, sigmoid=None, mark=None):
     """One pass of the gradient loop over the mini-batches held by this GPU (column layout).
 
     cols    : batch M*C of column ciphertexts (entry m*C + j)
@@ -240,30 +266,29 @@ def column_epoch_gradient(ev, cols, labels, w_bcast, C, B, scale, keys, encoder,
     returns : one gradient ciphertext, slot j = sum_m sum_i x_ij (sigma(x_i.w) - y_i), plus its level
 
     Per mini-batch the evaluator sequence is: z = sum_j multiply(col_j, w_j); relinearize; rescale;
-    sigmoid polynomial (Tree_cipher / Horner_cipher); sub labels; then, per feature j, the reference's
+    sigmoid polynomial (Tree_cipher / Horner_cipher; for method="chebyshev" chebyshev_cipher on z as it is, with
+    w_bcast holding w_j / bound, see ColumnLayout.weight_broadcasts); sub labels; then, per feature j, the reference's
     cipher_dot_product(col_j, pred - y, B) and the one-hot mask e_j (update_weights :295-311);
-    add_many; rescale.
+    add_many; rescale.  The M sums z are one grouped multiply_sum against the shared broadcasts.
 
     `units` (optional) restricts the gradient dot products to a list of (mini-batch, feature) pairs -- the
     sharding unit when ONE problem is split over several GPUs (SURVEY 8(e): "shard features j and
     mini-batches"); the prediction is still evaluated for every mini-batch held here, the result is the
     partial gradient sum over `units`.  `combine` (optional) is applied to the partial sum BEFORE the final rescale --
     pass parallel.combine_partials there (all-gather + mod-q add): summing first and rescaling once keeps the
-    sharded result bit-identical to the unsharded one (rescale rounds, so it does not commute with the sum)."""
+    sharded result bit-identical to the unsharded one (rescale rounds, so it does not commute with the sum).
+    `mark(name)` (optional) is called as each phase ends: prediction, polynomial, gradient, combine."""
+    mark = mark or (lambda name: None)
     M = labels.batch
-    wb = Ciphertext(w_bcast.ctx, w_bcast.data.repeat(M, 1, 1, 1), w_bcast.limbs, w_bcast.scale)
-    prods = ev.multiply(cols, wb)                                         # M*C size-3 products
-    z = []
-    for m in range(M):
-        z.append(ev.add_many(prods[m * C:(m + 1) * C]))
-    z = Ciphertext(cols.ctx, torch.cat([t.data for t in z], dim=0), prods.limbs, prods.scale)
+    z = ev.multiply_sum_grouped(cols, w_bcast, M)                         # M size-3 sums of C products
     z = ev.relinearize(z, keys)
     ev.rescale_to_next_inplace(z)
-    force_scale_pow2(z)
-    pred = _poly(method)(ev, z, folded_coeffs(degree), scale, keys, encoder, encryptor)
+    mark("prediction")
+    pred = sigmoid_cipher(ev, z, scale, keys, encoder, encryptor, degree, method, sigmoid)
     lab = ev.mod_switch_to(labels, pred.limbs)
     pred.scale = lab.scale
     pred_labels = ev.sub(pred, lab)                                       # batch M
+    mark("polynomial")
     colv = ev.mod_switch_to(cols, pred_labels.limbs)
     masks = np.zeros((C, C))
     masks[np.arange(C), np.arange(C)] = 1.0
@@ -284,8 +309,10 @@ def column_epoch_gradient(ev, cols, labels, w_bcast, C, B, scale, keys, encoder,
         mp = Ciphertext(cols.ctx, mask_pt.data.index_select(0, ji), mask_pt.limbs, mask_pt.scale)
     ev.multiply_plain_inplace(grads, mp)
     gradient = ev.add_many(grads)                                         # over features and mini-batches
+    mark("gradient")
     if combine is not None:
         gradient = combine(gradient)                                      # ... and over GPUs
+    mark("combine")
     ev.rescale_to_next_inplace(gradient)
     return force_scale_pow2(gradient)
 
@@ -299,3 +326,26 @@ def apply_gradient(ev, gradient, weights, lr, R, scale, encoder):
     w_low = ev.mod_switch_to(weights, g.limbs)
     w_low.scale = g.scale
     return ev.negate_inplace(ev.sub(g, w_low))
+
+
+def refresh_columns(new_weights, layout, scale, encoder, encryptor, decryptor, method="tree", sigmoid=None):
+    """the key holder's refresh of the column layout (repair R4): decrypt the updated weights, decode slots [0, C),
+    re-encode the packed weights and the C broadcasts at the top level and re-encrypt them (in this order)"""
+    decoded = encoder.decode(decryptor.decrypt(new_weights))[0, : layout.C]
+    weights = encryptor.encrypt(encoder.encode(layout.weights(decoded), scale))
+    w_bcast = encryptor.encrypt(encoder.encode(layout.weight_broadcasts(decoded, method, sigmoid), scale))
+    return weights, w_bcast
+
+
+def train_columns(ev, cols, labels, weights, w_bcast, lr, iters, layout, scale, keys, encoder, encryptor, decryptor,
+                  degree=7, method="tree", sigmoid=None):
+    """full-batch gradient descent in the column layout: `iters` x (column_epoch_gradient over every mini-batch,
+    apply_gradient, refresh_columns), the loop of train_cipher (logistic_regression_ckks.cpp:348-385).
+    `weights`: the packed weights (ColumnLayout.weights), `w_bcast`: the C broadcasts (ColumnLayout.weight_broadcasts
+    with the same method and sigmoid).  Returns the refreshed (weights, w_bcast), both at the top level."""
+    for _ in range(iters):
+        grad = column_epoch_gradient(ev, cols, labels, w_bcast, layout.C, layout.B, scale, keys, encoder, encryptor,
+                                     degree=degree, method=method, sigmoid=sigmoid)
+        new_weights = apply_gradient(ev, grad, weights, lr, layout.R, scale, encoder)
+        weights, w_bcast = refresh_columns(new_weights, layout, scale, encoder, encryptor, decryptor, method, sigmoid)
+    return weights, w_bcast

@@ -12,8 +12,10 @@ import torch.distributed as dist
 
 from . import capi
 from .engine import Ciphertext
-from .lr import SIGMOID_CHEBYSHEV, apply_gradient, prediction_masks, sigmoid_cipher
-from .workloads import _stack, chebyshev_keyswitches, cipher_dot_product, duplicate_fill, force_scale_pow2
+from .lr import (SIGMOID_CHEBYSHEV, apply_gradient, column_epoch_gradient, prediction_masks, refresh_columns,
+                 sigmoid_cipher)
+from .workloads import (_stack, chebyshev_depth, chebyshev_keyswitches, cipher_dot_product, duplicate_fill,
+                        force_scale_pow2)
 
 
 def world():
@@ -406,3 +408,79 @@ def sharded_train_cipher(ev, rows_local, row_ids, cols_local, feature_ids, label
             fresh = encryptor.encrypt(encoder.encode(layout.weights(decoded), scale))
         new_weights = _broadcast_ct(weights.ctx, fresh, rank, exchange)
     return new_weights
+
+
+# ------------------------------------------------------------------ sharded column-layout training
+def column_units(M, C, rank, world_size):
+    """this rank's (mini-batch, feature) gradient units of the column layout: a contiguous block of the M*C units in
+    (m, j) order, so that a rank touches as few mini-batches as possible.  The first M*C mod G ranks own one unit more;
+    with more ranks than units the last ranks own none."""
+    return [(u // C, u % C) for u in owned_block(M * C, rank, world_size)]
+
+
+def column_keyswitches(R, C, B, rank, world_size, method, degree=7, sigmoid=None):
+    """key switches of this rank in one sharded_train_columns iteration with the power-of-two Galois keys: per
+    mini-batch its units touch, 1 prediction relinearisation + the polynomial's relinearisations (chebyshev_keyswitches
+    of the sigmoid's degree, degree - 1 for Tree_cipher, degree for Horner_cipher; repeated on every rank that shares
+    the mini-batch); per own unit 1 relinearisation + rotate_vector(-B) (its NAF weight) + B - 1 chain steps"""
+    units = column_units(R // B, C, rank, world_size)
+    if method == "chebyshev":
+        poly = chebyshev_keyswitches((sigmoid or SIGMOID_CHEBYSHEV).degree)
+    else:
+        poly = degree - 1 if method == "tree" else degree
+    return len({m for m, _ in units}) * (1 + poly) + len(units) * (1 + naf_weight(B) + B - 1)
+
+
+def sharded_train_columns(ev, cols_local, labels_local, minibatch_ids, units, weights, w_bcast, lr, iters, layout, scale,
+                          keys, encoder, encryptor, decryptor, rank, world_size, exchange, method="chebyshev",
+                          sigmoid=None, mark=None):
+    """lr.train_columns with the M*C (mini-batch, feature) gradient units sharded over `world_size` ranks; after every
+    iteration every rank holds (weights, w_bcast) bit-identical to the one-GPU loop.
+
+    cols_local / labels_local: the column (entry k*C + j) and label ciphertexts of the mini-batches `minibatch_ids`
+    (increasing) that this rank's `units` (column_units, global (m, j) pairs) touch; both may be empty batches, which
+    still carry level and scale.  weights / w_bcast: replicated.  `encryptor` and `decryptor`: rank 0's, the key
+    holder's; the other ranks pass None.  `exchange`: TorchExchange, or a test emulation with all_gather and broadcast.
+
+    Each rank evaluates the prediction and the polynomial of its own mini-batches (repeated where ranks share one) and
+    the gradient chains of its own units; the partial gradients are summed by all-gather + mod-q add before the rescale
+    (a rank without units adds zero), and the learning-rate tail runs on every rank.  Rank 0 then refreshes the weights
+    (lr.refresh_columns) and broadcasts the packed weights and the C broadcasts.  Only method="chebyshev" is accepted:
+    Tree_cipher and Horner_cipher encrypt a coefficient on every call, so ranks evaluating the same mini-batch would
+    disagree.  `mark(name)`, when given, is called as each phase ends: prediction, polynomial, gradient, combine,
+    tail, refresh."""
+    if method != "chebyshev":
+        raise ValueError("sharded_train_columns: only method='chebyshev' is deterministic; the reference polynomials "
+                         "encrypt a coefficient, so ranks sharing a mini-batch would disagree")
+    C = layout.C
+    if (not 0 <= rank < world_size or cols_local.batch != len(minibatch_ids) * C or labels_local.batch != len(minibatch_ids)
+            or any(m not in minibatch_ids for m, _ in units)):
+        raise ValueError("sharded_train_columns: rank, shard sizes or units do not match")
+    mark = mark or (lambda name: None)
+    ctx = weights.ctx
+    pos = {m: k for k, m in enumerate(minibatch_ids)}
+    local = [(pos[m], j) for m, j in units]
+
+    def combine(part):
+        return _combine(ev, _active(part), exchange)
+    for _ in range(iters):
+        if local:
+            grad = column_epoch_gradient(ev, cols_local, labels_local, w_bcast, C, layout.B, scale, keys, encoder, encryptor,
+                                         method=method, units=local, combine=combine, sigmoid=sigmoid, mark=mark)
+        else:                               # no unit here: the prediction's level and scale give the zero partial
+            Lp = cols_local.limbs - 1 - chebyshev_depth((sigmoid or SIGMOID_CHEBYSHEV).degree)
+            part = _zero_partial(ctx, Lp - 1, _rescaled_pow2_scale(ctx, cols_local.scale * labels_local.scale, Lp) * scale)
+            for name in ("prediction", "polynomial", "gradient"):
+                mark(name)
+            grad = combine(part)
+            mark("combine")
+            ev.rescale_to_next_inplace(grad)
+            force_scale_pow2(grad)
+        new_weights = apply_gradient(ev, grad, weights, lr, layout.R, scale, encoder)
+        mark("tail")
+        fresh = (None, None)
+        if rank == 0:
+            fresh = refresh_columns(new_weights, layout, scale, encoder, encryptor, decryptor, method, sigmoid)
+        weights, w_bcast = [_broadcast_ct(ctx, ct, rank, exchange) for ct in fresh]
+        mark("refresh")
+    return weights, w_bcast
