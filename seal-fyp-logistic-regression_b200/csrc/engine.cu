@@ -131,6 +131,9 @@ struct ckks_ctx {
         uint64_t launches;
     };
     std::map<std::vector<uint64_t>, ChainGraph> chain_graphs;
+    // rotate-and-sum chains with c0 carried split (ChainV in kernels.cuh): V of a, V of b and V of acc, [3][batch][N][2]
+    u64 *chain_v = nullptr;
+    size_t chain_v_bytes = 0;
 };
 
 struct ckks_keyset {
@@ -252,6 +255,7 @@ extern "C" void ckks_ctx_destroy(ckks_ctx *c) {
     cudaFree(c->d_inv); cudaFree(c->d_invs); cudaFree(c->d_half);
     cudaFree(c->d_fp); cudaFree(c->d_twfd); cudaFree(c->d_twid);
     cudaFree(c->ws);
+    cudaFree(c->chain_v);
     delete c;
 }
 
@@ -635,9 +639,13 @@ static int pick_split(int forced, int tiles, int maxsplit) {
 // Batched key switch over `nslots` launch slots.
 // mode 1: relinearize (target = poly 2 of the source, base = polys 0,1)
 // mode 2: Galois      (target = permuted poly 1, base = permuted poly 0)
-static int keyswitch(ckks_ctx *c, int mode, int L, int nslots, KsRoute rt, cudaStream_t st, bool chained = false, int li = 0, int slot0 = 0) {
+// cv (Galois mode only): the step belongs to a rotate-and-sum chain whose c0 is carried split (ChainV, kernels.cuh); its
+// arrays are indexed by launch slot, like the views of rt.
+static int keyswitch(ckks_ctx *c, int mode, int L, int nslots, KsRoute rt, cudaStream_t st, bool chained = false, int li = 0, int slot0 = 0,
+                     const ChainV *cv = nullptr) {
     const int K = c->K;
     const size_t N = c->n;
+    if (cv && (mode != 2 || !c->fuse || !cv->vin)) return fail(CKKS_ERR_INVALID, "split chain step needs the fused Galois pipeline");
     const int Bc = ks_chunk(c, nslots, L);
     int rc;
     if ((rc = ensure_lane(c, li, ks_words_per_ct(c, L) * 8 * (size_t)Bc))) return rc;
@@ -682,6 +690,13 @@ static int keyswitch(ckks_ctx *c, int mode, int L, int nslots, KsRoute rt, cudaS
             bigl.kh[1] = 2;
         }
         rt.b0 = b0;
+        ChainV cvc{};
+        if (cv) {
+            cvc = *cv;
+            cvc.vin += (size_t)b0 * 2 * N;
+            cvc.vout += (size_t)b0 * 2 * N;
+            cvc.vacc += (size_t)b0 * 2 * N;
+        }
         DView dD{D, (u64)L * N, 0};
         DView spec{ACC + (size_t)L * N, (u64)(L + 1) * N, 0};             // special-prime limb of every (b,k)
         DView minu{ACC, 2 * (u64)(L + 1) * N, (u64)(L + 1) * N};
@@ -733,7 +748,8 @@ static int keyswitch(ckks_ctx *c, int mode, int L, int nslots, KsRoute rt, cudaS
         if (sfp != st && special_small) CU(cudaStreamWaitEvent(st, ln.join, 0));                                        \
         if (fuse) {                                                                                                     \
             const int ns3 = pick_split(c->split3, G::COL_TILES * 2 * bc, L);                                            \
-            launch_pdl(k_md_invcol_fwdcol<LN>, dim3(G::COL_TILES, ns3, 2 * bc), st, spec, T2, L, K - 1, ns3, c->t);     \
+            if (cv) launch_pdl(k_md_invcol_fwdcol<LN, true>, dim3(G::COL_TILES, ns3, 2 * bc), st, spec, T2, L, K - 1, ns3, cvc, c->t); \
+            else launch_pdl(k_md_invcol_fwdcol<LN, false>, dim3(G::COL_TILES, ns3, 2 * bc), st, spec, T2, L, K - 1, ns3, cvc, c->t); \
             LAUNCH_CHECK(c);                                                                                            \
         } else {                                                                                                        \
             launch_pdl(k_inv_row<LN>, dim3(G::ROW_TILES, 1, 2 * bc), st, spec, spec, 1, K - 1, c->t);           \
@@ -744,7 +760,8 @@ static int keyswitch(ckks_ctx *c, int mode, int L, int nslots, KsRoute rt, cudaS
             LAUNCH_CHECK(c);                                                                                            \
         }                                                                                                               \
         if (sfp != st && !special_small) CU(cudaStreamWaitEvent(st, ln.join, 0));                                       \
-        if (mode == 2) launch_pdl(k_md_fwd_row<LN, 2>, dim3(G::ROW_TILES, L, 2 * bc), st, T2, minu, rt, 2, L, K - 1, c->t); \
+        if (cv) launch_pdl(k_md_fwd_row<LN, 3>, dim3(G::ROW_TILES, L, 2 * bc), st, T2, minu, rt, 2, L, K - 1, c->t);   \
+        else if (mode == 2) launch_pdl(k_md_fwd_row<LN, 2>, dim3(G::ROW_TILES, L, 2 * bc), st, T2, minu, rt, 2, L, K - 1, c->t); \
         else launch_pdl(k_md_fwd_row<LN, 1>, dim3(G::ROW_TILES, L, 2 * bc), st, T2, minu, rt, 2, L, K - 1, c->t); \
         LAUNCH_CHECK(c);                                                                                                \
     }
@@ -949,11 +966,45 @@ extern "C" int ckks_rotate(ckks_ctx *c, const ckks_keyset *ks, const ckks_view *
 }
 
 // ------------------------------------------------------------------------------------ rotate-and-sum chain
+// End of a split chain: ct.c0 += NTT(-P^-1 (V mod q_j)) for every entry (ChainV, kernels.cuh), through the workspace in
+// chunks of entries.  V: [batch][N][2].
+static int chain_fold(ckks_ctx *c, const ckks_view *ct, const u64 *V, cudaStream_t st) {
+    const int L = ct->limbs, B = ct->batch;
+    const size_t N = c->n;
+    size_t E = c->ws_bytes / (8 * (size_t)L * N);
+    if (E > 65535) E = 65535;
+    if (E < 1) return fail(CKKS_ERR_INVALID, "chain fold: workspace too small");
+    for (int b0 = 0; b0 < B; b0 += (int)E) {
+        const int e = (B - b0) < (int)E ? (B - b0) : (int)E;
+        DView r{c->ws, (u64)L * N, 0};
+        DView v = dv(ct);
+        v.data += (u64)b0 * v.bs;
+        k_chain_fold_residues<<<dim3((unsigned)((N + 255) / 256), L, e), 256, 0, st>>>(V + (size_t)b0 * 2 * N, c->ws, L, c->K - 1,
+                                                                                     (int)N, c->t);
+        LAUNCH_CHECK(c);
+#define RUN(LN)                                                                                                   \
+    {                                                                                                             \
+        k_fwd_col<LN><<<dim3(NttGeo<LN>::COL_TILES, L, e), NTT_THREADS, 0, st>>>(r, r, L, 0, c->t);               \
+        LAUNCH_CHECK(c);                                                                                          \
+        k_fwd_row<LN><<<dim3(NttGeo<LN>::ROW_TILES, L, e), NTT_THREADS, 0, st>>>(r, r, L, 0, c->t);               \
+        LAUNCH_CHECK(c);                                                                                          \
+    }
+        DISPATCH_LOGN(c, RUN)
+#undef RUN
+        k_ew_addsub<0><<<ew_grid(c, L, e), 256, 0, st>>>(v, r, v, L, (int)N, c->t);
+        LAUNCH_CHECK(c);
+    }
+    return CKKS_OK;
+}
+
 // `count` iterations of   dup = rotate_vector(dup, steps);  acc += dup   (cipher_dot_product's loop,
 // helper.h:472-476) on a batch of independent ciphertexts.  The rotation ping-pongs between the
 // views a and b (a holds dup on entry); the add is fused into the key switch's last kernel; two
 // steps (a->b, b->a) are captured once into a CUDA graph and replayed, so the dependent chain costs
 // one graph launch per two key switches instead of 18 kernel launches.
+// On the graph-replayed steps c0 of dup and of acc is carried split (ChainV, kernels.cuh): the mod-down adds each step's
+// rounding remainder to one integer polynomial per ciphertext instead of transforming it into every data prime, and a
+// fold after the last replayed step puts it back (DESIGN.md section 4).
 extern "C" int ckks_rotate_sum_chain(ckks_ctx *c, const ckks_keyset *ks, const ckks_view *a, const ckks_view *b,
                                      const ckks_view *acc, int steps, int count, int *final_in_b, ckks_stream s) {
     int rc;
@@ -974,8 +1025,28 @@ extern "C" int ckks_rotate_sum_chain(ckks_ctx *c, const ckks_keyset *ks, const c
     const int L = a->limbs, B = a->batch;
     if ((rc = ensure_ws(c, ks_words_per_ct(c, L) * 8 * (size_t)ks_chunk(c, B, L)))) return rc;
     cudaStream_t user = (cudaStream_t)s;
-    // one step on the batch entries [off, off+cnt) through lane `li`
-    auto one = [&](const ckks_view *src, const ckks_view *dst, cudaStream_t st, bool chained, int li, int off, int cnt) -> int {
+#ifdef V_CHAIN_NOSPLIT   // experiment only: every step transforms c0's remainder (the A/B baseline of profiles/chain_split_ab.py)
+    const bool split_c0 = false;
+#else
+    const bool split_c0 = count >= 4 && c->fuse;   // the unfused pipeline (CKKS_FUSE=0) has no split mode
+#endif
+    const size_t vper = 2 * (size_t)c->n, vview = (size_t)B * vper;   // words of V per entry / per view
+    if (split_c0 && c->chain_v_bytes < 3 * vview * 8) {
+        if (c->chain_v) {
+            CU(cudaDeviceSynchronize());   // in-flight chains may still use the old arrays
+            CU(cudaFree(c->chain_v));
+            c->chain_v = nullptr;
+            c->chain_v_bytes = 0;
+        }
+        for (auto &kv : c->chain_graphs) cudaGraphExecDestroy(kv.second.exec);   // they hold the old addresses
+        c->chain_graphs.clear();
+        if (cudaMalloc((void **)&c->chain_v, 3 * vview * 8) != cudaSuccess) return fail(CKKS_ERR_NOMEM, "chain allocation failed");
+        c->chain_v_bytes = 3 * vview * 8;
+    }
+    uint64_t gi = g;   // g^-1 mod 2^64 by Newton's iteration (g is odd; each step doubles the correct low bits, 3 -> 96)
+    for (int r = 0; r < 5; r++) gi *= 2 - g * gi;
+    // one step on the batch entries [off, off+cnt) through lane `li`; vsrc >= 0: c0 split, V of view vsrc (0 = a, 1 = b) read
+    auto one = [&](const ckks_view *src, const ckks_view *dst, cudaStream_t st, bool chained, int li, int off, int cnt, int vsrc) -> int {
         ckks_view vs = *src, vd = *dst, va = *acc;
         vs.data += (uint64_t)off * vs.batch_stride;
         vd.data += (uint64_t)off * vd.batch_stride;
@@ -984,7 +1055,13 @@ extern "C" int ckks_rotate_sum_chain(ckks_ctx *c, const ckks_keyset *ks, const c
         KsRoute rt = uniform_route(c, &vs, &vd, perm, it->second);
         rt.accv = dv(&va);
         rt.has_acc = 1;
-        return keyswitch(c, 2, L, cnt, rt, st, chained, li);
+        if (vsrc < 0) return keyswitch(c, 2, L, cnt, rt, st, chained, li);
+        ChainV cv{};
+        cv.vin = c->chain_v + vsrc * vview + off * vper;
+        cv.vout = c->chain_v + (1 - vsrc) * vview + off * vper;
+        cv.vacc = c->chain_v + 2 * vview + off * vper;
+        cv.ginv = (unsigned)(gi & (2 * (uint64_t)c->n - 1));
+        return keyswitch(c, 2, L, cnt, rt, st, chained, li, 0, &cv);
     };
     int done = 0;
     if (count >= 4) {
@@ -1023,15 +1100,15 @@ extern "C" int ckks_rotate_sum_chain(ckks_ctx *c, const ckks_keyset *ks, const c
                 std::vector<uint64_t> key = {(uint64_t)a->data, (uint64_t)b->data, (uint64_t)acc->data, (uint64_t)resolve_key(c, it->second, &key_tiled), g,
                                              (uint64_t)L, (uint64_t)off, (uint64_t)cnt, a->batch_stride, a->poly_stride, b->batch_stride,
                                              b->poly_stride, acc->batch_stride, acc->poly_stride, (uint64_t)ln.ws, (uint64_t)c->t.round_half,
-                                             (uint64_t)gp[which]};
+                                             (uint64_t)gp[which], (uint64_t)(split_c0 ? c->chain_v : nullptr), (uint64_t)B};
                 auto gi = c->chain_graphs.find(key);
                 if (gi == c->chain_graphs.end()) {
                     cudaGraph_t graph = nullptr;
                     uint64_t before = c->launches;
                     CU(cudaStreamBeginCapture(ln.main, cudaStreamCaptureModeThreadLocal));
                     for (int q = 0; q < gp[which] && !rc; q++) {
-                        rc = one(a, b, ln.main, q > 0, li, off, cnt);
-                        if (!rc) rc = one(b, a, ln.main, true, li, off, cnt);
+                        rc = one(a, b, ln.main, q > 0, li, off, cnt, split_c0 ? 0 : -1);
+                        if (!rc) rc = one(b, a, ln.main, true, li, off, cnt, split_c0 ? 1 : -1);
                     }
                     cudaError_t ce = cudaStreamEndCapture(ln.main, &graph);
                     uint64_t per = c->launches - before;
@@ -1059,6 +1136,10 @@ extern "C" int ckks_rotate_sum_chain(ckks_ctx *c, const ckks_keyset *ks, const c
                 per_graph[which] += gi->second.launches;
             }
         }
+        if (split_c0) {   // V of dup and of acc start at zero: c0 = A
+            CU(cudaMemsetAsync(c->chain_v, 0, vview * 8, user));
+            CU(cudaMemsetAsync(c->chain_v + 2 * vview, 0, vview * 8, user));
+        }
         CU(cudaEventRecord(c->ev_in, user));
         for (int li = 0; li < nl; li++) CU(cudaStreamWaitEvent(c->lane[li].main, c->ev_in, 0));
         int left = pairs;
@@ -1076,10 +1157,12 @@ extern "C" int ckks_rotate_sum_chain(ckks_ctx *c, const ckks_keyset *ks, const c
             CU(cudaStreamWaitEvent(user, c->lane[li].end, 0));
         }
         done = pairs * 2;
+        // an even number of steps: dup is back in a, with its V in the first array
+        if (split_c0 && ((rc = chain_fold(c, a, c->chain_v, user)) || (rc = chain_fold(c, acc, c->chain_v + 2 * vview, user)))) return rc;
     }
     const ckks_view *src = a, *dst = b;
     for (; done < count; done++) {
-        if ((rc = one(src, dst, user, false, 0, 0, B))) return rc;
+        if ((rc = one(src, dst, user, false, 0, 0, B, -1))) return rc;
         const ckks_view *t = src;
         src = dst;
         dst = t;
@@ -1367,7 +1450,7 @@ extern "C" int ckks_rotate_plan_hoisted(ckks_ctx *c, const ckks_rotplan *p, cons
             DView minu{ACC, 2 * (u64)(L + 1) * N, (u64)(L + 1) * N};                                                \
             k_hoist_mac<LN><<<dim3(G::ROW_TILES, L + 1, bc), NTT_THREADS, 0, st>>>(T1, rt, ACC, L, c->t);           \
             LAUNCH_CHECK(c);                                                                                        \
-            k_md_invcol_fwdcol<LN><<<dim3(G::COL_TILES, 1, 2 * bc), NTT_THREADS, 0, st>>>(spec, T2, L, K - 1, 1, c->t); \
+            k_md_invcol_fwdcol<LN, false><<<dim3(G::COL_TILES, 1, 2 * bc), NTT_THREADS, 0, st>>>(spec, T2, L, K - 1, 1, ChainV{}, c->t); \
             LAUNCH_CHECK(c);                                                                                        \
             k_md_fwd_row<LN, 2><<<dim3(G::ROW_TILES, L, 2 * bc), NTT_THREADS, 0, st>>>(T2, minu, rt, 2, L, K - 1, c->t); \
             LAUNCH_CHECK(c);                                                                                        \
@@ -1446,7 +1529,7 @@ extern "C" int ckks_rescale(ckks_ctx *c, const ckks_view *in, const ckks_view *o
         LAUNCH_CHECK(c);                                                                                          \
         if (c->fuse) {                                                                                            \
             const int ns3 = pick_split(c->split3, G::COL_TILES * S * bc, Lo);                                     \
-            launch_pdl(k_md_invcol_fwdcol<LN>, dim3(G::COL_TILES, ns3, bc * S), st, Rz, T2, Lo, Lo, ns3, tr);   \
+            launch_pdl(k_md_invcol_fwdcol<LN, false>, dim3(G::COL_TILES, ns3, bc * S), st, Rz, T2, Lo, Lo, ns3, ChainV{}, tr); \
             LAUNCH_CHECK(c);                                                                                      \
         } else {                                                                                                  \
             launch_pdl(k_inv_col<LN, true>, dim3(G::COL_TILES, S, bc), st, dR, dR, 1, Lo, tr);          \

@@ -971,12 +971,34 @@ __global__ void __launch_bounds__(NTT_THREADS, 5) k_md_fwd_col(DView R, u64 *T2,
     for (int e = 0; e < 8; e++) out[col_fine_idx<LOGN>(c0, e)] = x[e];
 }
 
+// Rotate-and-sum chains carry c0 split in two (DESIGN.md section 4): c0 = A - P^-1 NTT(V) mod q_j, with A in NTT form
+// (written by k_md_fwd_row<MODE 3>) and V ONE signed integer polynomial in coefficient order, the same for every prime
+// -- the mod-down remainders w = r' - half of all steps so far, carried through the Galois maps.  V is stored as
+// 128-bit two's-complement words (lo, hi), one per coefficient: |V| < count * 2^60 and |sum of V| < count^2 * 2^60.
+struct ChainV {
+    const u64 *vin;   // [entry][N][2] V of the step's source ciphertext
+    u64 *vout;        // V of the step's destination
+    u64 *vacc;        // V of the accumulator (+= vout)
+    unsigned ginv;    // g^-1 mod 2N: coefficient k of sigma(V) is +-V[k g^-1 mod 2N]
+};
+__device__ __forceinline__ __int128 ld_i128(const ulonglong2 &v) {
+    return (__int128)(((unsigned __int128)v.y << 64) | v.x);
+}
+__device__ __forceinline__ ulonglong2 st_i128(__int128 x) {
+    return make_ulonglong2((u64)x, (u64)((unsigned __int128)x >> 64));
+}
+
 // (6+7) fused: inverse column pass of the divisor-prime limb (special prime P for a key switch, last data
 // prime for a rescale; its row pass is in R), the "+ half" of SEAL's rounding, and on the same tile the
 // column pass of (r' mod q_j) - (half mod q_j) for every remaining prime j.
 // grid: (COL_TILES, nsplit, instances); part p handles j = p, p + nsplit, ...
-template <int LOGN>
-__global__ void __launch_bounds__(NTT_THREADS, V_OCC_COL) k_md_invcol_fwdcol(DView R, u64 *T2, int Lout, int a, int nsplit, Tables t) {
+// CHAIN (Galois key switch of a rotate-and-sum chain, instance z = 2 entry + k): the c0 instances (k = 0) transform
+// nothing forward and write no T2; they fold w = r' - half into the chain's coefficient-form remainder instead,
+//     V_out[k] = sigma(V_in)[k] + w[k],   V_acc[k] += V_out[k]
+// (ChainV above); the c1 instances are unchanged.
+template <int LOGN, bool CHAIN>
+__global__ void __launch_bounds__(NTT_THREADS, V_OCC_COL) k_md_invcol_fwdcol(DView R, u64 *T2, int Lout, int a, int nsplit, ChainV cv,
+                                                                           Tables t) {
     typedef NttGeo<LOGN> G;
     __shared__ u64 smem[2][NTT_TILE];
     const int part = blockIdx.y, z = blockIdx.z;
@@ -1000,6 +1022,34 @@ __global__ void __launch_bounds__(NTT_THREADS, V_OCC_COL) k_md_invcol_fwdcol(DVi
         inv_col_pass<LOGN>(v, t.twi + (size_t)a * G::N, ma, smem[0]);
 #pragma unroll
         for (int e = 0; e < 8; e++) v[e] = csub(csub(csub(v[e], ma.p2), ma.p) + half, ma.p);
+    }
+    if (CHAIN && (z & 1) == 0) {
+        if (part != 0) return;
+        const size_t eo = (size_t)(z >> 1) * G::N;
+        const ulonglong2 *__restrict__ vi = reinterpret_cast<const ulonglong2 *>(cv.vin) + eo;
+        ulonglong2 *__restrict__ vo = reinterpret_cast<ulonglong2 *>(cv.vout) + eo;
+        ulonglong2 *__restrict__ va = reinterpret_cast<ulonglong2 *>(cv.vacc) + eo;
+        PDL_LATE();
+#pragma unroll
+        for (int h = 0; h < 8; h += 4) {   // four coefficients at a time: 64 registers hold 8 residues + 4 x 2 int128 loads
+            ulonglong2 src[4], acc[4];
+#pragma unroll
+            for (int e = 0; e < 4; e++) {
+                const unsigned k = col_coarse_idx<LOGN>(c0, h + e);
+                src[e] = vi[(k * cv.ginv) & (G::N - 1)];
+                acc[e] = va[k];
+            }
+#pragma unroll
+            for (int e = 0; e < 4; e++) {
+                const unsigned k = col_coarse_idx<LOGN>(c0, h + e);
+                __int128 x = ld_i128(src[e]);
+                if ((k * cv.ginv) & G::N) x = -x;   // source index >= N: X^N = -1
+                x += (__int128)((long long)v[h + e] - (long long)half);
+                vo[k] = st_i128(x);
+                va[k] = st_i128(ld_i128(acc[e]) + x);
+            }
+        }
+        return;
     }
     PDL_LATE();
     int buf = 1;
@@ -1034,6 +1084,9 @@ __global__ void __launch_bounds__(NTT_THREADS, V_OCC_COL) k_md_invcol_fwdcol(DVi
 //     out = (minuend - NTT(u)) * q_a^-1  [+ base]          mod q_j
 // MODE 0 (rescale): no base.  MODE 1 (relinearize): base = in[b][k].  MODE 2 (Galois):
 // base = permuted in[b][0] for k == 0 and nothing for k == 1 (SEAL wipes c1 before switching).
+// MODE 3 (Galois step of a rotate-and-sum chain whose c0 is carried split, see ChainV): as MODE 2, except that the
+// k == 0 CTAs read no T2 and run no transform -- they compute A_out = minuend * q_a^-1 + sigma(A_in); the remainder
+// that MODE 2 subtracts here went into V (k_md_invcol_fwdcol<CHAIN>).
 // z = b*S + s enumerates (ciphertext, poly).
 #ifndef V_MDROW_OCC
 #define V_MDROW_OCC 4
@@ -1045,13 +1098,41 @@ __global__ void __launch_bounds__(NTT_THREADS, V_MDROW_OCC) k_md_fwd_row(const u
     const int j = blockIdx.y, z = blockIdx.z, b = z / S, s = z % S;
     const KsSel sl = route_sel(rt, b);
     const DView base = rt.v[sl.src], dst = rt.v[sl.dst];
-    const uint32_t *__restrict__ perm = MODE == 2 ? route_perm(rt, sl) : nullptr;
+    const uint32_t *__restrict__ perm = MODE >= 2 ? route_perm(rt, sl) : nullptr;
     const u64 *in = T2 + ((u64)z * Lout + j) * G::N;
     const ModConst m = load_mod(t, j);
     const u64 qi = t.inv[a * t.K + j], qis = t.invs[a * t.K + j];
     const int t0 = blockIdx.x * NTT_TILE;
     u64 x[8];
     const FpConst f = t.fp[j];
+    if (MODE == 3 && s == 0) {
+        const u64 *mi = minuend.data + b * minuend.bs + (u64)j * G::N + t0 + 8 * threadIdx.x;
+        u64 *out = dst.data + sl.entry * dst.bs + (u64)j * G::N + t0 + 8 * threadIdx.x;
+        u64 *ap = rt.accv.data + sl.entry * rt.accv.bs + (u64)j * G::N + t0 + 8 * threadIdx.x;
+        const u64 *bp = base.data + sl.sentry * base.bs + (u64)j * G::N;
+        unsigned ix[8];
+        u64 mv[8], bv[8], av[8];
+        load_perm8(ix, perm + t0 + 8 * threadIdx.x);
+        pdl_wait();
+        load8(mv, mi);
+#pragma unroll
+        for (int e = 0; e < 8; e++) bv[e] = bp[ix[e]];
+        load8(av, ap);
+        PDL_LATE();
+        if (f.ok != 0.0) {
+            const double qd = fp_from_u64(qi);
+#pragma unroll
+            for (int e = 0; e < 8; e++) x[e] = fp_to_canonical(__dadd_rn(fp_mulmod(fp_from_u64(mv[e]), qd, f), fp_from_u64(bv[e])), f);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 8; e++) x[e] = addmod(csub(csub(shoup_lazy(mv[e], qi, qis, m.negp), m.p2), m.p), bv[e], m.p);
+        }
+        store8(out, x);
+#pragma unroll
+        for (int e = 0; e < 8; e++) av[e] = addmod(av[e], x[e], m.p);
+        store8(ap, av);
+        return;
+    }
     pdl_wait();
 #pragma unroll
     for (int e = 0; e < 8; e++) x[e] = VLOAD(e, in[t0 + row_strided_li<LOGN>(e)]);
@@ -1083,7 +1164,7 @@ __global__ void __launch_bounds__(NTT_THREADS, V_MDROW_OCC) k_md_fwd_row(const u
 #endif
         if (MODE == 1) {
             load8(bv, base.data + sl.sentry * base.bs + s * base.ps + (u64)j * G::N + t0 + 8 * threadIdx.x);
-        } else if (MODE == 2) {
+        } else if (MODE >= 2) {
             if (s == 0) {
                 unsigned ix[8];
                 load_perm8(ix, perm + t0 + 8 * threadIdx.x);
@@ -1103,7 +1184,7 @@ __global__ void __launch_bounds__(NTT_THREADS, V_MDROW_OCC) k_md_fwd_row(const u
 #pragma unroll
         for (int e = 0; e < 8; e++) {
             double r = fp_mulmod(__dadd_rn(fp_from_u64(mv[e]), -xd[e]), qd, f);
-            if (MODE == 1 || (MODE == 2 && s == 0)) r = __dadd_rn(r, fp_from_u64(bv[e]));
+            if (MODE == 1 || (MODE >= 2 && s == 0)) r = __dadd_rn(r, fp_from_u64(bv[e]));
             x[e] = fp_to_canonical(r, f);
         }
     } else {
@@ -1111,12 +1192,12 @@ __global__ void __launch_bounds__(NTT_THREADS, V_MDROW_OCC) k_md_fwd_row(const u
         for (int e = 0; e < 8; e++) {
             u64 r = shoup_lazy(mv[e] + p9 - x[e], qi, qis, m.negp);
             r = csub(csub(r, m.p2), m.p);
-            if (MODE == 1 || (MODE == 2 && s == 0)) r = addmod(r, bv[e], m.p);
+            if (MODE == 1 || (MODE >= 2 && s == 0)) r = addmod(r, bv[e], m.p);
             x[e] = r;
         }
     }
     store8(out, x);
-    if (MODE == 2 && rt.has_acc) {
+    if (MODE >= 2 && rt.has_acc) {
         // add_inplace(acc, rotated) of the rotate-and-sum loop (helper.h:472-476), fused
         u64 *ap = rt.accv.data + sl.entry * rt.accv.bs + s * rt.accv.ps + (u64)j * G::N + t0 + 8 * threadIdx.x;
         u64 av[8];
@@ -1125,6 +1206,19 @@ __global__ void __launch_bounds__(NTT_THREADS, V_MDROW_OCC) k_md_fwd_row(const u
         for (int e = 0; e < 8; e++) av[e] = addmod(av[e], x[e], m.p);
         store8(ap, av);
     }
+}
+
+// End of a split rotate-and-sum chain, first of three launches (then the forward NTT and a modular add into c0): the
+// coefficient-form residues -P^-1 (V mod q_j) of entry z, limb j, with P = q_a.  Exact 128-bit integer arithmetic; it runs
+// once per chain, so the software division is of no consequence.  grid (ceil(N / 256), L, entries).
+__global__ void __launch_bounds__(256) k_chain_fold_residues(const u64 *V, u64 *out, int L, int a, int n, Tables t) {
+    const int j = blockIdx.y, z = blockIdx.z, k = blockIdx.x * 256 + threadIdx.x;
+    if (k >= n) return;
+    const __int128 v = ld_i128(reinterpret_cast<const ulonglong2 *>(V)[(size_t)z * n + k]);
+    const u64 p = t.mod[j].p;
+    const u64 r = (u64)((unsigned __int128)(v < 0 ? -v : v) % p);   // |V| mod p
+    const u64 neg = v < 0 ? r : (r ? p - r : 0);                      // -V mod p
+    out[((size_t)z * L + j) * n + k] = (u64)((unsigned __int128)neg * t.inv[a * t.K + j] % p);
 }
 
 // =============================================================================== hoisted rotations (SURVEY 8 f4)
