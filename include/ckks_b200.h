@@ -203,6 +203,27 @@ int ckks_rotate_plan(ckks_ctx *ctx, const ckks_rotplan *plan, const ckks_view *i
  * to SEAL's (SEAL permutes before lifting the digits), so the reference-parity path never calls this. */
 int ckks_rotate_plan_hoisted(ckks_ctx *ctx, const ckks_rotplan *plan, const ckks_view *in, const ckks_view *out, ckks_stream s);
 
+/* Opt-in, double hoisting: plaintext-weighted sums of rotations with ONE digit decomposition per input and ONE mod-down
+ * per output,
+ *     out[o] = sum_{z in [first[o], first[o+1])} pt[pt_idx[z]] (.) rot(in[in_idx[z]], steps[z])      (pt_idx -1: weight 1)
+ * first[] has n_out + 1 non-decreasing entries from 0 to n_terms (the term table is sorted by output).
+ * The key inner product of every non-zero step is taken in the extended basis Q_L u {P}, multiplied there by the
+ * plaintext (pts are encoded at the key level: all K primes, limb K-1 = residue mod P), summed over the output's terms
+ * and divided by P once (the key-switch mod-down, rounding as set by ckks_ctx_set_rounding).  The c0 and step-0 terms are
+ * added after the mod-down.  Every non-zero step needs its own Galois key, |step| < N/2.  The result decrypts like
+ * ckks_rotate_plan_hoisted followed by ckks_multiply_plain_sum within key-switch noise; it is bit-identical to neither,
+ * so the reference-parity path never calls this.  The plan compiles the term table once; the run refreshes the key
+ * tables like ckks_rotate_plan.  in: n_in size-2 ciphertexts at L <= K-1 limbs; pts: n_pt plaintexts at K limbs (may be
+ * NULL when no term has a plaintext); out: n_out ciphertexts at L limbs, not overlapping in or pts. */
+typedef struct ckks_rmsplan ckks_rmsplan;
+int ckks_rmsplan_create(ckks_ctx *ctx, ckks_keyset *ks, int n_in, int n_pt, int n_out, const int *first, int n_terms,
+                        const int *in_idx, const int *steps, const int *pt_idx, ckks_rmsplan **out);
+void ckks_rmsplan_destroy(ckks_rmsplan *plan);
+uint64_t ckks_rmsplan_inner_products(const ckks_rmsplan *plan); /* key inner products per run (terms with a non-zero step) */
+uint64_t ckks_rmsplan_mod_downs(const ckks_rmsplan *plan);      /* mod-downs per run (outputs with a non-zero step) */
+int ckks_rotate_multiply_sum_hoisted(ckks_ctx *ctx, const ckks_rmsplan *plan, const ckks_view *in, const ckks_view *pts,
+                                     const ckks_view *out, ckks_stream s);
+
 /* The rotate-and-sum loop of cipher_dot_product (helper.h:472-476), `count` times:
  *     dup = rotate_vector(dup, steps);  acc = acc + dup
  * on a batch of independent ciphertexts.  `a` holds dup on entry; the rotation ping-pongs between

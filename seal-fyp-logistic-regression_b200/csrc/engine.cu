@@ -1461,6 +1461,253 @@ extern "C" int ckks_rotate_plan_hoisted(ckks_ctx *c, const ckks_rotplan *p, cons
     return CKKS_OK;
 }
 
+// ------------------------------------------------------------------------------------ double-hoisted rotate-multiply-sum
+// out[o] = sum_{z in o} pt[p_z] (.) rot(in[a_z], step_z) with one decomposition per input and one mod-down per output
+// (kernels.cuh, "double-hoisted rotate-multiply-sum").  Same decrypted values as rotate_plan_hoisted + multiply_plain_sum
+// within key-switch noise, bit-identical to neither: an explicit opt-in mode.
+struct ckks_rmsplan {
+    ckks_ctx *ctx;
+    ckks_keyset *ks;
+    int n_in = 0, n_pt = 0, n_out = 0;
+    bool uses_pt = false;
+    std::vector<int> ks_out;          // outputs with a non-zero step: one mod-down each, in output order
+    // work split for each level L (index L): per key-switched output k, its units [unit_first[k], unit_first[k+1]), partials
+    // [part_first[k], ...) and folds [fold_first[k], ...)
+    struct Split {
+        std::vector<int> unit_first, part_first, fold_first;
+        RmsUnit *d_units = nullptr;
+        RmsFold *d_folds = nullptr;
+    };
+    std::vector<Split> split;
+    int *d_first = nullptr;
+    RmsTerm *d_terms = nullptr, *d_nz = nullptr;
+    KsSel *d_sel = nullptr;           // mod-down routing: launch slot k -> output ks_out[k] of `out`
+    uint64_t inner_products = 0;
+};
+
+extern "C" void ckks_rmsplan_destroy(ckks_rmsplan *p) {
+    if (!p) return;
+    for (auto &s : p->split) {
+        cudaFree(s.d_units);
+        cudaFree(s.d_folds);
+    }
+    cudaFree(p->d_first);
+    cudaFree(p->d_terms);
+    cudaFree(p->d_nz);
+    cudaFree(p->d_sel);
+    delete p;
+}
+
+template <typename T>
+static bool rms_upload(T **dst, const std::vector<T> &v) {
+    if (v.empty()) return true;
+    return cudaMalloc((void **)dst, v.size() * sizeof(T)) == cudaSuccess &&
+           cudaMemcpy(*dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice) == cudaSuccess;
+}
+
+extern "C" int ckks_rmsplan_create(ckks_ctx *c, ckks_keyset *ks, int n_in, int n_pt, int n_out, const int *first,
+                                   int n_terms, const int *in_idx, const int *steps, const int *pt_idx, ckks_rmsplan **out) {
+    if (!c || !ks || !first || !out || n_in < 1 || n_pt < 0 || n_out < 1)
+        return fail(CKKS_ERR_INVALID, "rotate_multiply_sum plan: bad arguments");
+    if (n_out > 32767) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum plan: more than 32767 outputs");
+    if (first[0] != 0) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum plan: first[0] must be 0");
+    for (int o = 0; o < n_out; o++)
+        if (first[o + 1] < first[o]) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum plan: first[] must be non-decreasing");
+    if (first[n_out] != n_terms) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum plan: first[] must cover every term");
+    const int T = n_terms;
+    if (T > 0 && (!in_idx || !steps || !pt_idx)) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum plan: null term table");
+    int rc;
+    if ((rc = sync_key_tables(ks))) return rc;
+    std::vector<RmsTerm> terms(T);
+    for (int z = 0; z < T; z++) {
+        if (in_idx[z] < 0 || in_idx[z] >= n_in) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum plan: input index out of range");
+        if (pt_idx[z] < -1 || pt_idx[z] >= n_pt) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum plan: plaintext index out of range");
+        if (steps[z] <= -c->n / 2 || steps[z] >= c->n / 2) return fail(CKKS_ERR_INVALID, "step count too large");
+        terms[z] = RmsTerm{in_idx[z], -1, pt_idx[z], 0};
+        if (steps[z] == 0) continue;
+        const uint64_t g = ckks::galois_elt_from_step(c->log_n, steps[z]);
+        if (!g) return fail(CKKS_ERR_INVALID, "step count too large");
+        if (!ks->galois.count(g))
+            return fail(CKKS_ERR_INVALID, "Galois key not present (double hoisting needs a key for every step itself)");
+        terms[z].slot = ks->slot_of.at(g);
+    }
+    ckks_rmsplan *p = new ckks_rmsplan;
+    p->ctx = c;
+    p->ks = ks;
+    p->n_in = n_in;
+    p->n_pt = n_pt;
+    p->n_out = n_out;
+    std::vector<RmsTerm> nz;
+    std::vector<int> nz_first(1, 0);
+    std::vector<KsSel> sel;
+    for (int o = 0; o < n_out; o++) {
+        for (int z = first[o]; z < first[o + 1]; z++) {
+            p->uses_pt |= terms[z].p >= 0;
+            if (terms[z].slot >= 0) nz.push_back(terms[z]);
+        }
+        if ((int)nz.size() == nz_first.back()) continue;
+        nz_first.push_back((int)nz.size());
+        p->ks_out.push_back(o);
+        KsSel e;
+        e.entry = e.sentry = o;
+        e.slot = 0;
+        e.src = e.dst = 1;
+        sel.push_back(e);
+    }
+    p->inner_products = nz.size();
+    // Work split, chosen from the table shape: a unit costs ROW_TILES x (L + 1) CTAs; aim at about two waves of the inner
+    // product kernel (2 CTAs per SM) and split every output whose term list is longer than the resulting segment
+    int sms = 148;
+    if (cudaSetDevice(c->device) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device) != cudaSuccess) {
+        ckks_rmsplan_destroy(p);
+        return fail(CKKS_ERR_CUDA, "rotate_multiply_sum plan: device query failed");
+    }
+    p->split.resize(c->K);
+    const int nks = (int)p->ks_out.size();
+    for (int L = 1; L < c->K && nks > 0; L++) {
+        ckks_rmsplan::Split &s = p->split[L];
+        const int per_unit = (c->n / NTT_TILE) * (L + 1);
+        const int target = std::max(1, (4 * sms + per_unit - 1) / per_unit);
+        const int seg = std::min(RMS_SEG_MAX, std::max(1, ((int)nz.size() + target - 1) / target));
+        std::vector<RmsUnit> units;
+        std::vector<RmsFold> folds;
+        int parts = 0;
+        for (int k = 0; k < nks; k++) {
+            s.unit_first.push_back((int)units.size());
+            s.part_first.push_back(parts);
+            s.fold_first.push_back((int)folds.size());
+            const int tb = nz_first[k], n = nz_first[k + 1] - tb;
+            const int S = (n + seg - 1) / seg, len = (n + S - 1) / S;
+            if (S == 1) {
+                units.push_back(RmsUnit{k, -1, tb, tb + n});
+                continue;
+            }
+            folds.push_back(RmsFold{k, parts, S, 0});
+            for (int q = 0; q < S; q++) units.push_back(RmsUnit{k, parts++, tb + q * len, std::min(tb + n, tb + (q + 1) * len)});
+        }
+        s.unit_first.push_back((int)units.size());
+        s.part_first.push_back(parts);
+        s.fold_first.push_back((int)folds.size());
+        if (!rms_upload(&s.d_units, units) || !rms_upload(&s.d_folds, folds)) {
+            ckks_rmsplan_destroy(p);
+            return fail(CKKS_ERR_CUDA, "rotate_multiply_sum plan: device allocation failed");
+        }
+    }
+    if (!rms_upload(&p->d_first, std::vector<int>(first, first + n_out + 1)) || !rms_upload(&p->d_terms, terms) ||
+        !rms_upload(&p->d_nz, nz) || !rms_upload(&p->d_sel, sel)) {
+        ckks_rmsplan_destroy(p);
+        return fail(CKKS_ERR_CUDA, "rotate_multiply_sum plan: device allocation failed");
+    }
+    *out = p;
+    return CKKS_OK;
+}
+extern "C" uint64_t ckks_rmsplan_inner_products(const ckks_rmsplan *p) { return p->inner_products; }
+extern "C" uint64_t ckks_rmsplan_mod_downs(const ckks_rmsplan *p) { return p->ks_out.size(); }
+
+// words a view spans (its last entry's last active limb included)
+static size_t view_span(const ckks_ctx *c, const ckks_view *v) {
+    return (size_t)(v->batch - 1) * v->batch_stride + (size_t)(v->size - 1) * v->poly_stride + (size_t)v->limbs * c->n;
+}
+static bool views_overlap(const ckks_ctx *c, const ckks_view *a, const ckks_view *b) {
+    const uint64_t *a0 = a->data, *b0 = b->data;
+    return a0 < b0 + view_span(c, b) && b0 < a0 + view_span(c, a);
+}
+
+extern "C" int ckks_rotate_multiply_sum_hoisted(ckks_ctx *c, const ckks_rmsplan *p, const ckks_view *in, const ckks_view *pts,
+                                                const ckks_view *out, ckks_stream s) {
+    int rc;
+    if (!p) return fail(CKKS_ERR_INVALID, "null plan");
+    if ((rc = check_view(c, in, "encrypted")) || (rc = check_view(c, out, "out"))) return rc;
+    if (in->size != 2 || out->size != 2) return fail(CKKS_ERR_INVALID, "encrypted size must be 2");
+    if (in->limbs > c->K - 1) return fail(CKKS_ERR_INVALID, "encrypted is not valid for encryption parameters");
+    if (in->batch != p->n_in) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: in batch differs from the plan's inputs");
+    if (out->batch != p->n_out) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: out batch differs from the plan's outputs");
+    if (out->limbs != in->limbs) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: out level differs from in");
+    if (views_overlap(c, out, in)) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: out must not alias in");
+    if (p->uses_pt) {
+        if ((rc = check_view(c, pts, "plain"))) return rc;
+        if (pts->size != 1) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: plaintexts must have size 1");
+        if (pts->limbs != c->K) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: plaintexts must be encoded at the key level (all K primes)");
+        if (pts->batch != p->n_pt) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: pts batch differs from the plan's plaintexts");
+        if (views_overlap(c, out, pts)) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: out must not alias pts");
+    }
+    CU(cudaSetDevice(c->device));
+    // a Galois key replaced after the plan was compiled has a new engine-owned copy: refresh the device-side key table
+    if ((rc = sync_key_tables(p->ks))) return rc;
+    cudaStream_t st = (cudaStream_t)s;
+    const int L = in->limbs, K = c->K, nks = (int)p->ks_out.size();
+    const size_t N = c->n;
+    const DView vin = dv(in), vout = dv(out), vpt = p->uses_pt ? dv(pts) : DView{};
+    const uint32_t *const *perm_tab = p->ks->d_perm_tab;
+    const u64 *const *key_tab = p->ks->d_key_tab;
+    // workspace: D and the decomposition of every input, then per chunk of key-switched outputs ACC, T2 and the partials
+    const size_t fixed = (size_t)p->n_in * N * ((size_t)L + (size_t)L * (L + 1));
+    const size_t per_out = N * (2 * (size_t)(L + 1) + 2 * (size_t)L), per_part = N * 2 * (size_t)(L + 1);
+    const ckks_rmsplan::Split &sp = p->split[L];
+    auto cost = [&](int k) { return per_out + per_part * (size_t)(sp.part_first[k + 1] - sp.part_first[k]); };
+    const size_t budget = c->ws_cap / 8 > fixed ? c->ws_cap / 8 - fixed : 0;
+    std::vector<int> chunk(1, 0);
+    size_t most = 0;
+    for (int k = 0; k < nks;) {
+        size_t words = cost(k++);
+        while (k < nks && words + cost(k) <= budget) words += cost(k++);
+        chunk.push_back(k);
+        most = std::max(most, words);
+    }
+    if (nks && (rc = ensure_ws(c, (fixed + most) * 8))) return rc;
+    u64 *D = c->ws, *T1 = D + (size_t)p->n_in * L * N, *WS = T1 + (size_t)p->n_in * L * (L + 1) * N;
+    KsRoute r0{};      // decomposition of every input: no permutation, no per-entry routing
+    r0.v[0] = vin;
+    r0.tgt_poly = 1;
+    KsRoute rt{};      // mod-down: base and destination are `out`, launch slot k -> output ks_out[k]
+    rt.v[0] = rt.v[1] = rt.v[2] = vout;
+    rt.sel = p->d_sel;
+    int sms = 148;
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+#define RUN(LN)                                                                                                              \
+    {                                                                                                                        \
+        typedef NttGeo<LN> G;                                                                                                \
+        k_rms_base<LN><<<dim3(G::ROW_TILES, L, 2 * p->n_out), NTT_THREADS, 0, st>>>(vin, vpt, vout, p->d_first, p->d_terms,   \
+                                                                                     perm_tab, c->t);                        \
+        LAUNCH_CHECK(c);                                                                                                     \
+        if (nks) {                                                                                                           \
+            k_ks_intt_row<LN, false><<<dim3(G::ROW_TILES, L, p->n_in), NTT_THREADS, 0, st>>>(r0, D, L, c->t);                \
+            LAUNCH_CHECK(c);                                                                                                 \
+            k_ks_invcol_modup<LN><<<dim3(G::COL_TILES, L, p->n_in), NTT_THREADS, 0, st>>>(D, T1, L, 1, c->t);                \
+            LAUNCH_CHECK(c);                                                                                                 \
+            k_hoist_finish<LN><<<dim3(G::ROW_TILES, L *(L + 1), p->n_in), NTT_THREADS, 0, st>>>(T1, vin, L, c->t);           \
+            LAUNCH_CHECK(c);                                                                                                 \
+        }                                                                                                                    \
+        for (size_t q = 0; q + 1 < chunk.size(); q++) {                                                                      \
+            const int k0 = chunk[q], k1 = chunk[q + 1], nc = k1 - k0;                                                        \
+            const int u0 = sp.unit_first[k0], nu = sp.unit_first[k1] - u0;                                                   \
+            const int f0 = sp.fold_first[k0], nf = sp.fold_first[k1] - f0;                                                   \
+            u64 *ACC = WS, *T2 = ACC + (size_t)nc * 2 * (L + 1) * N, *PART = T2 + (size_t)nc * 2 * L * N;                    \
+            k_rms_mac<LN><<<dim3(G::ROW_TILES, L + 1, nu), NTT_THREADS, 0, st>>>(T1, sp.d_units + u0, p->d_nz, vpt, perm_tab, \
+                                                                                 key_tab, ACC, PART, k0, sp.part_first[k0], L, c->t); \
+            LAUNCH_CHECK(c);                                                                                                 \
+            if (nf) {                                                                                                        \
+                k_rms_fold<LN><<<dim3(G::ROW_TILES, L + 1, nf), NTT_THREADS, 0, st>>>(sp.d_folds + f0, PART, ACC, k0,        \
+                                                                                      sp.part_first[k0], L, c->t);           \
+                LAUNCH_CHECK(c);                                                                                             \
+            }                                                                                                                \
+            /* a few outputs leave most SMs idle in the column pass: split the target primes over more CTAs */               \
+            const int ns = std::max(1, std::min(L, sms / (2 * nc * G::COL_TILES)));                                         \
+            DView spec{ACC + (size_t)L * N, (u64)(L + 1) * N, 0};                                                            \
+            DView minu{ACC, 2 * (u64)(L + 1) * N, (u64)(L + 1) * N};                                                         \
+            k_md_invcol_fwdcol<LN, false><<<dim3(G::COL_TILES, ns, 2 * nc), NTT_THREADS, 0, st>>>(spec, T2, L, K - 1, ns,    \
+                                                                                                  ChainV{}, c->t);           \
+            LAUNCH_CHECK(c);                                                                                                 \
+            rt.b0 = k0;                                                                                                      \
+            k_md_fwd_row<LN, 1><<<dim3(G::ROW_TILES, L, 2 * nc), NTT_THREADS, 0, st>>>(T2, minu, rt, 2, L, K - 1, c->t);     \
+            LAUNCH_CHECK(c);                                                                                                 \
+        }                                                                                                                    \
+    }
+    DISPATCH_LOGN(c, RUN)
+#undef RUN
+    return CKKS_OK;
+}
+
 // ------------------------------------------------------------------------------------ fused products
 // out[g] = sum_i a[g*T + i] (.) b[i], g < groups, T = b->batch
 static int mul_sum(ckks_ctx *c, bool plain, const ckks_view *a, const ckks_view *b, int groups, const ckks_view *o,

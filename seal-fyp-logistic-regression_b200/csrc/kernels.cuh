@@ -1231,17 +1231,18 @@ __global__ void __launch_bounds__(256) k_chain_fold_residues(const u64 *V, u64 *
 //
 // (h1) finish the mod-up transform: T1[i][jj] holds the column pass (k_ks_invcol_modup); run the row pass and store the
 // canonical NTT values in place; the slot of the digit's own prime receives the NTT-form limb of c1 itself.
+// blockIdx.z = input ciphertext: T1 of input b starts at b * L * (L + 1) * N.
 template <int LOGN>
 __global__ void __launch_bounds__(NTT_THREADS, 4) k_hoist_finish(u64 *T1, DView ct, int L, Tables t) {
     typedef NttGeo<LOGN> G;
     __shared__ u64 smem[NTT_TILE];
-    const int i = blockIdx.y / (L + 1), jj = blockIdx.y % (L + 1);
+    const int i = blockIdx.y / (L + 1), jj = blockIdx.y % (L + 1), b = blockIdx.z;
     const int pj = jj == L ? t.K - 1 : jj;
-    u64 *tile = T1 + ((u64)i * (L + 1) + jj) * G::N + (u64)blockIdx.x * NTT_TILE;
+    u64 *tile = T1 + (((u64)b * L + i) * (L + 1) + jj) * G::N + (u64)blockIdx.x * NTT_TILE;
     const int t0 = blockIdx.x * NTT_TILE;
     u64 x[8];
     if (pj == i) {
-        load8(x, ct.data + ct.ps + (u64)i * G::N + t0 + 8 * threadIdx.x);   // poly 1, limb i
+        load8(x, ct.data + b * ct.bs + ct.ps + (u64)i * G::N + t0 + 8 * threadIdx.x);   // poly 1, limb i
         store8(tile + 8 * threadIdx.x, x);
         return;
     }
@@ -1361,6 +1362,258 @@ __global__ void __launch_bounds__(NTT_THREADS, 2) k_hoist_mac(const u64 *T1F, Ks
     }
     store8(o0 + 8 * threadIdx.x, r0);
     store8(o1 + 8 * threadIdx.x, r1);
+}
+
+// =============================================================================== double-hoisted rotate-multiply-sum
+//     out[o] = sum_{z in o} pt[p_z] (.) rot(in[a_z], step_z)
+// with one digit decomposition per input (k_ks_intt_row -> k_ks_invcol_modup -> k_hoist_finish) and ONE mod-down per
+// output: the key inner products u_z of all terms of an output are multiplied by their plaintext in the extended basis
+// Q_L u {P} (the plaintexts are encoded at the key level, limb K-1 holds the residue mod P) and summed there,
+//     ACC_o[k] = sum_{z in o, step != 0} w_z (.) sum_i sigma_z(D_i) (.) ksk_z[i][k],
+// and out_o[k] = ModDown_P(ACC_o[k]) + base_o[k], where base_o (k_rms_base) holds the c0 terms sum w_z (.) sigma_z(c0) and
+// the step-0 terms.  Adding base after the mod-down is exact: P * base has residue 0 mod P.
+// A work unit is a run of non-zero-step terms of one output (the host splits long term lists so that one output does not
+// run on ROW_TILES x (L + 1) CTAs alone); split outputs accumulate into partials that k_rms_fold sums.
+#define RMS_SEG_MAX 64   // terms per work unit: 64 products below p^2 < 2^122 fit the 128-bit accumulator (primes < 2^61)
+struct RmsTerm {
+    int a;      // input ciphertext
+    int slot;   // key / permutation slot of the step in the keyset, -1 for step 0
+    int p;      // plaintext, -1 = weight 1
+    int pad;
+};
+struct RmsUnit {
+    int acc;    // the output's index among the outputs that are key-switched (ACC slot = acc - the chunk's first)
+    int part;   // partial accumulator (slot = part - the chunk's first), -1 = the unit is the whole output
+    int tb, te; // non-zero-step terms [tb, te)
+};
+struct RmsFold {
+    int acc, pb, pn, pad;   // ACC slot, first partial, partial count
+};
+
+// canonical residues r0 / r1 of one tile of limb jj into acc[2][L + 1][N]; the special-prime limb continues into the
+// mod-down INTT's row pass (its column pass follows in k_md_invcol_fwdcol), as in k_hoist_mac
+template <int LOGN>
+__device__ __forceinline__ void rms_store_tile(u64 (&r0)[8], u64 (&r1)[8], u64 *acc, int jj, int L, int t0, const Tables &t, u64 *smem) {
+    typedef NttGeo<LOGN> G;
+    u64 *o0 = acc + (u64)jj * G::N + t0, *o1 = acc + (u64)(L + 1 + jj) * G::N + t0;
+    if (jj != L) {
+        store8(o0 + 8 * threadIdx.x, r0);
+        store8(o1 + 8 * threadIdx.x, r1);
+        return;
+    }
+    const int pj = t.K - 1;
+    const FpConst f = t.fp[pj];
+    if (f.ok != 0.0) {
+        double xd[8];
+#pragma unroll
+        for (int e = 0; e < 8; e++) xd[e] = fp_from_u64(r0[e]);
+        inv_row_pass_fp<LOGN>(xd, t.twid + (size_t)pj * G::N, f, t0, as_fp(smem));
+#pragma unroll
+        for (int e = 0; e < 8; e++) o0[row_strided_li<LOGN>(e)] = fp_bits(xd[e]);
+        __syncthreads();
+#pragma unroll
+        for (int e = 0; e < 8; e++) xd[e] = fp_from_u64(r1[e]);
+        inv_row_pass_fp<LOGN>(xd, t.twid + (size_t)pj * G::N, f, t0, as_fp(smem));
+#pragma unroll
+        for (int e = 0; e < 8; e++) o1[row_strided_li<LOGN>(e)] = fp_bits(xd[e]);
+    } else {
+        const ModConst m = load_mod(t, pj);
+        inv_row_pass<LOGN>(r0, t.twi + (size_t)pj * G::N, m, t0, smem);
+#pragma unroll
+        for (int e = 0; e < 8; e++) o0[row_strided_li<LOGN>(e)] = r0[e];
+        __syncthreads();
+        inv_row_pass<LOGN>(r1, t.twi + (size_t)pj * G::N, m, t0, smem);
+#pragma unroll
+        for (int e = 0; e < 8; e++) o1[row_strided_li<LOGN>(e)] = r1[e];
+    }
+}
+
+// (r1) per work unit: the plaintext-weighted sum of its terms' key inner products, for one tile of limb jj.
+// T1F of input a: [L][L + 1][N] at a * L * (L + 1) * N (canonical NTT values, k_hoist_finish).  Keys: tiled copies.
+// grid (ROW_TILES, L + 1, units of the chunk); ACC: [outputs of the chunk][2][L + 1][N], PART likewise per partial.
+template <int LOGN>
+__global__ void __launch_bounds__(NTT_THREADS, 2) k_rms_mac(const u64 *T1F, const RmsUnit *units, const RmsTerm *terms, DView pt,
+                                                           const uint32_t *const *perm_tab, const u64 *const *key_tab, u64 *ACC,
+                                                           u64 *PART, int out0, int part0, int L, Tables t) {
+    typedef NttGeo<LOGN> G;
+    __shared__ u64 smem[NTT_TILE];
+    const int jj = L - (int)blockIdx.y;   // special-prime limb first: its CTAs also run an inverse row pass
+    const RmsUnit u = units[blockIdx.z];
+    const int K = t.K, pj = jj == L ? K - 1 : jj;
+    const ModConst m = load_mod(t, pj);
+    const FpConst f = t.fp[pj];
+    const int t0 = blockIdx.x * NTT_TILE;
+    const u64 in_words = (u64)L * (L + 1) * G::N, dstride = (u64)(L + 1) * G::N;
+    const int koff = 2 * threadIdx.x;   // tiled key layout: word pair v of thread t at 512 v + 2 t
+    u64 r0[8], r1[8];
+    if (f.ok != 0.0) {   // small prime: products and sums on the FP64 pipe (|sum| < 2 L p per term, < 128 p overall)
+        double a0[8], a1[8];
+#pragma unroll
+        for (int e = 0; e < 8; e++) a0[e] = a1[e] = 0.0;
+        for (int z = u.tb; z < u.te; z++) {
+            const RmsTerm tm = terms[z];
+            const u64 *src = T1F + tm.a * in_words + (u64)jj * G::N;
+            const u64 *ksk = key_tab[tm.slot];
+            unsigned ix[8];
+            load_perm8(ix, perm_tab[tm.slot] + t0 + 8 * threadIdx.x);
+            u64 w[8];
+            if (tm.p >= 0) load8(w, pt.data + tm.p * pt.bs + (u64)pj * G::N + t0 + 8 * threadIdx.x);
+#pragma unroll
+            for (int v = 0; v < 4; v++) {
+                double s0x = 0.0, s0y = 0.0, s1x = 0.0, s1y = 0.0;
+                for (int i = 0; i < L; i++) {
+                    const u64 *d = src + i * dstride;
+                    const ulonglong2 a = __ldg(reinterpret_cast<const ulonglong2 *>(ksk + (((u64)i * 2 + 0) * K + pj) * G::N + t0 + koff) + 256 * v);
+                    const ulonglong2 c = __ldg(reinterpret_cast<const ulonglong2 *>(ksk + (((u64)i * 2 + 1) * K + pj) * G::N + t0 + koff) + 256 * v);
+                    const double x0 = fp_from_u64(d[ix[2 * v]]), x1 = fp_from_u64(d[ix[2 * v + 1]]);
+                    s0x = __dadd_rn(s0x, fp_mulmod(x0, bits_fp(a.x), f));
+                    s0y = __dadd_rn(s0y, fp_mulmod(x1, bits_fp(a.y), f));
+                    s1x = __dadd_rn(s1x, fp_mulmod(x0, bits_fp(c.x), f));
+                    s1y = __dadd_rn(s1y, fp_mulmod(x1, bits_fp(c.y), f));
+                }
+                s0x = fp_reduce(s0x, f); s0y = fp_reduce(s0y, f);
+                s1x = fp_reduce(s1x, f); s1y = fp_reduce(s1y, f);
+                if (tm.p >= 0) {
+                    const double wx = fp_from_u64(w[2 * v]), wy = fp_from_u64(w[2 * v + 1]);
+                    s0x = fp_mulmod(s0x, wx, f); s0y = fp_mulmod(s0y, wy, f);
+                    s1x = fp_mulmod(s1x, wx, f); s1y = fp_mulmod(s1y, wy, f);
+                }
+                a0[2 * v] = __dadd_rn(a0[2 * v], s0x);
+                a0[2 * v + 1] = __dadd_rn(a0[2 * v + 1], s0y);
+                a1[2 * v] = __dadd_rn(a1[2 * v], s1x);
+                a1[2 * v + 1] = __dadd_rn(a1[2 * v + 1], s1y);
+            }
+        }
+#pragma unroll
+        for (int e = 0; e < 8; e++) {
+            r0[e] = fp_to_canonical(a0[e], f);
+            r1[e] = fp_to_canonical(a1[e], f);
+        }
+    } else {   // large prime: 128-bit lazy sums, one Barrett reduction per inner product and one at the end
+        u64 lo0[8], hi0[8], lo1[8], hi1[8];
+#pragma unroll
+        for (int e = 0; e < 8; e++) lo0[e] = hi0[e] = lo1[e] = hi1[e] = 0;
+        for (int z = u.tb; z < u.te; z++) {
+            const RmsTerm tm = terms[z];
+            const u64 *src = T1F + tm.a * in_words + (u64)jj * G::N;
+            const u64 *ksk = key_tab[tm.slot];
+            unsigned ix[8];
+            load_perm8(ix, perm_tab[tm.slot] + t0 + 8 * threadIdx.x);
+            u64 w[8];
+            if (tm.p >= 0) load8(w, pt.data + tm.p * pt.bs + (u64)pj * G::N + t0 + 8 * threadIdx.x);
+#pragma unroll
+            for (int v = 0; v < 4; v++) {
+                u64 l0[2] = {0, 0}, h0[2] = {0, 0}, l1[2] = {0, 0}, h1[2] = {0, 0};
+                for (int i = 0; i < L; i++) {
+                    const u64 *d = src + i * dstride;
+                    const ulonglong2 a = __ldg(reinterpret_cast<const ulonglong2 *>(ksk + (((u64)i * 2 + 0) * K + pj) * G::N + t0 + koff) + 256 * v);
+                    const ulonglong2 c = __ldg(reinterpret_cast<const ulonglong2 *>(ksk + (((u64)i * 2 + 1) * K + pj) * G::N + t0 + koff) + 256 * v);
+                    const u64 x0 = d[ix[2 * v]], x1 = d[ix[2 * v + 1]];
+                    mac128(l0[0], h0[0], x0, a.x);
+                    mac128(l0[1], h0[1], x1, a.y);
+                    mac128(l1[0], h1[0], x0, c.x);
+                    mac128(l1[1], h1[1], x1, c.y);
+                }
+#pragma unroll
+                for (int e = 0; e < 2; e++) {
+                    const u64 u0 = barrett128(l0[e], h0[e], m), u1 = barrett128(l1[e], h1[e], m);
+                    const int q = 2 * v + e;
+                    if (tm.p >= 0) {
+                        mac128(lo0[q], hi0[q], u0, w[q]);
+                        mac128(lo1[q], hi1[q], u1, w[q]);
+                    } else {
+                        lo0[q] += u0; hi0[q] += lo0[q] < u0;
+                        lo1[q] += u1; hi1[q] += lo1[q] < u1;
+                    }
+                }
+            }
+        }
+#pragma unroll
+        for (int e = 0; e < 8; e++) {
+            r0[e] = barrett128(lo0[e], hi0[e], m);
+            r1[e] = barrett128(lo1[e], hi1[e], m);
+        }
+    }
+    if (u.part >= 0) {   // one of several partials of this output: canonical, summed by k_rms_fold
+        u64 *o = PART + (u64)(u.part - part0) * 2 * (L + 1) * G::N + t0 + 8 * threadIdx.x;
+        store8(o + (u64)jj * G::N, r0);
+        store8(o + (u64)(L + 1 + jj) * G::N, r1);
+        return;
+    }
+    rms_store_tile<LOGN>(r0, r1, ACC + (u64)(u.acc - out0) * 2 * (L + 1) * G::N, jj, L, t0, t, smem);
+}
+
+// (r2) outputs split over several work units: sum the partials mod p into ACC.  grid (ROW_TILES, L + 1, folds of the chunk)
+template <int LOGN>
+__global__ void __launch_bounds__(NTT_THREADS, 2) k_rms_fold(const RmsFold *folds, const u64 *PART, u64 *ACC, int out0, int part0, int L, Tables t) {
+    typedef NttGeo<LOGN> G;
+    __shared__ u64 smem[NTT_TILE];
+    const RmsFold fd = folds[blockIdx.z];
+    const int jj = blockIdx.y, pj = jj == L ? t.K - 1 : jj;
+    const u64 p = t.mod[pj].p;
+    const int t0 = blockIdx.x * NTT_TILE;
+    const u64 words = 2 * (u64)(L + 1) * G::N;
+    u64 r0[8], r1[8], x[8];
+#pragma unroll
+    for (int e = 0; e < 8; e++) r0[e] = r1[e] = 0;
+    for (int q = 0; q < fd.pn; q++) {
+        const u64 *src = PART + (u64)(fd.pb - part0 + q) * words + t0 + 8 * threadIdx.x;
+        load8(x, src + (u64)jj * G::N);
+#pragma unroll
+        for (int e = 0; e < 8; e++) r0[e] = addmod(r0[e], x[e], p);
+        load8(x, src + (u64)(L + 1 + jj) * G::N);
+#pragma unroll
+        for (int e = 0; e < 8; e++) r1[e] = addmod(r1[e], x[e], p);
+    }
+    rms_store_tile<LOGN>(r0, r1, ACC + (u64)(fd.acc - out0) * words, jj, L, t0, t, smem);
+}
+
+// (r3) base_o[k] = sum_{z in o} w_z (.) (step_z != 0 ? [k == 0] sigma_z(c0) : c_k), limbs j < L, written to out[o][k]; the
+// mod-down (k_md_fwd_row MODE 1 with base = out) adds ModDown_P(ACC_o[k]) to it.  grid (ROW_TILES, L, 2 * outputs)
+template <int LOGN>
+__global__ void __launch_bounds__(NTT_THREADS) k_rms_base(DView in, DView pt, DView out, const int *first, const RmsTerm *terms,
+                                                         const uint32_t *const *perm_tab, Tables t) {
+    typedef NttGeo<LOGN> G;
+    const int j = blockIdx.y, o = blockIdx.z >> 1, k = blockIdx.z & 1;
+    const int g0 = blockIdx.x * NTT_TILE + 8 * threadIdx.x;
+    const ModConst m = load_mod(t, j);
+    u64 lo[8], hi[8], x[8];
+#pragma unroll
+    for (int e = 0; e < 8; e++) lo[e] = hi[e] = 0;
+    int cnt = 0;
+    for (int z = first[o]; z < first[o + 1]; z++) {
+        const RmsTerm tm = terms[z];
+        if (tm.slot >= 0 && k == 1) continue;   // a rotated c1 is key-switched, not added
+        const u64 *src = in.data + tm.a * in.bs + k * in.ps + (u64)j * G::N;
+        if (tm.slot >= 0) {
+            unsigned ix[8];
+            load_perm8(ix, perm_tab[tm.slot] + g0);
+#pragma unroll
+            for (int e = 0; e < 8; e++) x[e] = src[ix[e]];
+        } else {
+            load8(x, src + g0);
+        }
+        if (tm.p >= 0) {
+            u64 w[8];
+            load8(w, pt.data + tm.p * pt.bs + (u64)j * G::N + g0);
+#pragma unroll
+            for (int e = 0; e < 8; e++) mac128(lo[e], hi[e], x[e], w[e]);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 8; e++) {
+                lo[e] += x[e];
+                hi[e] += lo[e] < x[e];
+            }
+        }
+        if (++cnt == RMS_SEG_MAX) {
+#pragma unroll
+            for (int e = 0; e < 8; e++) lo[e] = barrett128(lo[e], hi[e], m), hi[e] = 0;
+            cnt = 0;
+        }
+    }
+#pragma unroll
+    for (int e = 0; e < 8; e++) x[e] = barrett128(lo[e], hi[e], m);
+    store8(out.data + o * out.bs + k * out.ps + (u64)j * G::N + g0, x);
 }
 
 // Key-switch keys are static: at registration the engine makes a private copy in which, inside every 2048-word

@@ -545,6 +545,36 @@ class Evaluator:
         out.scale = ct.scale
         return out
 
+    def rotate_multiply_sum_hoisted(self, cts, pts, plan, out=None):
+        """Opt-in, double hoisting: out[o] = sum over the plan's terms (a, step, p) of output o of
+        pts[p] (.) rotate_vector(cts[a], step) (p = -1: weight 1), with one digit decomposition per input and one mod-down per
+        output (ckks_rotate_multiply_sum_hoisted).  `pts` are encoded at the key level (limbs = ctx.K) and may be None when
+        no term has a plaintext.  Every term of an output carries cts.scale * pts.scale (or cts.scale for weight 1): "scale
+        mismatch" otherwise.  Decrypts like rotate_plan_hoisted + multiply_plain_sum within key-switch noise; the
+        polynomials differ."""
+        if cts.batch != plan.n_in:
+            raise capi.CkksInvalidArgument("rotate_multiply_sum: in batch differs from the plan's inputs")
+        weighted = plan.weighted_outputs
+        if any(weighted) and pts is None:
+            raise capi.CkksInvalidArgument("rotate_multiply_sum: the plan needs plaintexts")
+        scales = set()
+        for w in plan.term_weights:
+            scales.update(cts.scale * pts.scale if x else cts.scale for x in w)
+        if len(scales) > 1:
+            raise capi.CkksInvalidArgument("scale mismatch")
+        scale = scales.pop() if scales else cts.scale
+        self._scale_ok(scale, cts.limbs)
+        if out is None:
+            out = Ciphertext(self.ctx, torch.empty((plan.n_out, 2, cts.cap, self.ctx.n), dtype=torch.int64,
+                                                   device=cts.data.device), cts.limbs, scale)
+        out.limbs = cts.limbs
+        vi, vo = cts.view(), out.view()
+        vp = pts.view() if pts is not None else None
+        check(self.lib.ckks_rotate_multiply_sum_hoisted(self.h, plan._h, C.byref(vi), C.byref(vp) if vp is not None else None,
+                                                        C.byref(vo), _stream()))
+        out.scale = scale
+        return out
+
     def rotate_sum_chain(self, dup, acc, steps, count, keys, scratch=None):
         """`count` times: dup = rotate_vector(dup, steps); acc += dup (fused, CUDA-graph replayed).
         Returns the Ciphertext that holds dup afterwards (dup's or scratch's storage)."""
@@ -622,6 +652,40 @@ class RotPlan:
         try:
             if self._h:
                 self.ctx.lib.ckks_rotplan_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+
+class RotMulSumPlan:
+    """The term table of Evaluator.rotate_multiply_sum_hoisted, compiled once: `outputs` is a list (one entry per output)
+    of lists of terms (input index, rotation step, plaintext index or -1 for weight 1).  `n_pt` is the plaintext batch the
+    runs pass.  inner_products / mod_downs: key-switch work per run."""
+
+    def __init__(self, ctx, keys, n_in, n_pt, outputs):
+        self.ctx, self.keys = ctx, keys
+        self.outputs = [[(int(a), int(s), int(p)) for a, s, p in terms] for terms in outputs]
+        self.n_in, self.n_pt, self.n_out = int(n_in), int(n_pt), len(self.outputs)
+        flat = [t for terms in self.outputs for t in terms]
+        first = [0]
+        for terms in self.outputs:
+            first.append(first[-1] + len(terms))
+        ints = lambda xs: (C.c_int * max(1, len(xs)))(*xs)
+        h = C.c_void_p()
+        check(ctx.lib.ckks_rmsplan_create(ctx._h, keys._h, self.n_in, self.n_pt, self.n_out, ints(first), len(flat),
+                                          ints([t[0] for t in flat]), ints([t[1] for t in flat]), ints([t[2] for t in flat]),
+                                          C.byref(h)))
+        self._h = h
+        self.inner_products = int(ctx.lib.ckks_rmsplan_inner_products(h))
+        self.mod_downs = int(ctx.lib.ckks_rmsplan_mod_downs(h))
+        self.term_weights = [[p >= 0 for _, _, p in terms] for terms in self.outputs]
+        self.weighted_outputs = [any(w) for w in self.term_weights]
+        self.terms = len(flat)
+
+    def __del__(self):
+        try:
+            if self._h:
+                self.ctx.lib.ckks_rmsplan_destroy(self._h)
                 self._h = None
         except Exception:
             pass

@@ -173,6 +173,36 @@ inline seal::Ciphertext Linear_Transform_Plain_hoisted(const seal::Ciphertext &c
     return out;
 }
 
+// Opt-in: Linear_Transform_Plain with DOUBLE hoisting -- one digit decomposition of ct_new, the d-1 key inner products
+// weighted by their diagonals and summed in the extended basis, ONE mod-down (ckks_rotate_multiply_sum_hoisted).
+// U_diagonals are encoded at the key level: encoder.encode(diag, context->key_parms_id(), scale, pt).  gal_keys: a key for
+// every step 1..d-1 and for -d.  Decrypts like Linear_Transform_Plain within key-switch noise; different polynomials.
+inline seal::Ciphertext Linear_Transform_Plain_double_hoisted(const seal::Ciphertext &ct, const std::vector<seal::Plaintext> &U_diagonals,
+                                                              const seal::GaloisKeys &gal_keys, const seal::EncryptionParameters &params) {
+    auto context = seal::SEALContext::Create(params);
+    seal::Evaluator evaluator(context);
+    const int d = (int)U_diagonals.size();
+    detail::Batch diags = detail::gather(U_diagonals);
+    seal::Ciphertext ct_new = detail::duplicate(ct, d, gal_keys, evaluator);
+    const detail::Poly &pn = ct_new.poly();
+    if (diags.limbs != pn.eng->K) throw std::invalid_argument("U_diagonals must be encoded at the key level (key_parms_id)");
+    detail::scale_ok(*pn.eng, pn.scale * diags.scale, pn.limbs);
+    if (!gal_keys.s || !gal_keys.s->ks) throw std::invalid_argument("galois_keys is not valid for encryption parameters");
+    std::vector<int> first{0, d}, in_idx(d, 0), steps(d), pt_idx(d);
+    for (int l = 0; l < d; l++) steps[l] = pt_idx[l] = l;
+    ckks_rmsplan *plan = nullptr;
+    detail::check(ckks_rmsplan_create(pn.eng->ctx, gal_keys.s->ks, 1, d, 1, first.data(), d, in_idx.data(), steps.data(),
+                                      pt_idx.data(), &plan));
+    seal::Ciphertext out;
+    out.poly().allocate(pn.eng, 2, pn.limbs);
+    out.poly().scale = pn.scale * diags.scale;
+    ckks_view vi = pn.view(), vd = diags.view(), vo = out.poly().view();
+    const int rc = ckks_rotate_multiply_sum_hoisted(pn.eng->ctx, plan, &vi, &vd, &vo, nullptr);
+    ckks_rmsplan_destroy(plan);
+    detail::check(rc);
+    return out;
+}
+
 // helper.h:212-234 -- the same with ciphertext diagonals; the result has size 3 (no relinearisation)
 inline seal::Ciphertext Linear_Transform_Cipher(const seal::Ciphertext &ct, const std::vector<seal::Ciphertext> &U_diagonals,
                                                 const seal::GaloisKeys &gal_keys, seal::Evaluator &evaluator) {

@@ -709,7 +709,9 @@ public:
 
 private:
     void check_target(double largest, int limbs, double scale) const {
-        if (limbs < 1 || limbs > e_->K - 1) throw std::invalid_argument("parms_id is not valid for encryption parameters");
+        // as in SEAL, any level of the context may be targeted, the key level (all K primes) included: the double-hoisted
+        // transforms multiply plaintexts into the extended basis Q_L u {P}
+        if (limbs < 1 || limbs > e_->K) throw std::invalid_argument("parms_id is not valid for encryption parameters");
         if (!(scale > 0)) throw std::invalid_argument("scale out of bounds");
         int bits = 0;
         for (int j = 0; j < limbs; j++) bits += 64 - __builtin_clzll(e_->primes[j]);

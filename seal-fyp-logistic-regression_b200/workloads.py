@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import capi
-from .engine import Ciphertext, RotPlan
+from .engine import Ciphertext, RotMulSumPlan, RotPlan
 
 
 def force_scale_pow2(ct):
@@ -33,6 +33,13 @@ class PlanCache:
         key = tuple(int(s) for s in steps)
         if key not in self._plans:
             self._plans[key] = RotPlan(self.ctx, self.keys, key)
+        return self._plans[key]
+
+    def rms(self, n_in, n_pt, outputs):
+        """the compiled term table of Evaluator.rotate_multiply_sum_hoisted (RotMulSumPlan)"""
+        key = ("rms", int(n_in), int(n_pt), tuple(tuple(t) for t in outputs))
+        if key not in self._plans:
+            self._plans[key] = RotMulSumPlan(self.ctx, self.keys, n_in, n_pt, outputs)
         return self._plans[key]
 
 
@@ -622,6 +629,122 @@ def cc_matrix_multiplication_nonzero(ev, ctA, ctB, d, sigma, tau, V, W, keys, pl
         return _stack(outs)
 
     Ak, Bk = step2(A0, V), step2(B0, W)
+    ev.rescale_to_next_inplace(Ak)
+    ev.rescale_to_next_inplace(Bk)
+    ctAB = ev.multiply(A0, B0)
+    ev.mod_switch_to_next_inplace(ctAB)
+    force_scale_pow2(Ak)
+    force_scale_pow2(Bk)
+    rest = ev.multiply_sum(Ak, Bk)
+    if rest.scale != ctAB.scale:
+        raise capi.CkksInvalidArgument("scale mismatch")
+    return ev.add(ctAB, rest)
+
+
+# ------------------------------------------------------------------ tolerance mode: double hoisting
+# Evaluator.rotate_multiply_sum_hoisted evaluates plaintext-weighted sums of rotations with one digit decomposition per
+# input and one mod-down per output (the key inner products are weighted and summed in the extended basis Q_L u {P}).
+# Its plaintexts are encoded at the key level: encoder.encode(..., limbs=ctx.K), BsgsDiagonals(..., limbs=ctx.K),
+# DiagonalSet.from_matrix(..., limbs=ctx.K).  Results decrypt like the hoisted modes within key-switch noise; ciphertext
+# polynomials differ -- tolerance-checked modes, never the default.
+def diagonal_terms(index_lists, inputs):
+    """term tables of diagonal sums: output s applies the diagonals index_lists[s] to input inputs[s]; the plaintexts are
+    numbered consecutively over all outputs (output s's diagonal i is plaintext sum_{r<s} len(index_lists[r]) + i)"""
+    outs, off = [], 0
+    for idx, a in zip(index_lists, inputs):
+        outs.append([(int(a), int(l), off + i) for i, l in enumerate(idx)])
+        off += len(idx)
+    return outs
+
+
+def bsgs_terms(d, b):
+    """(baby, giant) term tables of the BSGS transform: baby output g = sum_s diag_{gb+s} (.) rot(dup, s) (1 input, G
+    outputs); giant = sum_g rot(inner_g, g b) (G inputs, weight 1, 1 output)"""
+    G = (d + b - 1) // b
+    baby = [[(0, s, g * b + s) for s in range(min(b, d - g * b))] for g in range(G)]
+    giant = [[(g, g * b, -1) for g in range(G)]]
+    return baby, giant
+
+
+def term_steps(*tables):
+    """the non-zero rotation steps a set of term tables uses (each needs its own Galois key)"""
+    return {s for outputs in tables for terms in outputs for _, s, _ in terms if s != 0}
+
+
+def linear_transform_double_hoisted_steps(d):
+    """Galois steps of linear_transform_plain_double_hoisted: the duplicate fill (-d) and 1..d-1"""
+    return sorted({-d} | term_steps(diagonal_terms([range(d)], [0])))
+
+
+def bsgs_double_hoisted_steps(d, b):
+    """Galois steps of linear_transform_plain_bsgs_double_hoisted: -d, 1..b-1 and g b for g = 1..G-1"""
+    return sorted({-d} | term_steps(*bsgs_terms(d, b)))
+
+
+def _perm_diagonal_index(rows, cols, n):
+    """the non-empty diagonals (diag_l[k] = U[k][(k+l) mod n]) of a 0/1 matrix given by its non-zero entries"""
+    return sorted({int(x) for x in np.unique((np.asarray(cols) - np.asarray(rows)) % n)})
+
+
+def matmul_diagonal_indices(d):
+    """non-empty diagonals of U_sigma, U_tau, V_k and W_k (k = 1..d-1) from their closed forms (u_sigma ... w_k above)"""
+    n = d * d
+    i, j = np.meshgrid(np.arange(d), np.arange(d), indexing="ij")
+    r = (d * i + j).ravel()
+    sig = _perm_diagonal_index(r, (d * i + (i + j) % d).ravel(), n)
+    tau = _perm_diagonal_index(r, (d * ((i + j) % d) + j).ravel(), n)
+    V = [_perm_diagonal_index(r, (d * i + (j + k) % d).ravel(), n) for k in range(1, d)]
+    W = [_perm_diagonal_index(r, (d * ((i + k) % d) + j).ravel(), n) for k in range(1, d)]
+    return sig, tau, V, W
+
+
+def matmul_nonzero_hoisted_terms(sig, tau, V, W):
+    """term tables of cc_matrix_multiplication_nonzero_hoisted from the diagonal index lists: (sigma / tau: inputs
+    dup(A), dup(B), 2 outputs; step 2: inputs dup(A0), dup(B0), outputs V_1..V_{d-1}, W_1..W_{d-1})"""
+    first = diagonal_terms([sig, tau], [0, 1])
+    second = diagonal_terms(list(V) + list(W), [0] * len(V) + [1] * len(W))
+    return first, second
+
+
+def matmul_nonzero_hoisted_steps(d):
+    """Galois steps of cc_matrix_multiplication_nonzero_hoisted at dimension d: -d^2 and every non-empty diagonal"""
+    return sorted({-d * d} | term_steps(*matmul_nonzero_hoisted_terms(*matmul_diagonal_indices(d))))
+
+
+def linear_transform_plain_double_hoisted(ev, ct, diags, keys, plans):
+    """Linear_Transform_Plain (helper.h:237-262) with double hoisting: sum_l diag_l (.) rot(ct + rot(ct,-d), l) in one
+    rotate_multiply_sum_hoisted call (1 input, d terms, 1 output): d - 1 key inner products and ONE mod-down instead of
+    d - 1 mod-downs and d - 1 rotated ciphertexts.  `diags`: the d diagonals encoded at the key level (limbs = ctx.K).
+    `keys`: linear_transform_double_hoisted_steps(d)."""
+    d = diags.batch
+    dup = duplicate_fill(ev, ct, d, keys)
+    return ev.rotate_multiply_sum_hoisted(dup, diags, plans.rms(1, d, diagonal_terms([range(d)], [0])))
+
+
+def linear_transform_plain_bsgs_double_hoisted(ev, ct, bd, keys, plans):
+    """baby-step / giant-step Linear_Transform_Plain with double hoisting, two rotate_multiply_sum_hoisted calls: the
+    baby level (1 input, d terms, G outputs) and the giant level (G inputs, G unweighted terms, 1 output).  `bd`:
+    BsgsDiagonals encoded at the key level.  `keys`: bsgs_double_hoisted_steps(d, b)."""
+    d, b, G = bd.d, bd.b, bd.G
+    baby, giant = bsgs_terms(d, b)
+    inner = ev.rotate_multiply_sum_hoisted(duplicate_fill(ev, ct, d, keys), bd.plain, plans.rms(1, d, baby))
+    return ev.rotate_multiply_sum_hoisted(inner, None, plans.rms(G, 0, giant))
+
+
+def cc_matrix_multiplication_nonzero_hoisted(ev, ctA, ctB, d, sigma, tau, V, W, keys, plans):
+    """cc_matrix_multiplication_nonzero with double hoisting: sigma(A) and tau(B) in one rotate_multiply_sum_hoisted call
+    (2 inputs, 2 outputs), the V_k / W_k step in another (2 inputs, 2(d-1) outputs), then the same tail (rescale, forced
+    scales, size-3 accumulation).  The DiagonalSets are encoded at the key level.  `keys`: matmul_nonzero_hoisted_steps(d)."""
+    dd = d * d
+    first, second = matmul_nonzero_hoisted_terms(sigma.index, tau.index, [s.index for s in V], [s.index for s in W])
+    X = _stack([duplicate_fill(ev, ctA, dd, keys), duplicate_fill(ev, ctB, dd, keys)])
+    pts = _stack([sigma.special, tau.special])
+    AB0 = ev.rotate_multiply_sum_hoisted(X, pts, plans.rms(2, pts.batch, first))
+    A0, B0 = AB0[0], AB0[1]
+    Y = _stack([duplicate_fill(ev, A0, dd, keys), duplicate_fill(ev, B0, dd, keys)])
+    pts = _stack([s.special for s in list(V) + list(W)])
+    step2 = ev.rotate_multiply_sum_hoisted(Y, pts, plans.rms(2, pts.batch, second))
+    Ak, Bk = step2[0:d - 1], step2[d - 1:]
     ev.rescale_to_next_inplace(Ak)
     ev.rescale_to_next_inplace(Bk)
     ctAB = ev.multiply(A0, B0)
