@@ -223,6 +223,19 @@ uint64_t ckks_rmsplan_inner_products(const ckks_rmsplan *plan); /* key inner pro
 uint64_t ckks_rmsplan_mod_downs(const ckks_rmsplan *plan);      /* mod-downs per run (outputs with a non-zero step) */
 int ckks_rotate_multiply_sum_hoisted(ckks_ctx *ctx, const ckks_rmsplan *plan, const ckks_view *in, const ckks_view *pts,
                                      const ckks_view *out, ckks_stream s);
+/* ckks_rotate_multiply_sum_hoisted split at its mod-down, for sharding one term table over several devices.
+ * _partial writes part: n_out size-2 entries at L + 1 limbs (L = in->limbs), canonical NTT-form residues, limb j < L mod
+ * q_j and limb L mod P (the special prime K-1):
+ *     part[o] = sum_{z in o, step != 0} w_z (.) IP_z  +  P * base_o          (base_o: the c0 and step-0 terms)
+ * An output without terms gives zeros.  Arguments, checks and aliasing rules as ckks_rotate_multiply_sum_hoisted.
+ * ckks_rms_mod_down computes out[o] = ModDown_P(sum_{g < groups} parts[g * n + o]), n = out->batch, the sum taken modulo
+ * each limb's prime.  ModDown's correction depends on limb P alone and P * base = 0 mod P, so
+ * ModDown(x + P * base) = ModDown(x) + base word for word: the mod-down of the sum of the partials of term tables that
+ * split one table's terms is that table's ckks_rotate_multiply_sum_hoisted output, in every rounding mode.
+ * parts: groups * n entries at out->limbs + 1 limbs; out: n size-2 entries at L <= K-1 limbs, not overlapping parts. */
+int ckks_rotate_multiply_sum_hoisted_partial(ckks_ctx *ctx, const ckks_rmsplan *plan, const ckks_view *in, const ckks_view *pts,
+                                             const ckks_view *part, ckks_stream s);
+int ckks_rms_mod_down(ckks_ctx *ctx, const ckks_view *parts, int groups, const ckks_view *out, ckks_stream s);
 
 /* The rotate-and-sum loop of cipher_dot_product (helper.h:472-476), `count` times:
  *     dup = rotate_vector(dup, steps);  acc = acc + dup

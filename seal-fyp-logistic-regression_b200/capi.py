@@ -94,6 +94,8 @@ SIGNATURES = {
     "ckks_rmsplan_inner_products": (C.c_uint64, [C.c_void_p]),
     "ckks_rmsplan_mod_downs": (C.c_uint64, [C.c_void_p]),
     "ckks_rotate_multiply_sum_hoisted": (C.c_int, [C.c_void_p, C.c_void_p, _VP, _VP, _VP, C.c_void_p]),
+    "ckks_rotate_multiply_sum_hoisted_partial": (C.c_int, [C.c_void_p, C.c_void_p, _VP, _VP, _VP, C.c_void_p]),
+    "ckks_rms_mod_down": (C.c_int, [C.c_void_p, _VP, C.c_int, _VP, C.c_void_p]),
     "ckks_rotate_sum_chain": (C.c_int, [C.c_void_p, C.c_void_p, _VP, _VP, _VP, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_void_p]),
     "ckks_multiply_plain_sum": (C.c_int, [C.c_void_p, _VP, _VP, _VP, C.c_void_p]),
     "ckks_multiply_sum": (C.c_int, [C.c_void_p, _VP, _VP, _VP, C.c_void_p]),

@@ -1477,6 +1477,7 @@ struct ckks_rmsplan {
         std::vector<int> unit_first, part_first, fold_first;
         RmsUnit *d_units = nullptr;
         RmsFold *d_folds = nullptr;
+        RmsFold *d_ofolds = nullptr;   // _partial: per output o, {o, first unit, unit count} (no units: {o, 0, 0})
     };
     std::vector<Split> split;
     int *d_first = nullptr;
@@ -1490,6 +1491,7 @@ extern "C" void ckks_rmsplan_destroy(ckks_rmsplan *p) {
     for (auto &s : p->split) {
         cudaFree(s.d_units);
         cudaFree(s.d_folds);
+        cudaFree(s.d_ofolds);
     }
     cudaFree(p->d_first);
     cudaFree(p->d_terms);
@@ -1564,7 +1566,7 @@ extern "C" int ckks_rmsplan_create(ckks_ctx *c, ckks_keyset *ks, int n_in, int n
     }
     p->split.resize(c->K);
     const int nks = (int)p->ks_out.size();
-    for (int L = 1; L < c->K && nks > 0; L++) {
+    for (int L = 1; L < c->K; L++) {
         ckks_rmsplan::Split &s = p->split[L];
         const int per_unit = (c->n / NTT_TILE) * (L + 1);
         const int target = std::max(1, (4 * sms + per_unit - 1) / per_unit);
@@ -1588,7 +1590,11 @@ extern "C" int ckks_rmsplan_create(ckks_ctx *c, ckks_keyset *ks, int n_in, int n
         s.unit_first.push_back((int)units.size());
         s.part_first.push_back(parts);
         s.fold_first.push_back((int)folds.size());
-        if (!rms_upload(&s.d_units, units) || !rms_upload(&s.d_folds, folds)) {
+        std::vector<RmsFold> ofolds(n_out, RmsFold{0, 0, 0, 0});
+        for (int o = 0; o < n_out; o++) ofolds[o].acc = o;
+        for (int k = 0; k < nks; k++)
+            ofolds[p->ks_out[k]] = RmsFold{p->ks_out[k], s.unit_first[k], s.unit_first[k + 1] - s.unit_first[k], 0};
+        if (!rms_upload(&s.d_units, units) || !rms_upload(&s.d_folds, folds) || !rms_upload(&s.d_ofolds, ofolds)) {
             ckks_rmsplan_destroy(p);
             return fail(CKKS_ERR_CUDA, "rotate_multiply_sum plan: device allocation failed");
         }
@@ -1613,8 +1619,9 @@ static bool views_overlap(const ckks_ctx *c, const ckks_view *a, const ckks_view
     return a0 < b0 + view_span(c, b) && b0 < a0 + view_span(c, a);
 }
 
-extern "C" int ckks_rotate_multiply_sum_hoisted(ckks_ctx *c, const ckks_rmsplan *p, const ckks_view *in, const ckks_view *pts,
-                                                const ckks_view *out, ckks_stream s) {
+// arguments of a run; `extra` = limbs of out beyond in's (0 for the full call, 1 for the extended-basis partial)
+static int rms_check(ckks_ctx *c, const ckks_rmsplan *p, const ckks_view *in, const ckks_view *pts, const ckks_view *out,
+                     int extra) {
     int rc;
     if (!p) return fail(CKKS_ERR_INVALID, "null plan");
     if ((rc = check_view(c, in, "encrypted")) || (rc = check_view(c, out, "out"))) return rc;
@@ -1622,7 +1629,9 @@ extern "C" int ckks_rotate_multiply_sum_hoisted(ckks_ctx *c, const ckks_rmsplan 
     if (in->limbs > c->K - 1) return fail(CKKS_ERR_INVALID, "encrypted is not valid for encryption parameters");
     if (in->batch != p->n_in) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: in batch differs from the plan's inputs");
     if (out->batch != p->n_out) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: out batch differs from the plan's outputs");
-    if (out->limbs != in->limbs) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: out level differs from in");
+    if (out->limbs != in->limbs + extra)
+        return fail(CKKS_ERR_INVALID, extra ? "rotate_multiply_sum partial: out must have in's limbs + 1 (the special prime)"
+                                            : "rotate_multiply_sum: out level differs from in");
     if (views_overlap(c, out, in)) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: out must not alias in");
     if (p->uses_pt) {
         if ((rc = check_view(c, pts, "plain"))) return rc;
@@ -1631,6 +1640,13 @@ extern "C" int ckks_rotate_multiply_sum_hoisted(ckks_ctx *c, const ckks_rmsplan 
         if (pts->batch != p->n_pt) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: pts batch differs from the plan's plaintexts");
         if (views_overlap(c, out, pts)) return fail(CKKS_ERR_INVALID, "rotate_multiply_sum: out must not alias pts");
     }
+    return CKKS_OK;
+}
+
+extern "C" int ckks_rotate_multiply_sum_hoisted(ckks_ctx *c, const ckks_rmsplan *p, const ckks_view *in, const ckks_view *pts,
+                                                const ckks_view *out, ckks_stream s) {
+    int rc;
+    if ((rc = rms_check(c, p, in, pts, out, 0))) return rc;
     CU(cudaSetDevice(c->device));
     // a Galois key replaced after the plan was compiled has a new engine-owned copy: refresh the device-side key table
     if ((rc = sync_key_tables(p->ks))) return rc;
@@ -1700,6 +1716,119 @@ extern "C" int ckks_rotate_multiply_sum_hoisted(ckks_ctx *c, const ckks_rmsplan 
             LAUNCH_CHECK(c);                                                                                                 \
             rt.b0 = k0;                                                                                                      \
             k_md_fwd_row<LN, 1><<<dim3(G::ROW_TILES, L, 2 * nc), NTT_THREADS, 0, st>>>(T2, minu, rt, 2, L, K - 1, c->t);     \
+            LAUNCH_CHECK(c);                                                                                                 \
+        }                                                                                                                    \
+    }
+    DISPATCH_LOGN(c, RUN)
+#undef RUN
+    return CKKS_OK;
+}
+
+// The sum split at its mod-down: every unit's canonical partial (k_rms_mac<PARTIAL>), then per output the sum of its units'
+// partials plus P * base (k_rms_partial_fold) straight into the caller's extended-basis tensor.  Chunks of key-switched
+// outputs as in the full call; chunk q also folds the outputs without key-switched terms that precede the next chunk.
+extern "C" int ckks_rotate_multiply_sum_hoisted_partial(ckks_ctx *c, const ckks_rmsplan *p, const ckks_view *in,
+                                                        const ckks_view *pts, const ckks_view *part, ckks_stream s) {
+    int rc;
+    if ((rc = rms_check(c, p, in, pts, part, 1))) return rc;
+    CU(cudaSetDevice(c->device));
+    if ((rc = sync_key_tables(p->ks))) return rc;
+    cudaStream_t st = (cudaStream_t)s;
+    const int L = in->limbs, nks = (int)p->ks_out.size();
+    const size_t N = c->n;
+    const DView vin = dv(in), vpart = dv(part), vpt = p->uses_pt ? dv(pts) : DView{};
+    const uint32_t *const *perm_tab = p->ks->d_perm_tab;
+    const u64 *const *key_tab = p->ks->d_key_tab;
+    const ckks_rmsplan::Split &sp = p->split[L];
+    // workspace: D and the decomposition of every input, then per chunk the partials of its units
+    const size_t fixed = nks ? (size_t)p->n_in * N * ((size_t)L + (size_t)L * (L + 1)) : 0, per_part = N * 2 * (size_t)(L + 1);
+    auto cost = [&](int k) { return per_part * (size_t)(sp.unit_first[k + 1] - sp.unit_first[k]); };
+    const size_t budget = c->ws_cap / 8 > fixed ? c->ws_cap / 8 - fixed : 0;
+    std::vector<int> chunk(1, 0);
+    size_t most = 0;
+    for (int k = 0; k < nks;) {
+        size_t words = cost(k++);
+        while (k < nks && words + cost(k) <= budget) words += cost(k++);
+        chunk.push_back(k);
+        most = std::max(most, words);
+    }
+    if (nks && (rc = ensure_ws(c, (fixed + most) * 8))) return rc;
+    u64 *D = c->ws, *T1 = nks ? D + (size_t)p->n_in * L * N : nullptr, *PART = nks ? T1 + (size_t)p->n_in * L * (L + 1) * N : nullptr;
+    KsRoute r0{};
+    r0.v[0] = vin;
+    r0.tgt_poly = 1;
+    const int nq = std::max(1, (int)chunk.size() - 1);
+#define RUN(LN)                                                                                                              \
+    {                                                                                                                        \
+        typedef NttGeo<LN> G;                                                                                                \
+        if (nks) {                                                                                                           \
+            k_ks_intt_row<LN, false><<<dim3(G::ROW_TILES, L, p->n_in), NTT_THREADS, 0, st>>>(r0, D, L, c->t);                \
+            LAUNCH_CHECK(c);                                                                                                 \
+            k_ks_invcol_modup<LN><<<dim3(G::COL_TILES, L, p->n_in), NTT_THREADS, 0, st>>>(D, T1, L, 1, c->t);                \
+            LAUNCH_CHECK(c);                                                                                                 \
+            k_hoist_finish<LN><<<dim3(G::ROW_TILES, L *(L + 1), p->n_in), NTT_THREADS, 0, st>>>(T1, vin, L, c->t);           \
+            LAUNCH_CHECK(c);                                                                                                 \
+        }                                                                                                                    \
+        for (int q = 0; q < nq; q++) {                                                                                       \
+            const int k0 = nks ? chunk[q] : 0, k1 = nks ? chunk[q + 1] : 0;                                                  \
+            const int o0 = q == 0 ? 0 : p->ks_out[k0], o1 = k1 < nks ? p->ks_out[k1] : p->n_out;                             \
+            const int u0 = sp.unit_first[k0], nu = sp.unit_first[k1] - u0;                                                  \
+            if (nu) {                                                                                                        \
+                k_rms_mac<LN, true><<<dim3(G::ROW_TILES, L + 1, nu), NTT_THREADS, 0, st>>>(T1, sp.d_units + u0, p->d_nz, vpt, \
+                                                                                           perm_tab, key_tab, nullptr, PART, \
+                                                                                           0, 0, L, c->t);                   \
+                LAUNCH_CHECK(c);                                                                                             \
+            }                                                                                                                \
+            k_rms_partial_fold<LN><<<dim3(G::ROW_TILES, L + 1, o1 - o0), NTT_THREADS, 0, st>>>(                              \
+                sp.d_ofolds, PART, vin, vpt, vpart, p->d_first, p->d_terms, perm_tab, o0, u0, L, c->t);                      \
+            LAUNCH_CHECK(c);                                                                                                 \
+        }                                                                                                                    \
+    }
+    DISPATCH_LOGN(c, RUN)
+#undef RUN
+    return CKKS_OK;
+}
+
+// out[o] = ModDown_P(sum_g parts[g * n + o]): the grouped sum (k_rms_gsum, which also runs the special-prime limb's inverse row
+// pass), then the mod-down of the full call with a zero base (k_md_fwd_row MODE 0), in chunks of outputs under the workspace cap.
+extern "C" int ckks_rms_mod_down(ckks_ctx *c, const ckks_view *parts, int groups, const ckks_view *out, ckks_stream s) {
+    int rc;
+    if ((rc = check_view(c, parts, "parts")) || (rc = check_view(c, out, "out"))) return rc;
+    if (groups < 1) return fail(CKKS_ERR_INVALID, "rms_mod_down: groups must be at least 1");
+    if (parts->size != 2 || out->size != 2) return fail(CKKS_ERR_INVALID, "encrypted size must be 2");
+    if ((long long)parts->batch != (long long)groups * out->batch)
+        return fail(CKKS_ERR_INVALID, "rms_mod_down: parts batch must be groups x out batch");
+    if (out->limbs > c->K - 1) return fail(CKKS_ERR_INVALID, "encrypted is not valid for encryption parameters");
+    if (parts->limbs != out->limbs + 1)
+        return fail(CKKS_ERR_INVALID, "rms_mod_down: parts must have out's limbs + 1 (the special prime)");
+    if (views_overlap(c, out, parts)) return fail(CKKS_ERR_INVALID, "rms_mod_down: out must not alias parts");
+    CU(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)s;
+    const int L = out->limbs, K = c->K, n = out->batch;
+    const size_t N = c->n, per_out = N * (2 * (size_t)(L + 1) + 2 * (size_t)L);
+    const int nc = (int)std::max<size_t>(1, std::min<size_t>(n, c->ws_cap / 8 / per_out));
+    if ((rc = ensure_ws(c, (size_t)nc * per_out * 8))) return rc;
+    u64 *ACC = c->ws, *T2 = ACC + (size_t)nc * 2 * (L + 1) * N;
+    const DView vparts = dv(parts);
+    KsRoute rt{};      // MODE 0: no base; launch slot b of the chunk writes out[b0 + b]
+    rt.v[0] = rt.v[1] = rt.v[2] = dv(out);
+    int sms = 148;
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+#define RUN(LN)                                                                                                              \
+    {                                                                                                                        \
+        typedef NttGeo<LN> G;                                                                                                \
+        for (int o0 = 0; o0 < n; o0 += nc) {                                                                                 \
+            const int m = std::min(nc, n - o0);                                                                              \
+            k_rms_gsum<LN><<<dim3(G::ROW_TILES, L + 1, m), NTT_THREADS, 0, st>>>(vparts, groups, n, ACC, o0, L, c->t);      \
+            LAUNCH_CHECK(c);                                                                                                 \
+            const int ns = std::max(1, std::min(L, sms / (2 * m * G::COL_TILES)));                                          \
+            DView spec{ACC + (size_t)L * N, (u64)(L + 1) * N, 0};                                                            \
+            DView minu{ACC, 2 * (u64)(L + 1) * N, (u64)(L + 1) * N};                                                         \
+            k_md_invcol_fwdcol<LN, false><<<dim3(G::COL_TILES, ns, 2 * m), NTT_THREADS, 0, st>>>(spec, T2, L, K - 1, ns,     \
+                                                                                                 ChainV{}, c->t);            \
+            LAUNCH_CHECK(c);                                                                                                 \
+            rt.b0 = o0;                                                                                                      \
+            k_md_fwd_row<LN, 0><<<dim3(G::ROW_TILES, L, 2 * m), NTT_THREADS, 0, st>>>(T2, minu, rt, 2, L, K - 1, c->t);      \
             LAUNCH_CHECK(c);                                                                                                 \
         }                                                                                                                    \
     }

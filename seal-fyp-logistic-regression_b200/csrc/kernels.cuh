@@ -1431,7 +1431,8 @@ __device__ __forceinline__ void rms_store_tile(u64 (&r0)[8], u64 (&r1)[8], u64 *
 // (r1) per work unit: the plaintext-weighted sum of its terms' key inner products, for one tile of limb jj.
 // T1F of input a: [L][L + 1][N] at a * L * (L + 1) * N (canonical NTT values, k_hoist_finish).  Keys: tiled copies.
 // grid (ROW_TILES, L + 1, units of the chunk); ACC: [outputs of the chunk][2][L + 1][N], PART likewise per partial.
-template <int LOGN>
+// PARTIAL (ckks_rotate_multiply_sum_hoisted_partial): every unit stores its canonical partial, at slot blockIdx.z of PART.
+template <int LOGN, bool PARTIAL = false>
 __global__ void __launch_bounds__(NTT_THREADS, 2) k_rms_mac(const u64 *T1F, const RmsUnit *units, const RmsTerm *terms, DView pt,
                                                            const uint32_t *const *perm_tab, const u64 *const *key_tab, u64 *ACC,
                                                            u64 *PART, int out0, int part0, int L, Tables t) {
@@ -1534,8 +1535,8 @@ __global__ void __launch_bounds__(NTT_THREADS, 2) k_rms_mac(const u64 *T1F, cons
             r1[e] = barrett128(lo1[e], hi1[e], m);
         }
     }
-    if (u.part >= 0) {   // one of several partials of this output: canonical, summed by k_rms_fold
-        u64 *o = PART + (u64)(u.part - part0) * 2 * (L + 1) * G::N + t0 + 8 * threadIdx.x;
+    if (PARTIAL || u.part >= 0) {   // one of several partials of this output: canonical, summed by k_rms_fold
+        u64 *o = PART + (u64)(PARTIAL ? (int)blockIdx.z : u.part - part0) * 2 * (L + 1) * G::N + t0 + 8 * threadIdx.x;
         store8(o + (u64)jj * G::N, r0);
         store8(o + (u64)(L + 1 + jj) * G::N, r1);
         return;
@@ -1614,6 +1615,116 @@ __global__ void __launch_bounds__(NTT_THREADS) k_rms_base(DView in, DView pt, DV
 #pragma unroll
     for (int e = 0; e < 8; e++) x[e] = barrett128(lo[e], hi[e], m);
     store8(out.data + o * out.bs + k * out.ps + (u64)j * G::N + g0, x);
+}
+
+// ---- the double-hoisted sum split at its mod-down (sharding one term table over several devices)
+// (r4) extended-basis partial of output o: part[o][k][jj] = sum of its units' partials (k_rms_mac<PARTIAL>) + [jj < L] P * base_o[k],
+// canonical.  P * base is 0 mod P, so the mod-down of the sum of such partials adds base exactly (ckks_rms_mod_down).
+// Each c0 and step-0 term is read once, for both polynomials.  folds[o] = {-, first unit, unit count}.
+// grid (ROW_TILES, L + 1, outputs of the chunk); output o = o0 + blockIdx.z, its units' partials at PART slot unit - part0.
+template <int LOGN>
+__global__ void __launch_bounds__(NTT_THREADS) k_rms_partial_fold(const RmsFold *folds, const u64 *PART, DView in, DView pt, DView out,
+                                                                 const int *first, const RmsTerm *terms,
+                                                                 const uint32_t *const *perm_tab, int o0, int part0, int L, Tables t) {
+    typedef NttGeo<LOGN> G;
+    const int o = o0 + blockIdx.z, jj = blockIdx.y, pj = jj == L ? t.K - 1 : jj;
+    const RmsFold fd = folds[o];
+    const ModConst m = load_mod(t, pj);
+    const int g0 = blockIdx.x * NTT_TILE + 8 * threadIdx.x;
+    const u64 words = 2 * (u64)(L + 1) * G::N;
+    u64 r0[8], r1[8], x[8];
+#pragma unroll
+    for (int e = 0; e < 8; e++) r0[e] = r1[e] = 0;
+    for (int q = 0; q < fd.pn; q++) {
+        const u64 *src = PART + (u64)(fd.pb - part0 + q) * words + g0;
+        load8(x, src + (u64)jj * G::N);
+#pragma unroll
+        for (int e = 0; e < 8; e++) r0[e] = addmod(r0[e], x[e], m.p);
+        load8(x, src + (u64)(L + 1 + jj) * G::N);
+#pragma unroll
+        for (int e = 0; e < 8; e++) r1[e] = addmod(r1[e], x[e], m.p);
+    }
+    if (jj < L) {
+        u64 lo0[8], hi0[8], lo1[8], hi1[8], w[8];
+#pragma unroll
+        for (int e = 0; e < 8; e++) lo0[e] = hi0[e] = lo1[e] = hi1[e] = 0;
+        int cnt = 0;
+        for (int z = first[o]; z < first[o + 1]; z++) {
+            const RmsTerm tm = terms[z];
+            const u64 *src = in.data + tm.a * in.bs + (u64)jj * G::N;
+            if (tm.p >= 0) load8(w, pt.data + tm.p * pt.bs + (u64)jj * G::N + g0);
+            if (tm.slot >= 0) {   // sigma_z(c0); the rotated c1 is key-switched, not added
+                unsigned ix[8];
+                load_perm8(ix, perm_tab[tm.slot] + g0);
+#pragma unroll
+                for (int e = 0; e < 8; e++) x[e] = src[ix[e]];
+            } else {
+                load8(x, src + g0);
+            }
+#pragma unroll
+            for (int e = 0; e < 8; e++) {
+                if (tm.p >= 0) {
+                    mac128(lo0[e], hi0[e], x[e], w[e]);
+                } else {
+                    lo0[e] += x[e];
+                    hi0[e] += lo0[e] < x[e];
+                }
+            }
+            if (tm.slot < 0) {   // step 0: c1 as well
+                load8(x, src + in.ps + g0);
+#pragma unroll
+                for (int e = 0; e < 8; e++) {
+                    if (tm.p >= 0) {
+                        mac128(lo1[e], hi1[e], x[e], w[e]);
+                    } else {
+                        lo1[e] += x[e];
+                        hi1[e] += lo1[e] < x[e];
+                    }
+                }
+            }
+            if (++cnt == RMS_SEG_MAX) {
+#pragma unroll
+                for (int e = 0; e < 8; e++) {
+                    lo0[e] = barrett128(lo0[e], hi0[e], m), hi0[e] = 0;
+                    lo1[e] = barrett128(lo1[e], hi1[e], m), hi1[e] = 0;
+                }
+                cnt = 0;
+            }
+        }
+        const u64 P = reduce64(t.mod[t.K - 1].p, m);
+#pragma unroll
+        for (int e = 0; e < 8; e++) {
+            r0[e] = addmod(r0[e], mulmod(barrett128(lo0[e], hi0[e], m), P, m), m.p);
+            r1[e] = addmod(r1[e], mulmod(barrett128(lo1[e], hi1[e], m), P, m), m.p);
+        }
+    }
+    u64 *dst = out.data + o * out.bs + (u64)jj * G::N + g0;
+    store8(dst, r0);
+    store8(dst + out.ps, r1);
+}
+
+// (r5) ckks_rms_mod_down's load: ACC_z = sum_{g < groups} parts[g * n + o0 + z] modulo each limb's prime (canonical inputs),
+// the special-prime limb on into the mod-down INTT's row pass (rms_store_tile).  grid (ROW_TILES, L + 1, outputs of the chunk)
+template <int LOGN>
+__global__ void __launch_bounds__(NTT_THREADS, 2) k_rms_gsum(DView parts, int groups, int n, u64 *ACC, int o0, int L, Tables t) {
+    typedef NttGeo<LOGN> G;
+    __shared__ u64 smem[NTT_TILE];
+    const int jj = blockIdx.y, pj = jj == L ? t.K - 1 : jj;
+    const u64 p = t.mod[pj].p;
+    const int t0 = blockIdx.x * NTT_TILE;
+    u64 r0[8], r1[8], x[8];
+#pragma unroll
+    for (int e = 0; e < 8; e++) r0[e] = r1[e] = 0;
+    for (int g = 0; g < groups; g++) {
+        const u64 *src = parts.data + (u64)(g * n + o0 + (int)blockIdx.z) * parts.bs + (u64)jj * G::N + t0 + 8 * threadIdx.x;
+        load8(x, src);
+#pragma unroll
+        for (int e = 0; e < 8; e++) r0[e] = addmod(r0[e], x[e], p);
+        load8(x, src + parts.ps);
+#pragma unroll
+        for (int e = 0; e < 8; e++) r1[e] = addmod(r1[e], x[e], p);
+    }
+    rms_store_tile<LOGN>(r0, r1, ACC + (u64)blockIdx.z * 2 * (L + 1) * G::N, jj, L, t0, t, smem);
 }
 
 // Key-switch keys are static: at registration the engine makes a private copy in which, inside every 2048-word

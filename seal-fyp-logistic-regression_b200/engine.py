@@ -158,6 +158,21 @@ class Ciphertext:
 Plaintext = Ciphertext  # a plaintext is a size-1 batch entry
 
 
+class ExtendedPartial:
+    """size-2 sums in the extended basis Q_L u {P} (Evaluator.rotate_multiply_sum_hoisted_partial): data [n][2][L + 1][N],
+    limb j < L mod q_j, limb L mod the special prime P, canonical NTT-form residues.  Not a Ciphertext: its last limb is
+    not mod q_L, so add_many, rescale and the other ciphertext operations do not apply; Evaluator.rms_mod_down turns a
+    sum of partials into ciphertexts."""
+
+    __slots__ = ("ctx", "data", "limbs", "scale")
+
+    def __init__(self, ctx, data, limbs, scale):
+        assert data.dim() == 4 and data.dtype == torch.int64 and data.is_contiguous() and data.shape[2] == limbs + 1
+        self.ctx, self.data, self.limbs, self.scale = ctx, data, int(limbs), float(scale)
+
+    batch = property(lambda self: self.data.shape[0])
+
+
 class KeySet:
     """SEAL RelinKeys + GaloisKeys: device-resident key-switching keys."""
 
@@ -552,18 +567,7 @@ class Evaluator:
         no term has a plaintext.  Every term of an output carries cts.scale * pts.scale (or cts.scale for weight 1): "scale
         mismatch" otherwise.  Decrypts like rotate_plan_hoisted + multiply_plain_sum within key-switch noise; the
         polynomials differ."""
-        if cts.batch != plan.n_in:
-            raise capi.CkksInvalidArgument("rotate_multiply_sum: in batch differs from the plan's inputs")
-        weighted = plan.weighted_outputs
-        if any(weighted) and pts is None:
-            raise capi.CkksInvalidArgument("rotate_multiply_sum: the plan needs plaintexts")
-        scales = set()
-        for w in plan.term_weights:
-            scales.update(cts.scale * pts.scale if x else cts.scale for x in w)
-        if len(scales) > 1:
-            raise capi.CkksInvalidArgument("scale mismatch")
-        scale = scales.pop() if scales else cts.scale
-        self._scale_ok(scale, cts.limbs)
+        scale = self._rms_scale(cts, pts, plan)
         if out is None:
             out = Ciphertext(self.ctx, torch.empty((plan.n_out, 2, cts.cap, self.ctx.n), dtype=torch.int64,
                                                    device=cts.data.device), cts.limbs, scale)
@@ -572,6 +576,62 @@ class Evaluator:
         vp = pts.view() if pts is not None else None
         check(self.lib.ckks_rotate_multiply_sum_hoisted(self.h, plan._h, C.byref(vi), C.byref(vp) if vp is not None else None,
                                                         C.byref(vo), _stream()))
+        out.scale = scale
+        return out
+
+    def _rms_scale(self, cts, pts, plan):
+        """the scale of rotate_multiply_sum_hoisted's outputs, with its checks"""
+        if cts.batch != plan.n_in:
+            raise capi.CkksInvalidArgument("rotate_multiply_sum: in batch differs from the plan's inputs")
+        if any(plan.weighted_outputs) and pts is None:
+            raise capi.CkksInvalidArgument("rotate_multiply_sum: the plan needs plaintexts")
+        scales = set()
+        for w in plan.term_weights:
+            scales.update(cts.scale * pts.scale if x else cts.scale for x in w)
+        if len(scales) > 1:
+            raise capi.CkksInvalidArgument("scale mismatch")
+        scale = scales.pop() if scales else cts.scale
+        self._scale_ok(scale, cts.limbs)
+        return scale
+
+    def rotate_multiply_sum_hoisted_partial(self, cts, pts, plan):
+        """rotate_multiply_sum_hoisted without its mod-down: the extended-basis sums
+        sum_{z in o, step != 0} w_z (.) IP_z + P * base_o (ckks_rotate_multiply_sum_hoisted_partial), as an ExtendedPartial
+        with L + 1 limbs.  Partials of term tables that split one table's terms add up, modulo every prime, to that table's
+        partial; rms_mod_down of the sum is the output of rotate_multiply_sum_hoisted word for word.  Same checks as the
+        full call."""
+        scale = self._rms_scale(cts, pts, plan)
+        L = cts.limbs
+        data = torch.empty((plan.n_out, 2, L + 1, self.ctx.n), dtype=torch.int64, device=cts.data.device)
+        vi = cts.view()
+        vo = View(data.data_ptr(), 2 * (L + 1) * self.ctx.n, (L + 1) * self.ctx.n, plan.n_out, 2, L + 1, 0)
+        vp = pts.view() if pts is not None else None
+        check(self.lib.ckks_rotate_multiply_sum_hoisted_partial(self.h, plan._h, C.byref(vi),
+                                                                C.byref(vp) if vp is not None else None, C.byref(vo),
+                                                                _stream()))
+        return ExtendedPartial(self.ctx, data, L, scale)
+
+    def rms_mod_down(self, partials, groups, out=None):
+        """out[o] = ModDown_P(sum_{g < groups} parts[g * n + o]) (ckks_rms_mod_down), where parts is the concatenation of
+        `partials` (ExtendedPartials of one level, groups * n entries in all), e.g. one all-gathered partial of every
+        rank.  Returns a Ciphertext of n entries at L limbs; "scale mismatch" when the partials' scales differ."""
+        partials = [partials] if isinstance(partials, ExtendedPartial) else list(partials)
+        if len({p.limbs for p in partials}) != 1:
+            raise capi.CkksInvalidArgument("rms_mod_down: partials at different levels")
+        if len({p.scale for p in partials}) != 1:
+            raise capi.CkksInvalidArgument("scale mismatch")
+        L, scale = partials[0].limbs, partials[0].scale
+        data = partials[0].data if len(partials) == 1 else torch.cat([p.data for p in partials], 0)
+        total = data.shape[0]
+        if groups < 1 or total % groups:
+            raise capi.CkksInvalidArgument("rms_mod_down: parts batch must be groups x out batch")
+        n = total // groups
+        if out is None:
+            out = Ciphertext(self.ctx, torch.empty((n, 2, L, self.ctx.n), dtype=torch.int64, device=data.device), L, scale)
+        out.limbs = L
+        vp = View(data.data_ptr(), 2 * (L + 1) * self.ctx.n, (L + 1) * self.ctx.n, total, 2, L + 1, 0)
+        vo = out.view()
+        check(self.lib.ckks_rms_mod_down(self.h, C.byref(vp), int(groups), C.byref(vo), _stream()))
         out.scale = scale
         return out
 

@@ -11,11 +11,11 @@ import torch
 import torch.distributed as dist
 
 from . import capi
-from .engine import Ciphertext
+from .engine import Ciphertext, ExtendedPartial
 from .lr import (SIGMOID_CHEBYSHEV, apply_gradient, column_epoch_gradient, prediction_masks, refresh_columns,
                  sigmoid_cipher)
-from .workloads import (_stack, chebyshev_depth, chebyshev_keyswitches, cipher_dot_product, duplicate_fill,
-                        force_scale_pow2)
+from .workloads import (_stack, bsgs_terms, chebyshev_depth, chebyshev_keyswitches, cipher_dot_product, diagonal_terms,
+                        duplicate_fill, force_scale_pow2, matmul_diagonal_indices, matmul_nonzero_hoisted_terms, term_steps)
 
 
 def world():
@@ -484,3 +484,166 @@ def sharded_train_columns(ev, cols_local, labels_local, minibatch_ids, units, we
         weights, w_bcast = [_broadcast_ct(ctx, ct, rank, exchange) for ct in fresh]
         mark("refresh")
     return weights, w_bcast
+
+
+# ------------------------------------------------------------------ sharded double hoisting
+# An output of rotate_multiply_sum_hoisted is ModDown_P(sum_z w_z (.) IP_z) + base.  The sum is taken in Q_L u {P}, exact
+# modulo every prime and indifferent to how its terms are grouped, so ranks split the terms of one output, exchange their
+# extended-basis partials (rotate_multiply_sum_hoisted_partial, which folds P * base in) and each runs the one mod-down
+# (rms_mod_down) on the sum: one mod-down per output at every world size, word for word the one-GPU ciphertext.  A rank
+# needs the Galois keys of its own terms' steps only.
+def shard_terms(outputs, rank, world_size):
+    """this rank's share of a term table (one list of (input, step, plaintext) terms per output): the terms of all
+    outputs, in order, are cut into world_size contiguous runs with equal numbers of non-zero-step terms (key inner
+    products; owned_block of their count); a step-0 term goes with the next non-zero-step term (the last one when none
+    follows).  Returns one list per output, each a contiguous run of that output's terms in their order; ranks beyond
+    the number of non-zero-step terms get nothing."""
+    total = sum(1 for terms in outputs for _, s, _ in terms if s != 0)
+    block = owned_block(total, rank, world_size)
+    mine, k = [], 0
+    for terms in outputs:
+        run = []
+        for t in terms:
+            if (k in block) if total else rank == 0:
+                run.append(t)
+            if t[1] != 0:
+                k += 1
+            k = min(k, total - 1)
+        mine.append(run)
+    return mine
+
+
+def _rank_steps(fill, *tables):
+    """Galois steps of a rank's term tables, plus the duplicate-fill step when it runs any term"""
+    used = any(terms for outputs in tables for terms in outputs)
+    return sorted(term_steps(*tables) | ({fill} if used else set()))
+
+
+def linear_transform_double_hoisted_rank_steps(d, rank, world_size):
+    """Galois steps of this rank in sharded_linear_transform_plain_double_hoisted"""
+    return _rank_steps(-d, shard_terms(diagonal_terms([range(d)], [0]), rank, world_size))
+
+
+def _bsgs_rank_tables(d, b, rank, world_size):
+    """this rank's baby outputs (owned_block of the G outputs), their baby term table and its giant terms (inputs: the
+    owned baby outputs in order)"""
+    baby, _ = bsgs_terms(d, b)
+    own = list(owned_block(len(baby), rank, world_size))
+    return own, [baby[g] for g in own], [[(i, g * b, -1) for i, g in enumerate(own)]] if own else []
+
+
+def bsgs_double_hoisted_rank_steps(d, b, rank, world_size):
+    """Galois steps of this rank in sharded_linear_transform_plain_bsgs_double_hoisted"""
+    _, baby, giant = _bsgs_rank_tables(d, b, rank, world_size)
+    return _rank_steps(-d, baby, giant)
+
+
+def _matmul_rank_tables(sig, tau, V, W, rank, world_size):
+    """this rank's share of cc_matrix_multiplication_nonzero_hoisted: its sigma / tau terms (shard_terms), its block of
+    k (owned_block of d - 1) and the V_k / W_k term table of those k (plaintexts numbered V_k of own, then W_k of own)"""
+    first, _ = matmul_nonzero_hoisted_terms(sig, tau, V, W)
+    own = list(owned_block(len(V), rank, world_size))
+    second = diagonal_terms([V[k] for k in own] + [W[k] for k in own], [0] * len(own) + [1] * len(own))
+    return shard_terms(first, rank, world_size), own, second
+
+
+def matmul_nonzero_hoisted_rank_steps(d, rank, world_size):
+    """Galois steps of this rank in sharded_cc_matrix_multiplication_nonzero_hoisted"""
+    first, _, second = _matmul_rank_tables(*matmul_diagonal_indices(d), rank, world_size)
+    return _rank_steps(-d * d, first, second)
+
+
+def _zero_extended(ct, n):
+    """the extended-basis partial of a rank without terms: zeros"""
+    data = torch.zeros((n, 2, ct.limbs + 1, ct.ctx.n), dtype=torch.int64, device=ct.data.device)
+    return ExtendedPartial(ct.ctx, data, ct.limbs, ct.scale)
+
+
+def _mod_down_sum(ev, part, scale, world_size, exchange, mark):
+    """all-gather of every rank's partial, then the one mod-down of their sum.  `scale`: the one-GPU output scale (a
+    rank without terms holds zeros, whose scale is immaterial)"""
+    mark("partial")
+    gathered = exchange.all_gather(part.data)
+    mark("exchange")
+    out = ev.rms_mod_down(ExtendedPartial(part.ctx, gathered, part.limbs, scale), world_size)
+    mark("mod_down")
+    return out
+
+
+def sharded_linear_transform_plain_double_hoisted(ev, ct, diags, keys, plans, rank, world_size, exchange, mark=None):
+    """linear_transform_plain_double_hoisted with the terms of its one output sharded (shard_terms); every rank with
+    terms runs the duplicate fill, one all-gather of one partial, one mod-down.  Every rank returns the one-GPU
+    ciphertext.  `keys`: linear_transform_double_hoisted_rank_steps(d, rank, world_size).  `mark(name)`: optional
+    phase callback."""
+    mark = mark or (lambda name: None)
+    d = diags.batch
+    mine = shard_terms(diagonal_terms([range(d)], [0]), rank, world_size)
+    if mine[0]:
+        part = ev.rotate_multiply_sum_hoisted_partial(duplicate_fill(ev, ct, d, keys), diags, plans.rms(1, d, mine))
+    else:
+        part = _zero_extended(ct, 1)
+    return _mod_down_sum(ev, part, ct.scale * diags.scale, world_size, exchange, mark)
+
+
+def sharded_linear_transform_plain_bsgs_double_hoisted(ev, ct, bd, keys, plans, rank, world_size, exchange, mark=None):
+    """linear_transform_plain_bsgs_double_hoisted with whole baby outputs sharded by owned_block: a rank computes its
+    baby outputs (no exchange: a sub-plan's outputs equal the full plan's) and the partial of the giant terms over them;
+    one all-gather of one partial and one mod-down give every rank the one-GPU ciphertext.
+    `keys`: bsgs_double_hoisted_rank_steps(d, b, rank, world_size)."""
+    mark = mark or (lambda name: None)
+    d, b = bd.d, bd.b
+    own, baby, giant = _bsgs_rank_tables(d, b, rank, world_size)
+    if own:
+        inner = ev.rotate_multiply_sum_hoisted(duplicate_fill(ev, ct, d, keys), bd.plain, plans.rms(1, d, baby))
+        part = ev.rotate_multiply_sum_hoisted_partial(inner, None, plans.rms(len(own), 0, giant))
+    else:
+        part = _zero_extended(ct, 1)
+    return _mod_down_sum(ev, part, ct.scale * bd.plain.scale, world_size, exchange, mark)
+
+
+def sharded_cc_matrix_multiplication_nonzero_hoisted(ev, ctA, ctB, d, sigma, tau, V, W, keys, plans, rank, world_size,
+                                                     exchange, mark=None):
+    """cc_matrix_multiplication_nonzero_hoisted over world_size ranks; every rank returns the one-GPU product word for word.
+    1. sigma(A) / tau(B) with sharded terms: all-gather of the partials and one mod-down, A0 and B0 on every rank.
+    2. V_k / W_k for this rank's block of k (owned_block(d - 1)), whole outputs, no exchange.
+    3. The tail of sharded_cc_matrix_multiplication: rescale, forced scales, multiply_sum over the owned k, all-gather +
+       mod-q add of the size-3 partials, + mod_switch(A0 x B0).
+    `keys`: matmul_nonzero_hoisted_rank_steps(d, rank, world_size)."""
+    mark = mark or (lambda name: None)
+    dd = d * d
+    first, own, second = _matmul_rank_tables(sigma.index, tau.index, [s.index for s in V], [s.index for s in W], rank,
+                                             world_size)
+    pts = _stack([sigma.special, tau.special])
+    if any(first):
+        X = _stack([duplicate_fill(ev, ctA, dd, keys), duplicate_fill(ev, ctB, dd, keys)])
+        part = ev.rotate_multiply_sum_hoisted_partial(X, pts, plans.rms(2, pts.batch, first))
+    else:
+        part = _zero_extended(ctA, 2)
+    AB0 = _mod_down_sum(ev, part, ctA.scale * pts.scale, world_size, exchange, mark)
+    A0, B0 = AB0[0], AB0[1]
+
+    ctAB = ev.multiply(A0, B0)
+    ev.mod_switch_to_next_inplace(ctAB)
+    pt_scale = V[0].special.scale
+    if own:
+        Y = _stack([duplicate_fill(ev, A0, dd, keys), duplicate_fill(ev, B0, dd, keys)])
+        pts = _stack([V[k].special for k in own] + [W[k].special for k in own])
+        XK = ev.rotate_multiply_sum_hoisted(Y, pts, plans.rms(2, pts.batch, second))
+        mark("step2")
+        Ak, Bk = XK[0:len(own)], XK[len(own):]
+        for X in (Ak, Bk):
+            ev.rescale_to_next_inplace(X)
+            force_scale_pow2(X)
+        rest = ev.multiply_sum(Ak, Bk)
+    else:                                   # more ranks than products: this rank adds zero
+        mark("step2")
+        scale = (_rescaled_pow2_scale(A0.ctx, A0.scale * pt_scale, A0.limbs)
+                 * _rescaled_pow2_scale(B0.ctx, B0.scale * pt_scale, B0.limbs))
+        rest = _zeros(A0, 3, 1, scale)
+        rest.limbs = A0.limbs - 1
+    rest = _combine(ev, rest, exchange)
+    if rest.scale != ctAB.scale:
+        raise capi.CkksInvalidArgument("scale mismatch")
+    out = ev.add(ctAB, rest)
+    mark("tail")
+    return out
