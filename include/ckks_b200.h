@@ -259,6 +259,13 @@ int ckks_multiply_sum(ckks_ctx *ctx, const ckks_view *a, const ckks_view *b, con
  * CKKS_ERR_INVALID for groups < 1, mismatched batch, limbs or sizes, and out aliasing an input. */
 int ckks_multiply_sum_grouped(ckks_ctx *ctx, const ckks_view *a, const ckks_view *b, int groups, const ckks_view *out,
                               ckks_stream s);
+/* ciphertext matrix product in one launch: out[i*cols + j] (size 3) = sum_{r < inner} a[i*inner + r] x b[r*cols + j]
+ * for size-2 a (rows x inner) and b (inner x cols), all at one limb count -- per output multiply + add_many, bit-identical
+ * to that sequence.  cols = 1 is ckks_multiply_sum_grouped with groups = rows.  CKKS_ERR_INVALID for rows, inner or
+ * cols below 1, batches other than rows*inner, inner*cols and rows*cols, mismatched limbs or sizes, and out
+ * overlapping an input. */
+int ckks_multiply_sum_matrix(ckks_ctx *ctx, const ckks_view *a, const ckks_view *b, int rows, int inner, int cols,
+                             const ckks_view *out, ckks_stream s);
 
 /* ---- rescale / mod switch */
 /* Evaluator::rescale_to_next_inplace (helper.h:441,543; matrix_multiplication.cpp:71-72):

@@ -100,6 +100,7 @@ SIGNATURES = {
     "ckks_multiply_plain_sum": (C.c_int, [C.c_void_p, _VP, _VP, _VP, C.c_void_p]),
     "ckks_multiply_sum": (C.c_int, [C.c_void_p, _VP, _VP, _VP, C.c_void_p]),
     "ckks_multiply_sum_grouped": (C.c_int, [C.c_void_p, _VP, _VP, C.c_int, _VP, C.c_void_p]),
+    "ckks_multiply_sum_matrix": (C.c_int, [C.c_void_p, _VP, _VP, C.c_int, C.c_int, C.c_int, _VP, C.c_void_p]),
     "ckks_rescale": (C.c_int, [C.c_void_p, _VP, _VP, C.c_void_p]),
     "ckks_mod_switch_drop": (C.c_int, [C.c_void_p, _VP, _VP, C.c_void_p]),
     "ckks_encode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_double, _VP, C.c_void_p]),

@@ -1838,32 +1838,49 @@ extern "C" int ckks_rms_mod_down(ckks_ctx *c, const ckks_view *parts, int groups
 }
 
 // ------------------------------------------------------------------------------------ fused products
-// out[g] = sum_i a[g*T + i] (.) b[i], g < groups, T = b->batch
-static int mul_sum(ckks_ctx *c, bool plain, const ckks_view *a, const ckks_view *b, int groups, const ckks_view *o,
+// out[g*cols + q] = sum_i a[g*T + i] (.) b[i*cols + q], g < groups, q < cols, T = b->batch / cols.  cols = 1 is the
+// fused multiply + add_many (k_ew_mul_sum, b shared by the groups); cols > 1 (ciphertexts only) the matrix product.
+static int mul_sum(ckks_ctx *c, bool plain, const ckks_view *a, const ckks_view *b, int groups, int cols, const ckks_view *o,
                    cudaStream_t st) {
     int rc;
     if ((rc = check_view(c, a, "a")) || (rc = check_view(c, b, "b")) || (rc = check_view(c, o, "out"))) return rc;
     if (groups < 1) return fail(CKKS_ERR_INVALID, "multiply_sum: groups must be at least 1");
-    if ((long long)groups * b->batch != a->batch || a->limbs != b->limbs || o->limbs != a->limbs || o->batch != groups)
+    const long long T = b->batch / cols;
+    if (T * cols != b->batch || (long long)groups * T != a->batch || a->limbs != b->limbs || o->limbs != a->limbs ||
+        (long long)o->batch != (long long)groups * cols)
         return fail(CKKS_ERR_INVALID, "multiply_sum: parameter mismatch");
     if (plain ? (b->size != 1 || o->size != a->size) : (a->size != 2 || b->size != 2 || o->size != 3))
         return fail(CKKS_ERR_INVALID, "multiply_sum: size mismatch");
     if (o->data == a->data || o->data == b->data) return fail(CKKS_ERR_INVALID, "multiply_sum: out must not alias an input");
     CU(cudaSetDevice(c->device));
     if (plain) k_ew_mul_sum<true><<<ew_grid(c, a->size * a->limbs, 1), 256, 0, st>>>(dv(a), dv(b), dv(o), b->batch, a->limbs, c->n, c->t);
-    else k_ew_mul_sum<false><<<ew_grid(c, a->limbs, groups), 256, 0, st>>>(dv(a), dv(b), dv(o), b->batch, a->limbs, c->n, c->t);
+    else if (cols == 1) k_ew_mul_sum<false><<<ew_grid(c, a->limbs, groups), 256, 0, st>>>(dv(a), dv(b), dv(o), b->batch, a->limbs, c->n, c->t);
+    else {
+        k_ew_mul_sum_matrix<<<dim3((c->n / 2 + 255) / 256, a->limbs, (unsigned)groups * cols), 256, 0, st>>>(
+            dv(a), dv(b), dv(o), groups, (int)T, cols, c->n, c->t);
+    }
     LAUNCH_CHECK(c);
     return CKKS_OK;
 }
 extern "C" int ckks_multiply_plain_sum(ckks_ctx *c, const ckks_view *cts, const ckks_view *pts, const ckks_view *o, ckks_stream s) {
-    return mul_sum(c, true, cts, pts, 1, o, (cudaStream_t)s);
+    return mul_sum(c, true, cts, pts, 1, 1, o, (cudaStream_t)s);
 }
 extern "C" int ckks_multiply_sum(ckks_ctx *c, const ckks_view *a, const ckks_view *b, const ckks_view *o, ckks_stream s) {
-    return mul_sum(c, false, a, b, 1, o, (cudaStream_t)s);
+    return mul_sum(c, false, a, b, 1, 1, o, (cudaStream_t)s);
 }
 extern "C" int ckks_multiply_sum_grouped(ckks_ctx *c, const ckks_view *a, const ckks_view *b, int groups, const ckks_view *o,
                                          ckks_stream s) {
-    return mul_sum(c, false, a, b, groups, o, (cudaStream_t)s);
+    return mul_sum(c, false, a, b, groups, 1, o, (cudaStream_t)s);
+}
+extern "C" int ckks_multiply_sum_matrix(ckks_ctx *c, const ckks_view *a, const ckks_view *b, int rows, int inner, int cols,
+                                        const ckks_view *o, ckks_stream s) {
+    int rc;
+    if (rows < 1 || inner < 1 || cols < 1) return fail(CKKS_ERR_INVALID, "multiply_sum_matrix: rows, inner and cols must be at least 1");
+    if ((rc = check_view(c, a, "a")) || (rc = check_view(c, b, "b")) || (rc = check_view(c, o, "out"))) return rc;
+    if ((long long)rows * inner != a->batch || (long long)inner * cols != b->batch || (long long)rows * cols != o->batch)
+        return fail(CKKS_ERR_INVALID, "multiply_sum_matrix: batches must be rows x inner, inner x cols and rows x cols");
+    if (views_overlap(c, o, a) || views_overlap(c, o, b)) return fail(CKKS_ERR_INVALID, "multiply_sum_matrix: out must not overlap an input");
+    return mul_sum(c, false, a, b, rows, cols, o, (cudaStream_t)s);
 }
 
 // ------------------------------------------------------------------------------------ rescale

@@ -1893,6 +1893,63 @@ __global__ void __launch_bounds__(256) k_ew_add_many_grouped(DView in, DView o, 
     *vpw(o, b, s, j, n, c) = acc;
 }
 
+// sum_{q < T} a[a0 + q] (x) b[b0 + q * bstride] -> o[oi] (size 3) for the two coefficients at c of limb j: size-2 x size-2
+// ciphertext products summed lazily, FP64 below 2^41 (|term| < 2p < 2^42, at most 2 * 128 terms between reductions,
+// < 2^51) and 128-bit otherwise (products < 2^120, at most 2 * 8 between reductions, < 2^124), so exact for any T.
+__device__ __forceinline__ void ct_mul_sum(const DView &a, int a0, const DView &b, int b0, int bstride, const DView &o, int oi,
+                                           int T, int j, int n, u64 c, const ModConst &m, const FpConst &f) {
+    if (f.ok != 0.0) {
+        double sx[3] = {0.0, 0.0, 0.0}, sy[3] = {0.0, 0.0, 0.0};
+        for (int q = 0; q < T; q++) {
+            ulonglong2 a0v = *vp(a, a0 + q, 0, j, n, c), a1 = *vp(a, a0 + q, 1, j, n, c);
+            ulonglong2 b0v = *vp(b, b0 + q * bstride, 0, j, n, c), b1 = *vp(b, b0 + q * bstride, 1, j, n, c);
+            const double a0x = fp_from_u64(a0v.x), a0y = fp_from_u64(a0v.y), a1x = fp_from_u64(a1.x), a1y = fp_from_u64(a1.y);
+            const double b0x = fp_from_u64(b0v.x), b0y = fp_from_u64(b0v.y), b1x = fp_from_u64(b1.x), b1y = fp_from_u64(b1.y);
+            sx[0] = __dadd_rn(sx[0], fp_mulmod(a0x, b0x, f)); sy[0] = __dadd_rn(sy[0], fp_mulmod(a0y, b0y, f));
+            sx[1] = __dadd_rn(sx[1], __dadd_rn(fp_mulmod(a0x, b1x, f), fp_mulmod(a1x, b0x, f)));
+            sy[1] = __dadd_rn(sy[1], __dadd_rn(fp_mulmod(a0y, b1y, f), fp_mulmod(a1y, b0y, f)));
+            sx[2] = __dadd_rn(sx[2], fp_mulmod(a1x, b1x, f)); sy[2] = __dadd_rn(sy[2], fp_mulmod(a1y, b1y, f));
+            if ((q & 127) == 127) {
+#pragma unroll
+                for (int k = 0; k < 3; k++) { sx[k] = fp_reduce(sx[k], f); sy[k] = fp_reduce(sy[k], f); }
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 3; k++) {
+            ulonglong2 r;
+            r.x = fp_to_canonical(sx[k], f);
+            r.y = fp_to_canonical(sy[k], f);
+            *vpw(o, oi, k, j, n, c) = r;
+        }
+        return;
+    }
+    u64 lo[3][2], hi[3][2];
+#pragma unroll
+    for (int k = 0; k < 3; k++) lo[k][0] = lo[k][1] = hi[k][0] = hi[k][1] = 0;
+    for (int q = 0; q < T; q++) {
+        ulonglong2 a0v = *vp(a, a0 + q, 0, j, n, c), a1 = *vp(a, a0 + q, 1, j, n, c);
+        ulonglong2 b0v = *vp(b, b0 + q * bstride, 0, j, n, c), b1 = *vp(b, b0 + q * bstride, 1, j, n, c);
+        mac128(lo[0][0], hi[0][0], a0v.x, b0v.x); mac128(lo[0][1], hi[0][1], a0v.y, b0v.y);
+        mac128(lo[1][0], hi[1][0], a0v.x, b1.x); mac128(lo[1][1], hi[1][1], a0v.y, b1.y);
+        mac128(lo[1][0], hi[1][0], a1.x, b0v.x); mac128(lo[1][1], hi[1][1], a1.y, b0v.y);
+        mac128(lo[2][0], hi[2][0], a1.x, b1.x); mac128(lo[2][1], hi[2][1], a1.y, b1.y);
+        if ((q & 7) == 7) {
+#pragma unroll
+            for (int k = 0; k < 3; k++) {
+                lo[k][0] = barrett128(lo[k][0], hi[k][0], m); hi[k][0] = 0;
+                lo[k][1] = barrett128(lo[k][1], hi[k][1], m); hi[k][1] = 0;
+            }
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        ulonglong2 r;
+        r.x = barrett128(lo[k][0], hi[k][0], m);
+        r.y = barrett128(lo[k][1], hi[k][1], m);
+        *vpw(o, oi, k, j, n, c) = r;
+    }
+}
+
 // fused multiply + add_many: out[g] = sum_b a[g*B + b] (.) b[b] for g = blockIdx.z (b shared by every group)
 //   PLAIN: b is a plaintext batch (every poly of a[b] times pt[b]), output size = size of a
 //   else : size-2 x size-2 ciphertext products, output size 3 (Linear_Transform_Cipher; with several groups the
@@ -1924,28 +1981,7 @@ __global__ void __launch_bounds__(256) k_ew_mul_sum(DView a, DView b, DView o, i
             r.y = fp_to_canonical(s1, f);
             *vpw(o, 0, s, j, n, c) = r;
         } else {
-            double sx[3] = {0.0, 0.0, 0.0}, sy[3] = {0.0, 0.0, 0.0};
-            for (int q = 0; q < B; q++) {
-                ulonglong2 a0 = *vp(a, q, 0, j, n, c), a1 = *vp(a, q, 1, j, n, c);
-                ulonglong2 b0 = *vp(b, q, 0, j, n, c), b1 = *vp(b, q, 1, j, n, c);
-                const double a0x = fp_from_u64(a0.x), a0y = fp_from_u64(a0.y), a1x = fp_from_u64(a1.x), a1y = fp_from_u64(a1.y);
-                const double b0x = fp_from_u64(b0.x), b0y = fp_from_u64(b0.y), b1x = fp_from_u64(b1.x), b1y = fp_from_u64(b1.y);
-                sx[0] = __dadd_rn(sx[0], fp_mulmod(a0x, b0x, f)); sy[0] = __dadd_rn(sy[0], fp_mulmod(a0y, b0y, f));
-                sx[1] = __dadd_rn(sx[1], __dadd_rn(fp_mulmod(a0x, b1x, f), fp_mulmod(a1x, b0x, f)));
-                sy[1] = __dadd_rn(sy[1], __dadd_rn(fp_mulmod(a0y, b1y, f), fp_mulmod(a1y, b0y, f)));
-                sx[2] = __dadd_rn(sx[2], fp_mulmod(a1x, b1x, f)); sy[2] = __dadd_rn(sy[2], fp_mulmod(a1y, b1y, f));
-                if ((q & 127) == 127) {
-#pragma unroll
-                    for (int k = 0; k < 3; k++) { sx[k] = fp_reduce(sx[k], f); sy[k] = fp_reduce(sy[k], f); }
-                }
-            }
-#pragma unroll
-            for (int k = 0; k < 3; k++) {
-                ulonglong2 r;
-                r.x = fp_to_canonical(sx[k], f);
-                r.y = fp_to_canonical(sy[k], f);
-                *vpw(o, 0, k, j, n, c) = r;
-            }
+            ct_mul_sum(a, 0, b, 0, 1, o, 0, B, j, n, c, m, f);
         }
         return;
     }
@@ -1965,32 +2001,22 @@ __global__ void __launch_bounds__(256) k_ew_mul_sum(DView a, DView b, DView o, i
         r.y = barrett128(l1, h1, m);
         *vpw(o, 0, s, j, n, c) = r;
     } else {
-        u64 lo[3][2], hi[3][2];
-#pragma unroll
-        for (int k = 0; k < 3; k++) lo[k][0] = lo[k][1] = hi[k][0] = hi[k][1] = 0;
-        for (int q = 0; q < B; q++) {
-            ulonglong2 a0 = *vp(a, q, 0, j, n, c), a1 = *vp(a, q, 1, j, n, c);
-            ulonglong2 b0 = *vp(b, q, 0, j, n, c), b1 = *vp(b, q, 1, j, n, c);
-            mac128(lo[0][0], hi[0][0], a0.x, b0.x); mac128(lo[0][1], hi[0][1], a0.y, b0.y);
-            mac128(lo[1][0], hi[1][0], a0.x, b1.x); mac128(lo[1][1], hi[1][1], a0.y, b1.y);
-            mac128(lo[1][0], hi[1][0], a1.x, b0.x); mac128(lo[1][1], hi[1][1], a1.y, b0.y);
-            mac128(lo[2][0], hi[2][0], a1.x, b1.x); mac128(lo[2][1], hi[2][1], a1.y, b1.y);
-            if ((q & 7) == 7) {
-#pragma unroll
-                for (int k = 0; k < 3; k++) {
-                    lo[k][0] = barrett128(lo[k][0], hi[k][0], m); hi[k][0] = 0;
-                    lo[k][1] = barrett128(lo[k][1], hi[k][1], m); hi[k][1] = 0;
-                }
-            }
-        }
-#pragma unroll
-        for (int k = 0; k < 3; k++) {
-            ulonglong2 r;
-            r.x = barrett128(lo[k][0], hi[k][0], m);
-            r.y = barrett128(lo[k][1], hi[k][1], m);
-            *vpw(o, 0, k, j, n, c) = r;
-        }
+        ct_mul_sum(a, 0, b, 0, 1, o, 0, B, j, n, c, m, f);
     }
+}
+
+// ciphertext matrix product (ckks_multiply_sum_matrix, cols > 1): out[i*cols + q] = sum_{r < inner} a[i*inner + r] (x)
+// b[r*cols + q], the schedule of k_ew_mul_sum with b read at column stride (no gathered copy of b's columns).
+// blockIdx.x = coefficient chunk, blockIdx.y = limb, blockIdx.z = i + rows * q: the chunks of one output run side by side
+// and the rows of one column follow each other, so their reads of the same b words (and the columns' reads of a row's
+// a words) meet in L2.  Blocks of several columns per CTA, which read a once per block, measured slower on a B200 (the
+// per-thread chains of lazy sums grow with the block; DESIGN §4).
+__global__ void __launch_bounds__(256) k_ew_mul_sum_matrix(DView a, DView b, DView o, int rows, int inner, int cols, int n,
+                                                           Tables t) {
+    const int i = blockIdx.z % rows, q = blockIdx.z / rows, j = blockIdx.y;
+    const u64 c = ((u64)blockIdx.x * blockDim.x + threadIdx.x) * 2;
+    if (c >= (u64)n) return;
+    ct_mul_sum(a, i * inner, b, q, cols, o, i * cols + q, inner, j, n, c, t.mod[j], t.fp[j]);
 }
 
 // constant-coefficient sums (ckks_multiply_const_sum).  The residues of the encoded constants are computed on the host

@@ -691,6 +691,28 @@ class Evaluator:
         out.scale = scale
         return out
 
+    def multiply_sum_matrix(self, a, b, rows, cols, out=None):
+        """matrix product of ciphertexts: a (rows x inner, row-major) times b (inner x cols) -> rows x cols size-3
+        entries, out[i*cols + j] = sum_r multiply(a[i*inner + r], b[r*cols + j]), in one kernel
+        (ckks_multiply_sum_matrix); each output equals multiply + add_many of its products word for word"""
+        rows, cols = int(rows), int(cols)
+        if rows < 1 or cols < 1 or a.batch % rows:
+            raise capi.CkksInvalidArgument("encrypted1 and encrypted2 parameter mismatch")
+        inner = a.batch // rows
+        if a.limbs != b.limbs or b.batch != inner * cols:
+            raise capi.CkksInvalidArgument("encrypted1 and encrypted2 parameter mismatch")
+        scale = a.scale * b.scale
+        self._scale_ok(scale, a.limbs)
+        if out is None:
+            out = Ciphertext(self.ctx, torch.empty((rows * cols, 3, a.limbs, self.ctx.n), dtype=torch.int64,
+                                                   device=a.data.device), a.limbs)
+        out.limbs = a.limbs
+        va, vb, vo = a.view(), b.view(), out.view()
+        check(self.lib.ckks_multiply_sum_matrix(self.h, C.byref(va), C.byref(vb), rows, inner, cols, C.byref(vo),
+                                                _stream()))
+        out.scale = scale
+        return out
+
 
 class RotPlan:
     """a fixed list of rotation steps (one per batch entry) compiled into batched rounds"""

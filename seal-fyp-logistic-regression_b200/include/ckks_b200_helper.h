@@ -15,6 +15,7 @@
 //   C_Matrix_Decode                   :325-360         b200::C_Matrix_Decode
 //   cipher_dot_product                :416-502         b200::cipher_dot_product
 //   CC_Matrix_Multiplication (matrix_mult_benchmark.cpp:13-71)  b200::CC_Matrix_Multiplication
+//   (no counterpart: per tile, summed over l)                   b200::CC_Matrix_Multiplication_blocked
 //
 // A maintainer switches a call site by prefixing it with b200:: (or `using b200::Linear_Transform_Plain;`).
 // Differences from the reference, all deliberate: arguments are taken by const reference (the reference
@@ -22,6 +23,7 @@
 // "result ciphertext is transparent" (the reference's drivers add an epsilon to avoid it).
 #pragma once
 #include <cmath>
+#include <memory>
 #include <stdexcept>
 #include <vector>
 
@@ -119,6 +121,38 @@ inline seal::Ciphertext duplicate(const seal::Ciphertext &ct, int d, const seal:
     ev.rotate_vector(ct, -d, gk, rot);
     ev.add(ct, rot, out);
     return out;
+}
+
+// The V_k (W_k) step of CC_Matrix_Multiplication for k = 1..K1 on the sigma (tau) transform `base`: the d*d rotations of
+// base + rotate_vector(base, -d*d) are computed once and shared by the K1 transforms, which are rescaled and given the
+// reference's "manual rescale" power-of-two scale.  Returns the K1 results as one batch at base's level - 1.
+inline Batch shifted(const seal::Ciphertext &base, const std::vector<std::vector<seal::Plaintext>> &sets, int K1,
+                     const seal::GaloisKeys &gal_keys, seal::Evaluator &evaluator) {
+    const int dd = (int)sets[0].size();
+    std::vector<int> steps(dd);
+    for (int l = 0; l < dd; l++) steps[l] = l;
+    seal::Ciphertext dup = duplicate(base, dd, gal_keys, evaluator);
+    const Poly &pn = dup.poly();
+    Batch rots = rotate_all(pn.view(), pn.eng, pn.scale, gal_keys, steps);
+    double pscale = sets[0][0].poly().scale;
+    scale_ok(*pn.eng, pn.scale * pscale, pn.limbs);
+    Batch out(pn.eng, K1, 2, pn.limbs, pn.scale * pscale);
+    for (int k = 0; k < K1; k++) {
+        if ((int)sets[k].size() != dd) throw std::invalid_argument("encrypted and plain parameter mismatch");
+        Batch diags = gather(sets[k]);
+        if (diags.limbs != pn.limbs || diags.scale != pscale) throw std::invalid_argument("encrypted and plain parameter mismatch");
+        ckks_view vr = rots.view(), vd = diags.view(), vo = out.view();
+        vo.data += (std::size_t)k * out.entry_words();
+        vo.batch = 1;
+        check(ckks_multiply_plain_sum(pn.eng->ctx, &vr, &vd, &vo, nullptr));
+    }
+    // rescale_to_next_inplace on every A_k / B_k, then the reference's "manual rescale" of the scale
+    Batch low(pn.eng, K1, 2, pn.limbs - 1, 0.0);
+    if (pn.limbs < 2) throw std::invalid_argument("end of modulus switching chain reached");
+    ckks_view vi = out.view(), vl = low.view();
+    check(ckks_rescale(pn.eng->ctx, &vi, &vl, nullptr));
+    low.scale = std::pow(2.0, (int)std::log2(out.scale / (double)pn.eng->primes[pn.limbs - 1]));
+    return low;
 }
 
 }  // namespace detail
@@ -340,34 +374,9 @@ inline seal::Ciphertext CC_Matrix_Multiplication(const seal::Ciphertext &ctA, co
     evaluator.multiply(A0, B0, ctAB);
     evaluator.mod_switch_to_next_inplace(ctAB);
     if (dimension == 1) return ctAB;
-    const int dd = (int)V_diagonals[0].size(), K1 = dimension - 1;
-    std::vector<int> steps(dd);
-    for (int l = 0; l < dd; l++) steps[l] = l;
-    auto shifted = [&](const seal::Ciphertext &base, const std::vector<std::vector<seal::Plaintext>> &sets) {
-        seal::Ciphertext dup = detail::duplicate(base, dd, gal_keys, evaluator);
-        const detail::Poly &pn = dup.poly();
-        detail::Batch rots = detail::rotate_all(pn.view(), pn.eng, pn.scale, gal_keys, steps);
-        double pscale = sets[0][0].poly().scale;
-        detail::scale_ok(*pn.eng, pn.scale * pscale, pn.limbs);
-        detail::Batch out(pn.eng, K1, 2, pn.limbs, pn.scale * pscale);
-        for (int k = 0; k < K1; k++) {
-            if ((int)sets[k].size() != dd) throw std::invalid_argument("encrypted and plain parameter mismatch");
-            detail::Batch diags = detail::gather(sets[k]);
-            if (diags.limbs != pn.limbs || diags.scale != pscale) throw std::invalid_argument("encrypted and plain parameter mismatch");
-            ckks_view vr = rots.view(), vd = diags.view(), vo = out.view();
-            vo.data += (std::size_t)k * out.entry_words();
-            vo.batch = 1;
-            detail::check(ckks_multiply_plain_sum(pn.eng->ctx, &vr, &vd, &vo, nullptr));
-        }
-        // rescale_to_next_inplace on every A_k / B_k, then the reference's "manual rescale" of the scale
-        detail::Batch low(pn.eng, K1, 2, pn.limbs - 1, 0.0);
-        if (pn.limbs < 2) throw std::invalid_argument("end of modulus switching chain reached");
-        ckks_view vi = out.view(), vl = low.view();
-        detail::check(ckks_rescale(pn.eng->ctx, &vi, &vl, nullptr));
-        low.scale = std::pow(2.0, (int)std::log2(out.scale / (double)pn.eng->primes[pn.limbs - 1]));
-        return low;
-    };
-    detail::Batch Ak = shifted(A0, V_diagonals), Bk = shifted(B0, W_diagonals);
+    const int K1 = dimension - 1;
+    detail::Batch Ak = detail::shifted(A0, V_diagonals, K1, gal_keys, evaluator),
+                  Bk = detail::shifted(B0, W_diagonals, K1, gal_keys, evaluator);
     detail::scale_ok(*Ak.e, Ak.scale * Bk.scale, Ak.limbs);
     seal::Ciphertext rest;
     rest.poly().allocate(Ak.e, 3, Ak.limbs);
@@ -376,6 +385,63 @@ inline seal::Ciphertext CC_Matrix_Multiplication(const seal::Ciphertext &ctA, co
     detail::check(ckks_multiply_sum(Ak.e->ctx, &va, &vb, &vo, nullptr));
     seal::Ciphertext out;
     evaluator.add(ctAB, rest, out);
+    return out;
+}
+
+// Blocked encrypted matrix product of any shape (eprint 2018/1041 per d x d tile): A is tn x tm tiles, B tm x tp, each
+// tile a ciphertext in the reference's row-major d*d-slot layout, both vectors in row-major tile order.  Returns the
+// tn*tp size-3 tiles of A B (row-major, not relinearised), output (i, j) bit-identical to adding
+// CC_Matrix_Multiplication(A_il, B_lj) over l with Evaluator::add.  One tile product is
+//     ModSwitch(A0 x B0) + sum_{k>=1} A_k x B_k = sum_{k=0}^{d-1} X_k x Y_k,  X_0 = ModSwitch(A0), X_k = A_k (Y for B),
+// since the mod switch drops a limb and the tensor product works limb by limb; so every tile is transformed once
+// (tn*tm + tm*tp transforms instead of 2 tn*tm*tp) and the sums over l and k are one ckks_multiply_sum_matrix.
+// dimension must be at least 2: 1 x 1 tiles, which CC_Matrix_Multiplication accepts, throw std::invalid_argument.
+inline std::vector<seal::Ciphertext> CC_Matrix_Multiplication_blocked(
+    const std::vector<seal::Ciphertext> &A_tiles, const std::vector<seal::Ciphertext> &B_tiles, int tn, int tm, int tp,
+    int dimension, const std::vector<seal::Plaintext> &U_sigma_diagonals, const std::vector<seal::Plaintext> &U_tau_diagonals,
+    const std::vector<std::vector<seal::Plaintext>> &V_diagonals, const std::vector<std::vector<seal::Plaintext>> &W_diagonals,
+    const seal::GaloisKeys &gal_keys, const seal::EncryptionParameters &params) {
+    auto context = seal::SEALContext::Create(params);
+    seal::Evaluator evaluator(context);
+    if (tn < 1 || tm < 1 || tp < 1 || (long long)A_tiles.size() != (long long)tn * tm || (long long)B_tiles.size() != (long long)tm * tp)
+        throw std::invalid_argument("tile vectors do not match the tile counts");
+    if (dimension < 2 || (int)V_diagonals.size() < dimension - 1 || (int)W_diagonals.size() < dimension - 1)
+        throw std::invalid_argument("dimension does not match the diagonal sets");
+    const int d = dimension, K1 = d - 1;
+    // the d entries of every tile; X in row-major tile order (entry (i*tm + l)*d + k = i*(tm d) + l d + k), Y in the
+    // contraction's row order (entry (l d + k)*tp + j)
+    std::unique_ptr<detail::Batch> X, Y;
+    double s0[2] = {0, 0};
+    auto operand = [&](const seal::Ciphertext &tile, const std::vector<seal::Plaintext> &first,
+                       const std::vector<std::vector<seal::Plaintext>> &sets, std::unique_ptr<detail::Batch> &dst, int n,
+                       int side, auto index) {
+        seal::Ciphertext x0 = Linear_Transform_Plain(tile, first, gal_keys, params);
+        detail::Batch xk = detail::shifted(x0, sets, K1, gal_keys, evaluator);
+        evaluator.mod_switch_to_next_inplace(x0);
+        if (!dst) {
+            dst.reset(new detail::Batch(xk.e, n * d, 2, xk.limbs, xk.scale));
+            s0[side] = x0.poly().scale;
+        }
+        if (xk.scale != dst->scale || x0.poly().scale != s0[side] || xk.limbs != dst->limbs)
+            throw std::invalid_argument("scale mismatch");
+        dst->put(index(0), x0.poly());
+        for (int k = 1; k < d; k++)
+            detail::check(ckks_copy(xk.e->ctx, dst->buf->p + (std::size_t)index(k) * dst->entry_words(),
+                                    xk.buf->p + (std::size_t)(k - 1) * xk.entry_words(), xk.entry_words() * 8, nullptr));
+    };
+    for (int t = 0; t < tn * tm; t++)
+        operand(A_tiles[t], U_sigma_diagonals, V_diagonals, X, tn * tm, 0, [&](int k) { return t * d + k; });
+    for (int t = 0; t < tm * tp; t++) {
+        const int l = t / tp, j = t % tp;
+        operand(B_tiles[t], U_tau_diagonals, W_diagonals, Y, tm * tp, 1, [&](int k) { return (l * d + k) * tp + j; });
+    }
+    if (s0[0] * s0[1] != X->scale * Y->scale) throw std::invalid_argument("scale mismatch");
+    detail::scale_ok(*X->e, X->scale * Y->scale, X->limbs);
+    detail::Batch C(X->e, tn * tp, 3, X->limbs, X->scale * Y->scale);
+    ckks_view va = X->view(), vb = Y->view(), vo = C.view();
+    detail::check(ckks_multiply_sum_matrix(X->e->ctx, &va, &vb, tn, tm * d, tp, &vo, nullptr));
+    std::vector<seal::Ciphertext> out(tn * tp);
+    for (int o = 0; o < tn * tp; o++) C.get(o, out[o].poly());
     return out;
 }
 

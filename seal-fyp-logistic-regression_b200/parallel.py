@@ -14,8 +14,9 @@ from . import capi
 from .engine import Ciphertext, ExtendedPartial
 from .lr import (SIGMOID_CHEBYSHEV, apply_gradient, column_epoch_gradient, prediction_masks, refresh_columns,
                  sigmoid_cipher)
-from .workloads import (_stack, bsgs_terms, chebyshev_depth, chebyshev_keyswitches, cipher_dot_product, diagonal_terms,
-                        duplicate_fill, force_scale_pow2, matmul_diagonal_indices, matmul_nonzero_hoisted_terms, term_steps)
+from .workloads import (MatmulEntries, _column_major_rows, _stack, bsgs_terms, chebyshev_depth, chebyshev_keyswitches,
+                        cipher_dot_product, diagonal_terms, duplicate_fill, force_scale_pow2, matmul_diagonal_indices,
+                        matmul_nonzero_hoisted_terms, matmul_operands, term_steps)
 
 
 def world():
@@ -647,3 +648,91 @@ def sharded_cc_matrix_multiplication_nonzero_hoisted(ev, ctA, ctB, d, sigma, tau
     out = ev.add(ctAB, rest)
     mark("tail")
     return out
+
+
+# ------------------------------------------------------------------ sharded blocked matrix product
+def blocked_shards(tiles, rank, world_size):
+    """this rank's share of cc_matrix_multiplication_blocked at tile grid (t_n, t_m, t_p): a contiguous run of the
+    t_n t_m + t_m t_p operand transforms (A's tiles, then B's, row-major) and a contiguous block of the t_n t_p output
+    tiles (owned_block of each count; ranks beyond a count get an empty range)"""
+    tn, tm, tp = tiles
+    return owned_block(tn * tm + tm * tp, rank, world_size), owned_block(tn * tp, rank, world_size)
+
+
+def _operand_scales(ctx, ct, first, sets, limbs):
+    """(scale of the entries k >= 1, scale0) of matmul_operands for tiles like `ct`, from the scale arithmetic alone (a
+    rank that transforms no tile of this operand still needs them)"""
+    s0 = ct.scale * first.special.scale
+    return _rescaled_pow2_scale(ctx, s0 * sets[0].special.scale, limbs), s0
+
+
+def sharded_cc_matrix_multiplication_blocked(ev, A_tiles, B_tiles, tiles, d, sigma, tau, V, W, keys, plans, rank,
+                                             world_size, exchange, method="reference"):
+    """cc_matrix_multiplication_blocked over world_size ranks; every rank returns the t_n t_p output tiles of the one-GPU
+    call word for word.  Every rank holds all input tiles and needs the one-GPU call's Galois keys.
+
+    1. The rank transforms its contiguous run of the t_n t_m + t_m t_p tiles (blocked_shards; matmul_operands, A's and
+       B's tiles of the run in one call each).  One all-gather of the entries, padded to the longest run: d size-2
+       ciphertexts per transformed tile at the product's level L - 1, so (t_n t_m + t_m t_p) d * 2 (L - 1) N words in
+       all (plus padding).  A rank with no tile sends zeros.
+    2. It contracts its owned_block of the output tiles (row-major), one multiply_sum_matrix per touched tile row.
+    3. A second all-gather of the t_n t_p size-3 outputs (3 (L - 1) N words each, padded; zeros from ranks that own
+       none) gives every rank all of them."""
+    tn, tm, tp = (int(x) for x in tiles)
+    if min(tn, tm, tp) < 1 or A_tiles.batch != tn * tm or B_tiles.batch != tm * tp:
+        raise ValueError("sharded_cc_matrix_multiplication_blocked: tile batches do not match the tile grid")
+    ctx, nA = A_tiles.ctx, tn * tm
+    mine, outs = blocked_shards((tn, tm, tp), rank, world_size)
+    L = A_tiles.limbs - 1
+    sX, sX0 = _operand_scales(ctx, A_tiles, sigma, V, A_tiles.limbs)
+    sY, sY0 = _operand_scales(ctx, B_tiles, tau, W, B_tiles.limbs)
+    # 1. this rank's transforms, padded to the longest run, all-gathered
+    per = -(-(nA + tm * tp) // world_size)
+    send = torch.zeros((per * d, 2, L, ctx.n), dtype=torch.int64, device=A_tiles.data.device)
+    pos = 0
+    for src, lo, hi, side in ((A_tiles, mine.start, min(mine.stop, nA), 0),
+                              (B_tiles, max(mine.start, nA) - nA, mine.stop - nA, 1)):
+        if hi > lo:
+            ent = matmul_operands(ev, src[lo:hi], [side] * (hi - lo), d, sigma, tau, V, W, keys, plans, method)
+            send[pos:pos + ent.data.batch] = ent.data.data[:, :, :L]
+            pos += ent.data.batch
+    got = exchange.all_gather(send)
+    order = []
+    for q in range(world_size):
+        blk = owned_block(nA + tm * tp, q, world_size)
+        order += range(q * per * d, q * per * d + len(blk) * d)
+    got = got.index_select(0, torch.as_tensor(order, device=got.device))
+    X = MatmulEntries(Ciphertext(ctx, got[:nA * d].contiguous(), L, sX), d, sX0)
+    Y = MatmulEntries(Ciphertext(ctx, got[nA * d:].contiguous(), L, sY), d, sY0)
+    del got
+    if X.scale0 * Y.scale0 != X.data.scale * Y.data.scale:
+        raise capi.CkksInvalidArgument("scale mismatch")
+    # 2. the owned output tiles, one contraction per touched tile row
+    per_out = -(-(tn * tp) // world_size)
+    part = torch.zeros((per_out, 3, L, ctx.n), dtype=torch.int64, device=send.device)
+    del send
+    if len(outs):
+        Yc = _column_major_rows(Y, tp)
+        inner = tm * d
+        o = outs.start
+        while o < outs.stop:
+            i, j0 = divmod(o, tp)
+            j1 = min(tp, j0 + outs.stop - o)
+            if j1 - j0 == tp:
+                b = Yc
+            else:
+                cols = torch.arange(j0, j1, device=part.device)
+                idx = (torch.arange(inner, device=part.device)[:, None] * tp + cols[None, :]).reshape(-1)
+                b = Ciphertext(ctx, Yc.data.index_select(0, idx), L, Yc.scale)
+            a = X.data[i * inner:(i + 1) * inner]
+            r = ev.multiply_sum_matrix(a, b, 1, j1 - j0)
+            part[o - outs.start:o - outs.start + j1 - j0] = r.data[:, :, :L]
+            o += j1 - j0
+    # 3. every rank's outputs
+    got = exchange.all_gather(part)
+    order = []
+    for q in range(world_size):
+        blk = owned_block(tn * tp, q, world_size)
+        order += range(q * per_out, q * per_out + len(blk))
+    got = got.index_select(0, torch.as_tensor(order, device=got.device))
+    return Ciphertext(ctx, got, L, sX * sY)

@@ -566,29 +566,184 @@ def linear_transform_plain_sparse(ev, ct, dset, keys, plans, rots=None, s_all=No
 
 def cc_matrix_multiplication_sparse(ev, ctA, ctB, d, sigma, tau, V, W, keys, plans):
     """CC_Matrix_Multiplication with DiagonalSets (sigma, tau, V[k], W[k]); same op sequence and
-    bit-identical result as cc_matrix_multiplication, feasible at d = 64 (d^2 = 4096 = N/4)"""
-    dd = d * d
-    A0 = linear_transform_plain_sparse(ev, ctA, sigma, keys, plans)
-    B0 = linear_transform_plain_sparse(ev, ctB, tau, keys, plans)
-    rotA = rotations_of(ev, duplicate_fill(ev, A0, dd, keys), dd, plans)
-    sA = ev.add_many(rotA)
-    A = [linear_transform_plain_sparse(ev, None, V[k], keys, plans, rots=rotA, s_all=sA) for k in range(d - 1)]
-    del rotA
-    rotB = rotations_of(ev, duplicate_fill(ev, B0, dd, keys), dd, plans)
-    sB = ev.add_many(rotB)
-    B = [linear_transform_plain_sparse(ev, None, W[k], keys, plans, rots=rotB, s_all=sB) for k in range(d - 1)]
-    del rotB
-    Ak, Bk = _stack(A), _stack(B)
-    ev.rescale_to_next_inplace(Ak)
-    ev.rescale_to_next_inplace(Bk)
-    ctAB = ev.multiply(A0, B0)
-    ev.mod_switch_to_next_inplace(ctAB)
-    force_scale_pow2(Ak)
-    force_scale_pow2(Bk)
-    rest = ev.multiply_sum(Ak, Bk)
-    if rest.scale != ctAB.scale:
+    bit-identical result as cc_matrix_multiplication, feasible at d = 64 (d^2 = 4096 = N/4).
+    The operand transforms are matmul_operands(method="reference"), the tail a 1 x 1 matmul_contract."""
+    X = matmul_operands(ev, ctA, [0], d, sigma, tau, V, W, keys, plans)
+    Y = matmul_operands(ev, ctB, [1], d, sigma, tau, V, W, keys, plans)
+    return matmul_contract(ev, X, Y, 1, 1)
+
+
+# ------------------------------------------------------------------ blocked matrix products
+# One tile product P(A, B) = ModSwitch(A0 x B0) + sum_{k=1}^{d-1} A_k x B_k (A0 = sigma(A), B0 = tau(B), A_k / B_k the
+# V_k / W_k transforms after the rescale and the forced scale).  ModSwitch drops the last limb and the tensor product
+# works limb by limb, so ModSwitch(A0 x B0) = ModSwitch(A0) x ModSwitch(B0) word for word, and
+#     P(A, B) = sum_{k=0}^{d-1} X_k x Y_k,   X_0 = ModSwitch(A0), X_k = A_k   (Y likewise for B).
+# A tile's X (or Y) does not depend on the tile it is paired with, and sums modulo q are exact, so the blocked product
+# C_ij = sum_l P(A_il, B_lj) is one ciphertext matrix product of the entries: (t_n x t_m d) by (t_m d x t_p).
+class MatmulEntries:
+    """the operand side of encrypted matrix products: d size-2 ciphertexts per tile at the product's level, tile-major
+    (entry t*d + k, k = 0 first) or, when `cols` is set, for a t_m x cols grid of B tiles in the contraction's row order
+    (entry (l*d + k)*cols + j for tile (l, j)).  `data` carries the scale of the entries k >= 1 (rescaled, power of two);
+    `scale0` is the scale of the entries k = 0 (the mod-switched sigma / tau transform)."""
+
+    def __init__(self, data, d, scale0, cols=None):
+        self.data, self.d, self.scale0, self.cols = data, int(d), float(scale0), cols
+
+    tiles = property(lambda self: self.data.batch // self.d)
+
+    def __getitem__(self, idx):
+        """the entries of tiles idx (a slice)"""
+        lo, hi, _ = idx.indices(self.tiles)
+        return MatmulEntries(self.data[lo * self.d:hi * self.d], self.d, self.scale0)
+
+
+def _entries(X0, Xk, d, order=None):
+    """MatmulEntries from n size-2 sigma / tau transforms X0 (mod-switched) and their n (d - 1) rescaled V_k / W_k
+    transforms Xk (tile-major): entry k of tile t goes to position order[t*d + k] (default t*d + k)"""
+    n, L = X0.batch, Xk.limbs
+    dev = X0.data.device
+    pos = torch.arange(n * d, device=dev) if order is None else torch.as_tensor(np.asarray(order), device=dev)
+    pos = pos.reshape(n, d)
+    data = torch.empty((n * d, 2, L, X0.ctx.n), dtype=torch.int64, device=dev)
+    data.index_copy_(0, pos[:, 0].contiguous(), X0.data[:, :, :L])
+    data.index_copy_(0, pos[:, 1:].reshape(-1), Xk.data[:, :, :L])
+    return MatmulEntries(Ciphertext(X0.ctx, data, L, Xk.scale), d, X0.scale)
+
+
+def matmul_row_order(tm, cols, d):
+    """positions of the entries of a t_m x cols grid of B tiles (row-major tile order, d per tile) in the contraction's
+    row order: tile (l, j), entry k -> (l*d + k)*cols + j"""
+    l, j, k = np.meshgrid(np.arange(tm), np.arange(cols), np.arange(d), indexing="ij")
+    return ((l * d + k) * cols + j).reshape(-1)
+
+
+def matmul_operands(ev, cts, sides, d, sigma, tau, V, W, keys, plans, method="reference", order=None):
+    """the operand side of CC_Matrix_Multiplication for a batch of tiles: cts[t] is a tile of A (sides[t] = 0: sigma and
+    the V_k) or of B (sides[t] = 1: tau and the W_k).  Returns MatmulEntries (d per tile, in the order of cts, or entry k
+    of tile t at position order[t*d + k]).
+
+    method="reference": the transforms of cc_matrix_multiplication_sparse, tile by tile (the d^2 rotations of each
+    transformed tile are shared by its d - 1 V_k / W_k transforms), every ciphertext bit-identical to the reference's
+    sequence.
+    method="hoisted": those of cc_matrix_multiplication_nonzero_hoisted (DiagonalSets encoded at the key level), all tiles
+    in one rotate_multiply_sum_hoisted call per step; the plaintexts of a side are shared by its tiles.  That call holds
+    the inputs, outputs and digit decompositions of every tile at once, so its memory grows with the number of tiles;
+    where that is too much, pass blocks of tiles in separate calls -- a sub-plan's outputs equal the full plan's word for
+    word."""
+    dd, n = d * d, cts.batch
+    if len(sides) != n:
+        raise ValueError("matmul_operands: one side per tile")
+    if method == "reference":
+        X0, Xk = [], []
+        for t, side in enumerate(sides):
+            first, sets = (sigma, V) if side == 0 else (tau, W)
+            x0 = linear_transform_plain_sparse(ev, cts[t], first, keys, plans)
+            rots = rotations_of(ev, duplicate_fill(ev, x0, dd, keys), dd, plans)
+            s_all = ev.add_many(rots)
+            Xk.append(_stack([linear_transform_plain_sparse(ev, None, ds, keys, plans, rots=rots, s_all=s_all)
+                              for ds in sets]))
+            del rots
+            X0.append(x0)
+        X0, Xk = _stack(X0), _stack(Xk)
+    elif method == "hoisted":
+        present = sorted(set(sides))
+        firsts = [(sigma, tau)[s] for s in present]
+        sets = [ds for s in present for ds in (V, W)[s]]
+        base, off = {}, 0
+        for s, ds in zip(present, firsts):
+            base[s], off = off, off + len(ds.index)
+        first = [[(t, int(l), base[s] + i) for i, l in enumerate((sigma, tau)[s].index)] for t, s in enumerate(sides)]
+        base2, off = {}, 0
+        for s in present:
+            for k, ds in enumerate((V, W)[s]):
+                base2[s, k], off = off, off + len(ds.index)
+        second = [[(t, int(l), base2[s, k] + i) for i, l in enumerate(ds.index)]
+                  for t, s in enumerate(sides) for k, ds in enumerate((V, W)[s])]
+        pts = _stack([ds.special for ds in firsts])
+        X0 = ev.rotate_multiply_sum_hoisted(duplicate_fill(ev, cts, dd, keys), pts, plans.rms(n, pts.batch, first))
+        pts = _stack([ds.special for ds in sets])
+        Xk = ev.rotate_multiply_sum_hoisted(duplicate_fill(ev, X0, dd, keys), pts, plans.rms(n, pts.batch, second))
+    else:
+        raise ValueError("unknown matrix product method")
+    ev.rescale_to_next_inplace(Xk)
+    force_scale_pow2(Xk)
+    ev.mod_switch_to_next_inplace(X0)
+    return _entries(X0, Xk, d, order)
+
+
+def _column_major_rows(Y, cols):
+    """entries of tiles (l, j) in row-major tile order (l < t_m, j < cols), d per tile -> the t_m d x cols matrix of the
+    contraction, row r = l d + k"""
+    d = Y.d
+    if cols == 1:
+        return Y.data
+    inner = Y.tiles // cols
+    l, k, j = np.meshgrid(np.arange(inner), np.arange(d), np.arange(cols), indexing="ij")
+    idx = torch.as_tensor(((l * cols + j) * d + k).reshape(-1), device=Y.data.data.device)
+    data = Y.data.data.index_select(0, idx)
+    return Ciphertext(Y.data.ctx, data, Y.data.limbs, Y.data.scale)
+
+
+def matmul_contract(ev, X, Y, rows, cols):
+    """C_ij = sum_l sum_k X_{il,k} x Y_{lj,k} for MatmulEntries X (rows x t_m tiles, tile-major) and Y (t_m x cols tiles,
+    tile-major or already in the contraction's row order, Y.cols == cols): one multiply_sum_matrix, rows x cols size-3
+    ciphertexts (not relinearised).  Each equals the sum over l of the tile products, word for word."""
+    if X.d != Y.d or X.tiles % rows or Y.tiles % cols or X.tiles // rows != Y.tiles // cols:
+        raise ValueError("matmul_contract: tile grids do not match")
+    if X.scale0 * Y.scale0 != X.data.scale * Y.data.scale:
         raise capi.CkksInvalidArgument("scale mismatch")
-    return ev.add(ctAB, rest)
+    b = Y.data if Y.cols == cols else _column_major_rows(Y, cols)
+    return ev.multiply_sum_matrix(X.data, b, rows, cols)
+
+
+def cc_matrix_multiplication_blocked(ev, A_tiles, B_tiles, tiles, d, sigma, tau, V, W, keys, plans, method="reference"):
+    """Encrypted matrix product of any shape from d x d tiles (matrix_tiles): A is t_n x t_m tiles, B t_m x t_p
+    (`tiles` = (t_n, t_m, t_p)), both batches in row-major tile order.  Returns the t_n t_p size-3 tiles of A B, row-major,
+    not relinearised (as CC_Matrix_Multiplication returns them).
+
+    Output tile (i, j) equals word for word the sum over l (Evaluator.add, in any order) of the per-tile products
+    cc_matrix_multiplication_sparse(A_il, B_lj) (method="reference", DiagonalSets as for it) or
+    cc_matrix_multiplication_nonzero_hoisted(A_il, B_lj) (method="hoisted", DiagonalSets at the key level, `keys`:
+    matmul_nonzero_hoisted_steps(d)).  Each tile is transformed once (t_n t_m + t_m t_p operand transforms instead of
+    2 t_n t_m t_p), then one ciphertext contraction (matmul_contract).  d >= 2."""
+    tn, tm, tp = (int(x) for x in tiles)
+    if min(tn, tm, tp) < 1 or A_tiles.batch != tn * tm or B_tiles.batch != tm * tp:
+        raise ValueError("cc_matrix_multiplication_blocked: tile batches do not match the tile grid")
+    if d < 2:
+        raise ValueError("cc_matrix_multiplication_blocked: tiles must be at least 2 x 2")
+    if method == "hoisted":
+        if A_tiles.scale != B_tiles.scale or A_tiles.limbs != B_tiles.limbs:
+            raise capi.CkksInvalidArgument("scale mismatch")
+        nA = tn * tm * d
+        order = np.concatenate([np.arange(nA), nA + matmul_row_order(tm, tp, d)])
+        XY = matmul_operands(ev, _stack([A_tiles, B_tiles]), [0] * (tn * tm) + [1] * (tm * tp), d, sigma, tau, V, W,
+                             keys, plans, method, order=order)
+        X, Y = XY[0:tn * tm], MatmulEntries(XY.data[nA:], d, XY.scale0, cols=tp)
+    else:
+        X = matmul_operands(ev, A_tiles, [0] * (tn * tm), d, sigma, tau, V, W, keys, plans, method)
+        Y = matmul_operands(ev, B_tiles, [1] * (tm * tp), d, sigma, tau, V, W, keys, plans, method,
+                            order=matmul_row_order(tm, tp, d))
+        Y.cols = tp
+    return matmul_contract(ev, X, Y, tn, tp)
+
+
+def matrix_tiles(M, d):
+    """an n x m matrix -> its ceil(n/d) x ceil(m/d) zero-padded d x d tiles in row-major tile order, each in the
+    reference's row-major d^2-slot layout (C_Matrix_Encode form): array [tiles, d*d] and the tile grid shape"""
+    M = np.asarray(M, dtype=np.float64)
+    n, m = M.shape
+    tr, tc = -(-n // d), -(-m // d)
+    P = np.zeros((tr * d, tc * d))
+    P[:n, :m] = M
+    return P.reshape(tr, d, tc, d).transpose(0, 2, 1, 3).reshape(tr * tc, d * d), (tr, tc)
+
+
+def matrix_from_tiles(slots, shape, d):
+    """inverse of matrix_tiles: decoded tiles (row-major tile order, at least d*d slots each) -> the n x m matrix"""
+    n, m = shape
+    tr, tc = -(-n // d), -(-m // d)
+    T = np.asarray(slots)[:tr * tc, :d * d].reshape(tr, tc, d, d)
+    return T.transpose(0, 2, 1, 3).reshape(tr * d, tc * d)[:n, :m]
 
 
 # ------------------------------------------------------------------ tolerance mode: only the non-empty diagonals
@@ -734,24 +889,7 @@ def linear_transform_plain_bsgs_double_hoisted(ev, ct, bd, keys, plans):
 def cc_matrix_multiplication_nonzero_hoisted(ev, ctA, ctB, d, sigma, tau, V, W, keys, plans):
     """cc_matrix_multiplication_nonzero with double hoisting: sigma(A) and tau(B) in one rotate_multiply_sum_hoisted call
     (2 inputs, 2 outputs), the V_k / W_k step in another (2 inputs, 2(d-1) outputs), then the same tail (rescale, forced
-    scales, size-3 accumulation).  The DiagonalSets are encoded at the key level.  `keys`: matmul_nonzero_hoisted_steps(d)."""
-    dd = d * d
-    first, second = matmul_nonzero_hoisted_terms(sigma.index, tau.index, [s.index for s in V], [s.index for s in W])
-    X = _stack([duplicate_fill(ev, ctA, dd, keys), duplicate_fill(ev, ctB, dd, keys)])
-    pts = _stack([sigma.special, tau.special])
-    AB0 = ev.rotate_multiply_sum_hoisted(X, pts, plans.rms(2, pts.batch, first))
-    A0, B0 = AB0[0], AB0[1]
-    Y = _stack([duplicate_fill(ev, A0, dd, keys), duplicate_fill(ev, B0, dd, keys)])
-    pts = _stack([s.special for s in list(V) + list(W)])
-    step2 = ev.rotate_multiply_sum_hoisted(Y, pts, plans.rms(2, pts.batch, second))
-    Ak, Bk = step2[0:d - 1], step2[d - 1:]
-    ev.rescale_to_next_inplace(Ak)
-    ev.rescale_to_next_inplace(Bk)
-    ctAB = ev.multiply(A0, B0)
-    ev.mod_switch_to_next_inplace(ctAB)
-    force_scale_pow2(Ak)
-    force_scale_pow2(Bk)
-    rest = ev.multiply_sum(Ak, Bk)
-    if rest.scale != ctAB.scale:
-        raise capi.CkksInvalidArgument("scale mismatch")
-    return ev.add(ctAB, rest)
+    scales, size-3 accumulation): matmul_operands(method="hoisted") of both tiles and a 1 x 1 matmul_contract.  The
+    DiagonalSets are encoded at the key level.  `keys`: matmul_nonzero_hoisted_steps(d)."""
+    XY = matmul_operands(ev, _stack([ctA, ctB]), [0, 1], d, sigma, tau, V, W, keys, plans, method="hoisted")
+    return matmul_contract(ev, XY[0:1], XY[1:2], 1, 1)
